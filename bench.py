@@ -24,6 +24,9 @@ One JSON line on stdout (rank 0):
   cudnn_baseline  the reference's own torch graph (oracle port, F.conv1d -> cuDNN) on this GPU, TF32 on and off
   cpu_baseline  the oracle port of the reference's CPU path on this box's host cores (N=1 only)
 --impl reference times that CPU path alone (the reference arm).
+
+--dump-outputs DIR writes what the last timed device-resident step returned (rank 0's o_hat and frames) as DIR/<name>.npy,
+so that two builds run with the same arguments, hence on the same seeded inputs, can be compared output for output.
 """
 import argparse
 import json
@@ -38,11 +41,14 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the benchmark leaves the tree as it found it (which may be read-only)
 
 SR = 22050
 HOP = 256
 GFLOP_PER_FRAME = 0.65766          # SURVEY.md section 8d: 657.66 MFLOP per spectrogram frame
 FFMA_PEAK_TFLOPS = 74.4            # nominal 148 SM x 128 lanes x 2 x 1.965 GHz (fallback)
+DUMP_BYTES = 60_000_000            # --dump-outputs: o_hat + frames written whole up to this size ...
+DUMP_SAMPLE = 4_000_000            # ... else this many seeded samples of o_hat (values + float64 indices: 48 MB)
 
 
 def ffma_peak():
@@ -279,6 +285,23 @@ def cudnn_reference(B, secs, steps=3):
     return out
 
 
+def dump_outputs(path, o_hat, frames):
+    """What the last timed step returned: path/o_hat.npy (float32 [B, hop * T]) and path/frames.npy (float64 [B]).
+    An o_hat too large for DUMP_BYTES is written as a fixed, seeded sample of DUMP_SAMPLE of its elements instead:
+    o_hat.npy holds the values, o_hat_index.npy their flat indices (float64, exact below 2**53)."""
+    os.makedirs(path, exist_ok=True)
+    o = o_hat.cpu().numpy()
+    out = {"frames": frames.cpu().numpy().astype(np.float64)}
+    if o.nbytes + out["frames"].nbytes <= DUMP_BYTES:
+        out["o_hat"] = o
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(o.size, DUMP_SAMPLE, replace=False))
+        out["o_hat"] = o.reshape(-1)[idx]
+        out["o_hat_index"] = idx.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def latency_config1(conv, secs_list=(3.0, 10.0), iters=20):
     """BASELINE configs[0] on the GPU: ToneColorConverter.convert of ONE clip (batch 1), host array in, host array
     out, median wall time."""
@@ -322,7 +345,13 @@ def main():
     ap.add_argument("--no-modes", action="store_true", help="skip the short side measurements of the other precisions")
     ap.add_argument("--no-cudnn", action="store_true", help="skip the reference-on-this-GPU (PyTorch / cuDNN) column")
     ap.add_argument("--no-sides", action="store_true", help="skip every side measurement (modes, config1/3/4, cudnn, cpu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed device-resident step returned (o_hat, frames) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs: only the native arm has a device-resident timed path")
     if args.impl == "reference":
         return run_reference(args)
     if args.no_sides:
@@ -376,8 +405,7 @@ def main():
     frames_dev = torch.empty(B, dtype=torch.int64, device=dev)
 
     def device_step(seed):      # every buffer at a stable address: the library replays the call from a CUDA graph
-        o, _ = conv.model.native.convert_waveform(wav_dev, wav_len, src, tgt, tau=0.3, seed=seed, out=out_dev, frames_out=frames_dev)
-        return o
+        return conv.model.native.convert_waveform(wav_dev, wav_len, src, tgt, tau=0.3, seed=seed, out=out_dev, frames_out=frames_dev)
 
     def barrier():
         if world > 1:
@@ -402,11 +430,13 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for s in range(args.steps):
-        device_step(1000 + s)
+        last = device_step(1000 + s)
     e1.record()
     barrier()
     ms_dev = max_over_ranks(e0.elapsed_time(e1)) / args.steps
     launches_per_call = native.last_launch_count
+    if args.dump_outputs and rank == 0:     # before the legs below reuse the output buffers
+        dump_outputs(args.dump_outputs, *last)
 
     # ---- per-kernel leg (roofline): the same steps again with CUDA events around every conv launch
     native.profile_enable(True)

@@ -13,6 +13,8 @@ import numpy as np
 import pytest
 import torch
 
+from oracle.golden import Golden
+
 pytestmark = pytest.mark.gpu
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -20,7 +22,7 @@ CASES = ["tts_b1_t37", "tts_b2_padded", "tts_b1_t121_tails"]
 
 
 def load(name):
-    d = np.load(os.path.join(GOLD, name + ".npz"))
+    d = Golden(os.path.join(GOLD, name + ".npz"))
     return d, json.loads(str(d["meta"]))
 
 
@@ -90,11 +92,11 @@ def test_infer_matches_reference(name, precision, tts):
     yl = d["y_lengths"]
     assert np.array_equal(y_mask[:, 0].sum(1).long().cpu().numpy(), yl)
     assert np.array_equal(attn[:, 0].sum(1).cpu().numpy(), d["w_ceil"])          # frames per token
-    assert tuple(o.shape) == d["o"].shape
+    assert tuple(o.shape) == d.shape("o")
     ym = y_mask.cpu().numpy()
-    e_zp = np.abs(z_p.cpu().numpy() - d["z_p"] * ym).max() / rms(d["z_p"])
-    e_z = np.abs(z.cpu().numpy() * ym - d["z"] * ym).max() / rms(d["z"])
-    e_o = np.abs(o.cpu().numpy() - d["o"]).max() / rms(d["o"])
+    e_zp = np.abs(d.pick("z_p", z_p.cpu().numpy()) - d["z_p"] * d.pick("z_p", ym)).max() / d.rms("z_p")
+    e_z = np.abs(d.pick("z", z.cpu().numpy() * ym) - d["z"] * d.pick("z", ym)).max() / d.rms("z")
+    e_o = np.abs(d.pick("o", o.cpu().numpy()) - d["o"]).max() / d.rms("o")
     print(name, precision, dict(z_p=e_zp, z=e_z, o=e_o))
     assert e_zp < 1e-4 and e_z < 1e-4 and e_o < 1e-4
 

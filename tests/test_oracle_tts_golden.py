@@ -8,13 +8,19 @@ import pytest
 import torch
 
 from oracle import tts_oracle as T
+from oracle.golden import Golden
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 CASES = ["tts_b1_t37", "tts_b2_padded", "tts_b1_t121_tails"]
+# max |oracle - reference| per tensor.  The goldens are the reference's fp32 output on one CPU; on a CPU with another vector
+# width or thread count the oracle's fp32 sums round differently, by up to a few times the reference's own fp32 noise floor
+# (fp32 vs fp64 twin, floor_* in golden/REPORT_tts.json).  Where that floor is large -- logw_sdp 4.8e-5 (amplified by the
+# spline inverses), z_p / z 8.8e-6, x 1.9e-6 -- the bound is about 4x it; on the other tensors the floor is <= 1.6e-6.
+TOL = {"x": 8e-6, "m_p": 4e-6, "logs_p": 4e-6, "logw_sdp": 2e-4, "logw_dp": 4e-6, "z_p": 4e-5, "z": 4e-5}
 
 
 def load(name):
-    d = np.load(os.path.join(GOLD, name + ".npz"))
+    d = Golden(os.path.join(GOLD, name + ".npz"))
     return d, json.loads(str(d["meta"]))
 
 
@@ -38,10 +44,12 @@ def test_infer_matches_reference(name, tts_sd):
     d, c = load(name)
     r = run_case(tts_sd, c)
     for key in ("x", "m_p", "logs_p", "logw_sdp", "logw_dp", "z_p", "z"):
-        assert np.abs(r[key].numpy() - d[key]).max() < 4e-6, key
+        err = np.abs(d.pick(key, r[key].numpy()) - d[key]).max()
+        assert err < TOL[key], (key, err)
     assert np.array_equal(r["w_ceil"][:, 0].numpy(), d["w_ceil"])
     assert np.array_equal(r["y_lengths"].numpy(), d["y_lengths"])
-    assert np.abs(r["o"].numpy() - d["o"]).max() < 1e-6
+    assert r["o"].shape == d.shape("o")
+    assert np.abs(d.pick("o", r["o"].numpy()) - d["o"]).max() < 1e-6
 
 
 def test_spline_inverse_undoes_forward():
