@@ -83,8 +83,9 @@ OVC_API void ovc_destroy(ovc_ctx* ctx);
 OVC_API int ovc_load_tensor(ovc_ctx* ctx, const char* key, const float* data, const int64_t* shape, int ndim);
 
 /* Fold weight-norm (g*v/||v||, per dim-0 slice), absorb the channel Flips of the flow into the
- * coupling weights, repack every conv for the kernels and upload.  OVC_ERR_MISSING names the
- * first missing key. */
+ * coupling weights, repack every conv for the kernels and upload.  The first bad tensor fails the
+ * call and the message names its key: OVC_ERR_MISSING when it is missing, OVC_ERR_INVALID when
+ * its shape is wrong. */
 OVC_API int ovc_finalize_weights(ovc_ctx* ctx);
 
 /* Number of floats of device workspace a call with (B, Tmax) needs (informational; the arena

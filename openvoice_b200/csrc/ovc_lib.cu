@@ -10,7 +10,9 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <optional>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/ovc.h"
@@ -59,6 +61,12 @@ struct DeviceGuard {
     if (e_ != cudaSuccess)                                                                        \
       return fail(OVC_ERR_CUDA, "%s failed: %s (%s:%d)", #expr, cudaGetErrorString(e_), __FILE__, \
                   __LINE__);                                                                      \
+  } while (0)
+
+#define TRY(expr)                   \
+  do {                              \
+    int rc_ = (expr);               \
+    if (rc_ != OVC_OK) return rc_;  \
   } while (0)
 
 // cuTensorMapEncodeTiled, resolved through the runtime (no link-time dependency on libcuda)
@@ -156,6 +164,13 @@ struct TtsLayers {
   size_t cf_pre_w[4] = {0}, cf_pre_b[4] = {0}, cf_pw[4] = {0}, cf_pb[4] = {0};
 };
 
+// one profiled launch: kernel variant, family (1 = MRF conv: the roofline total of ovc_profile_read), algorithmic work
+struct ProfRec {
+  int variant = 0, family = 0;
+  double flops = 0, bytes = 0;
+  int tag = 0;   // (Cin << 16 | K << 8 | dilation) of a tensor-core launch, else 0
+};
+
 struct DebugBuf {
   float* d = nullptr;
   int64_t shape[4] = {0, 0, 0, 0};
@@ -235,14 +250,10 @@ struct ovc_ctx {
   size_t tts_floats = 0;
   int tts_B = 0, tts_T = 0;
 
-  // profiling
+  // profiling: launch k of prof_log is bracketed by events ev[2k], ev[2k + 1]
   bool prof = false;
   std::vector<cudaEvent_t> ev;
-  size_t ev_used = 0;
-  double prof_ms = 0, prof_flops = 0, prof_bytes = 0;
-  int64_t prof_launches = 0;
-  std::vector<double> ev_flops, ev_bytes;
-  std::vector<int> ev_variant, ev_family, ev_tag;   // tag: (Cin << 16 | K << 8 | dilation) of a tensor-core launch, else 0
+  std::vector<ovc::ProfRec> prof_log;
 
   // debug taps
   bool debug = false;
@@ -277,29 +288,69 @@ static const HostTensor* find(const ovc_ctx* c, const std::string& k) {
   return it == c->sd.end() ? nullptr : &it->second;
 }
 
-// effective weight of a (possibly weight-normed) conv: g * v / ||v|| over dims != 0
-// (torch.nn.utils.weight_norm dim=0; modules.py:160,172,182, models.py:247)
-static int effective_weight(const ovc_ctx* c, const std::string& prefix, HostTensor* out, std::string* missing) {
-  if (const HostTensor* w = find(c, prefix + ".weight")) {
-    *out = *w;
-    return 0;
+// Checkpoint tensors by key and expected shape (-1: any extent; an empty shape: not checked).  The first error is kept
+// -- a missing key is OVC_ERR_MISSING, a mis-shaped one OVC_ERR_INVALID, both naming the key -- and a failed read
+// returns null / an empty tensor, so a packing step checks ok() once after its reads.
+struct Reader {
+  ovc_ctx* c;
+  int code = OVC_OK;
+  std::string msg;
+
+  bool ok() const { return code == OVC_OK; }
+  int status() const { return ok() ? OVC_OK : fail(code, "%s", msg.c_str()); }
+  void error(int cd, const std::string& k, const std::string& what) {
+    if (ok()) { code = cd; msg = "checkpoint tensor '" + k + "' " + what; }
   }
-  const HostTensor* v = find(c, prefix + ".weight_v");
-  const HostTensor* g = find(c, prefix + ".weight_g");
-  if (!v) { *missing = prefix + ".weight_v"; return -1; }
-  if (!g) { *missing = prefix + ".weight_g"; return -1; }
-  *out = *v;
-  const int64_t d0 = v->shape[0];
-  const int64_t inner = v->numel() / d0;
-  if (g->numel() != d0) { *missing = prefix + ".weight_g(shape)"; return -1; }
-  for (int64_t i = 0; i < d0; ++i) {
-    double ss = 0;
-    for (int64_t j = 0; j < inner; ++j) { const double q = v->data[i * inner + j]; ss += q * q; }
-    const float scale = g->data[i] / (float)std::sqrt(ss);
-    for (int64_t j = 0; j < inner; ++j) out->data[i * inner + j] = v->data[i * inner + j] * scale;
+  const HostTensor* get(const std::string& k, std::initializer_list<int64_t> shape) {
+    const HostTensor* t = find(c, k);
+    if (!t) { error(OVC_ERR_MISSING, k, "is missing"); return nullptr; }
+    bool good = !shape.size() || t->shape.size() == shape.size();
+    size_t i = 0;
+    for (int64_t d : shape) { if (good && d >= 0 && t->shape[i] != d) good = false; ++i; }
+    if (!good) { error(OVC_ERR_INVALID, k, "has shape " + dims(t->shape) + ", expected " + dims(shape)); return nullptr; }
+    return t;
   }
-  return 0;
-}
+  // effective weight of a (possibly weight-normed) conv: g * v / ||v|| over dims != 0
+  // (torch.nn.utils.weight_norm dim=0; modules.py:160,172,182, models.py:247)
+  HostTensor weff(const std::string& prefix, std::initializer_list<int64_t> shape) {
+    if (find(c, prefix + ".weight")) {
+      const HostTensor* w = get(prefix + ".weight", shape);
+      return w ? *w : HostTensor();
+    }
+    const HostTensor* v = get(prefix + ".weight_v", shape);
+    const HostTensor* g = v ? get(prefix + ".weight_g", {}) : nullptr;
+    if (!g) return HostTensor();
+    const int64_t d0 = v->shape[0];
+    const int64_t inner = v->numel() / d0;
+    if (g->numel() != d0) {
+      error(OVC_ERR_INVALID, prefix + ".weight_g", "has " + std::to_string(g->numel()) + " elements, expected " + std::to_string(d0));
+      return HostTensor();
+    }
+    HostTensor out = *v;
+    for (int64_t i = 0; i < d0; ++i) {
+      double ss = 0;
+      for (int64_t j = 0; j < inner; ++j) { const double q = v->data[i * inner + j]; ss += q * q; }
+      const float scale = g->data[i] / (float)std::sqrt(ss);
+      for (int64_t j = 0; j < inner; ++j) out.data[i * inner + j] = v->data[i * inner + j] * scale;
+    }
+    return out;
+  }
+  // append to the fp32 parameter arena (256-byte aligned blobs); 0 for a failed read
+  size_t put(const std::vector<float>& v) {
+    const size_t o = round_up(c->h_w.size(), 64);
+    c->h_w.resize(o + v.size());
+    std::copy(v.begin(), v.end(), c->h_w.begin() + o);
+    return o;
+  }
+  size_t put(const HostTensor* t) { return t ? put(t->data) : 0; }
+
+  template <class S>
+  static std::string dims(const S& s) {
+    std::string r;
+    for (int64_t d : s) r += (r.empty() ? "(" : ", ") + (d < 0 ? std::string("*") : std::to_string(d));
+    return r + ")";
+  }
+};
 
 // append a packed conv to the staging arena.  wfun(row_packed, ci, k) -> weight; bfun(row) -> bias
 template <class WF, class BF>
@@ -383,32 +434,6 @@ static bool key_is_hot(const std::string& k) {
          k.rfind("enc_p.", 0) == 0 || k.rfind("dp.", 0) == 0 || k.rfind("sdp.", 0) == 0 || k.rfind("emb_g.", 0) == 0;
 }
 
-static int pack_wn(ovc_ctx* c, const std::string& prefix, int n_layers, WNLayers* out, std::string* missing) {
-  const int H = 192;
-  for (int i = 0; i < n_layers; ++i) {
-    HostTensor w;
-    const std::string pin = prefix + ".in_layers." + std::to_string(i);
-    if (effective_weight(c, pin, &w, missing)) return -1;
-    if (w.shape.size() != 3 || w.shape[0] != 2 * H || w.shape[1] != H || w.shape[2] != 5) { *missing = pin + "(shape)"; return -1; }
-    // bias of the in_layer is folded into the per-batch conditioning vector (cond kernel)
-    out->in.push_back(pack_conv(
-        c, V_WN_IN, 2 * H, H,
-        [&](int p, int ci, int k) { return w.data[((size_t)paired_row(p, H) * H + ci) * 5 + k]; },
-        [&](int) { return 0.f; }, 0, 5, 2 * H));
-    const std::string prs = prefix + ".res_skip_layers." + std::to_string(i);
-    HostTensor r;
-    if (effective_weight(c, prs, &r, missing)) return -1;
-    const HostTensor* rb = find(c, prs + ".bias");
-    if (!rb) { *missing = prs + ".bias"; return -1; }
-    const int rows = (i < n_layers - 1) ? 2 * H : H;
-    if (r.shape[0] != rows || r.shape[1] != H) { *missing = prs + "(shape)"; return -1; }
-    out->rs.push_back(pack_conv(
-        c, V_WN_RS, rows, H, [&](int p, int ci, int) { return r.data[(size_t)p * H + ci]; },
-        [&](int p) { return rb->data[p]; }, rows, 1, rows));
-  }
-  return 0;
-}
-
 // tensor-core copy of a conv: fp16 [n_tile][Cin/16][K][column block][hi|lo][TN][8]: hi = fp16(w), lo = fp16((w - hi) * 2^11)
 // (ovc_tc.cuh), laid out exactly as the kernel's shared-memory operand slots (one TMA bulk copy per slot)
 template <class WF, class BF>
@@ -442,26 +467,33 @@ static TcLayer pack_tc(ovc_ctx* c, int Ntot, int Cin, int K, int DIL, WF wfun, B
   return T;
 }
 
-static int pack_wn_tc(ovc_ctx* c, const std::string& prefix, int n_layers, WNLayers* out, std::string* missing) {
+// one WN stack (modules.py:160-182), both packed forms: FFMA [C][T] layers and their tensor-core twins
+static void pack_wn(ovc_ctx* c, Reader& rd, const std::string& prefix, int n_layers, WNLayers* out) {
   const int H = 192;
-  for (int i = 0; i < n_layers; ++i) {
-    HostTensor w;
+  *out = WNLayers();
+  for (int i = 0; i < n_layers && rd.ok(); ++i) {
     const std::string pin = prefix + ".in_layers." + std::to_string(i);
-    if (effective_weight(c, pin, &w, missing)) return -1;
+    const HostTensor w = rd.weff(pin, {2 * H, H, 5});
+    const std::string prs = prefix + ".res_skip_layers." + std::to_string(i);
+    const int rows = (i < n_layers - 1) ? 2 * H : H;
+    const HostTensor r = rd.weff(prs, {rows, H, -1});
+    const HostTensor* rb = rd.get(prs + ".bias", {});
+    if (!rd.ok()) return;
+    // bias of the in_layer is folded into the per-batch conditioning vector (cond kernel)
+    out->in.push_back(pack_conv(
+        c, V_WN_IN, 2 * H, H,
+        [&](int p, int ci, int k) { return w.data[((size_t)paired_row(p, H) * H + ci) * 5 + k]; },
+        [&](int) { return 0.f; }, 0, 5, 2 * H));
+    out->rs.push_back(pack_conv(
+        c, V_WN_RS, rows, H, [&](int p, int ci, int) { return r.data[(size_t)p * H + ci]; },
+        [&](int p) { return rb->data[p]; }, rows, 1, rows));
     out->tc_in.push_back(pack_tc(
         c, 2 * H, H, 5, 1, [&](int p, int ci, int k) { return w.data[((size_t)paired_row32(p, H) * H + ci) * 5 + k]; },
-        [&](int) { return 0.f; }));   // bias comes per utterance from the cond kernel
-    const std::string prs = prefix + ".res_skip_layers." + std::to_string(i);
-    HostTensor r;
-    if (effective_weight(c, prs, &r, missing)) return -1;
-    const HostTensor* rb = find(c, prs + ".bias");
-    if (!rb) { *missing = prs + ".bias"; return -1; }
-    const int rows = (i < n_layers - 1) ? 2 * H : H;
+        [&](int) { return 0.f; }));
     out->tc_rs.push_back(pack_tc(
         c, rows, H, 1, 1, [&](int p, int ci, int) { return r.data[(size_t)p * H + ci]; },
         [&](int p) { return rb->data[p]; }));
   }
-  return 0;
 }
 
 #include "ovc_tts_pack.inc"   // pack_tts(): V1 TTS front-half weights (text encoder, duration predictors, emb_g)
@@ -469,32 +501,24 @@ static int pack_wn_tc(ovc_ctx* c, const std::string& prefix, int n_layers, WNLay
 static int finalize(ovc_ctx* c) {
   const ovc_hparams& hp = c->hp;
   const int H = 192, S = hp.spec_channels, G = hp.gin_channels;
-  std::string miss;
+  Reader rd{c};
   drop_graphs(c);               // captured launches point at the old weight arenas
   c->h_w.clear();
   c->h_tcw.clear();
-#define NEED(ptr, key)                                                                     \
-  const HostTensor* ptr = find(c, key);                                                    \
-  if (!ptr) return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing", std::string(key).c_str())
-#define WEFF(var, prefix)                                                                  \
-  HostTensor var;                                                                          \
-  if (effective_weight(c, prefix, &var, &miss)) return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str())
 
   // ---- posterior encoder (models.py:182-221)
   {
-    NEED(w, "enc_q.pre.weight");
-    NEED(b, "enc_q.pre.bias");
-    if (w->shape.size() != 3 || w->shape[0] != H || w->shape[1] != S) return fail(OVC_ERR_INVALID, "enc_q.pre.weight has the wrong shape");
+    const HostTensor* w = rd.get("enc_q.pre.weight", {H, S, -1});
+    const HostTensor* b = rd.get("enc_q.pre.bias", {});
+    if (!rd.ok()) return rd.status();
     c->enc_pre = pack_conv(c, V_ENC_PRE, H, S, [&](int p, int ci, int) { return w->data[(size_t)p * S + ci]; },
                            [&](int p) { return b->data[p]; }, H, 1, H);
     c->enc_pre16 = c->enc_pre;            // same packing, 16-byte cp.async when the spectrogram pitch allows it
     c->enc_pre16.variant = V_FLOW_PRE;
-    c->enc_wn = WNLayers();
-    if (pack_wn(c, "enc_q.enc", 16, &c->enc_wn, &miss) || pack_wn_tc(c, "enc_q.enc", 16, &c->enc_wn, &miss))
-      return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
-    NEED(pw, "enc_q.proj.weight");
-    NEED(pb, "enc_q.proj.bias");
-    if (pw->shape[0] != 2 * H || pw->shape[1] != H) return fail(OVC_ERR_INVALID, "enc_q.proj.weight has the wrong shape");
+    pack_wn(c, rd, "enc_q.enc", 16, &c->enc_wn);
+    const HostTensor* pw = rd.get("enc_q.proj.weight", {2 * H, H, -1});
+    const HostTensor* pb = rd.get("enc_q.proj.bias", {});
+    if (!rd.ok()) return rd.status();
     c->enc_proj = pack_conv(c, V_ENC_PROJ, 2 * H, H,
                             [&](int p, int ci, int) { return pw->data[(size_t)paired_row(p, H) * H + ci]; },
                             [&](int p) { return pb->data[paired_row(p, H)]; }, 2 * H, 1, 2 * H);
@@ -505,29 +529,27 @@ static int finalize(ovc_ctx* c) {
   for (int f = 0; f < 4; ++f) {
     const std::string p = "flow.flows." + std::to_string(2 * f);
     const bool flipped = f & 1;
-    NEED(w, p + ".pre.weight");
-    NEED(b, p + ".pre.bias");
-    if (w->shape[0] != H || w->shape[1] != 96) return fail(OVC_ERR_INVALID, "%s.pre.weight has the wrong shape", p.c_str());
+    const HostTensor* w = rd.get(p + ".pre.weight", {H, 96, -1});
+    const HostTensor* b = rd.get(p + ".pre.bias", {});
+    if (!rd.ok()) return rd.status();
     c->flow_pre[f] = pack_conv(
         c, V_FLOW_PRE, H, 96,
         [&](int r, int ci, int) { return w->data[(size_t)r * 96 + (flipped ? 95 - ci : ci)]; },
         [&](int r) { return b->data[r]; }, H, 1, H);
-    c->flow_wn[f] = WNLayers();
-    if (pack_wn(c, p + ".enc", 4, &c->flow_wn[f], &miss) || pack_wn_tc(c, p + ".enc", 4, &c->flow_wn[f], &miss))
-      return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
-    NEED(pw, p + ".post.weight");
-    NEED(pb, p + ".post.bias");
-    if (pw->shape[0] != 96 || pw->shape[1] != H) return fail(OVC_ERR_INVALID, "%s.post.weight has the wrong shape (mean_only couplings only)", p.c_str());
+    pack_wn(c, rd, p + ".enc", 4, &c->flow_wn[f]);
+    const HostTensor* pw = rd.get(p + ".post.weight", {96, H, -1});   // mean_only couplings only
+    const HostTensor* pb = rd.get(p + ".post.bias", {});
+    if (!rd.ok()) return rd.status();
     c->flow_post[f] = pack_conv(
         c, V_FLOW_POST, 96, H,
         [&](int r, int ci, int) { return pw->data[(size_t)(flipped ? 95 - r : r) * H + ci]; },
         [&](int r) { return pb->data[flipped ? 95 - r : r]; }, 96, 1, 96);
   }
   // ---- generator (models.py:224-291)
-  NEED(cpb, "dec.conv_pre.bias");
+  const HostTensor* cpb = rd.get("dec.conv_pre.bias", {});
   {
-    NEED(w, "dec.conv_pre.weight");
-    if (w->shape[0] != 512 || w->shape[1] != H || w->shape[2] != 7) return fail(OVC_ERR_INVALID, "dec.conv_pre.weight has the wrong shape");
+    const HostTensor* w = rd.get("dec.conv_pre.weight", {512, H, 7});
+    if (!rd.ok()) return rd.status();
     // bias comes per batch item from the cond kernel (conv_pre.bias + cond(g))
     c->dec_pre = pack_conv(c, V_A_K7D1, 512, H, [&](int r, int ci, int k) { return w->data[((size_t)r * H + ci) * 7 + k]; },
                            [&](int) { return 0.f; }, 0, 7, 512);
@@ -539,9 +561,9 @@ static int finalize(ovc_ctx* c) {
     const int s = hp.upsample_rates[i], kk = hp.upsample_kernel_sizes[i], pad = (kk - s) / 2;
     const int cin = ch, cout = ch / 2;
     const std::string p = "dec.ups." + std::to_string(i);
-    WEFF(w, p);   // [cin][cout][kk], weight-norm over dim 0 = cin (SURVEY appendix C.12)
-    NEED(b, p + ".bias");
-    if (w.shape[0] != cin || w.shape[1] != cout || w.shape[2] != kk) return fail(OVC_ERR_INVALID, "%s weight has the wrong shape", p.c_str());
+    const HostTensor w = rd.weff(p, {cin, cout, kk});   // [cin][cout][kk], weight-norm over dim 0 = cin (SURVEY appendix C.12)
+    const HostTensor* b = rd.get(p + ".bias", {});
+    if (!rd.ok()) return rd.status();
     const int variant = s == 8 ? V_UPS8_A : (cout * s >= 128 ? V_UPS2_A : V_UPS2_B);
     // polyphase: out[co, s*n+ph] = sum_ci sum_m x[ci, n-m] * W[ci, co, s*m + ph + pad];
     // packed row = co*s + ph, tap 0/1/2 <-> x[n-1], x[n], x[n+1] <-> m = 1, 0, -1
@@ -570,9 +592,9 @@ static int finalize(ovc_ctx* c) {
       for (int d = 0; d < 3; ++d) {
         for (int which = 0; which < 2; ++which) {
           const std::string q = "dec.resblocks." + std::to_string(rbi) + (which ? ".convs2." : ".convs1.") + std::to_string(d);
-          WEFF(rw, q);
-          NEED(rbias, q + ".bias");
-          if (rw.shape[0] != ch || rw.shape[1] != ch || rw.shape[2] != K) return fail(OVC_ERR_INVALID, "%s weight has the wrong shape", q.c_str());
+          const HostTensor rw = rd.weff(q, {ch, ch, K});
+          const HostTensor* rbias = rd.get(q + ".bias", {});
+          if (!rd.ok()) return rd.status();
           const int dil = which ? 1 : hp.resblock_dilations[j][d];
           ConvLayer L = pack_conv(c, dec_variant(ch, K, dil), ch, ch,
                                   [&](int r, int ci, int k) { return rw.data[((size_t)r * ch + ci) * K + k]; },
@@ -585,28 +607,21 @@ static int finalize(ovc_ctx* c) {
       }
     }
   }
-  {
-    NEED(w, "dec.conv_post.weight");
-    if (w->shape[0] != 1 || w->shape[1] != 32 || w->shape[2] != 7) return fail(OVC_ERR_INVALID, "dec.conv_post.weight has the wrong shape");
-    c->post_w_off = round_up(c->h_w.size(), 64);
-    c->h_w.resize(c->post_w_off + 32 * 7);
-    std::copy(w->data.begin(), w->data.end(), c->h_w.begin() + c->post_w_off);
-  }
+  c->post_w_off = rd.put(rd.get("dec.conv_post.weight", {1, 32, 7}));
+  if (!rd.ok()) return rd.status();
   // ---- speaker conditioning mat-vec: stack cond_layer of enc_q, of the 4 couplings and dec.cond
   std::vector<int> wrow, sel;
   std::vector<float> cbias;
   {
     std::vector<float> cw;
-    auto add_wn = [&](const std::string& prefix, int n_layers, int first_row, int selv, bool add_matrix, bool tc_order = false) -> int {
-      HostTensor w;
-      if (effective_weight(c, prefix + ".cond_layer", &w, &miss)) return -1;
-      const HostTensor* cb = find(c, prefix + ".cond_layer.bias");
-      if (!cb) { miss = prefix + ".cond_layer.bias"; return -1; }
-      if (w.shape[0] != 2 * H * n_layers || w.shape[1] != G) { miss = prefix + ".cond_layer(shape)"; return -1; }
+    auto add_wn = [&](const std::string& prefix, int n_layers, int first_row, int selv, bool add_matrix, bool tc_order) {
+      const HostTensor w = rd.weff(prefix + ".cond_layer", {2 * H * n_layers, G, -1});
+      const HostTensor* cb = rd.get(prefix + ".cond_layer.bias", {});
+      if (!rd.ok()) return;
       if (add_matrix) cw.insert(cw.end(), w.data.begin(), w.data.end());
       for (int l = 0; l < n_layers; ++l) {
-        const HostTensor* ib = find(c, prefix + ".in_layers." + std::to_string(l) + ".bias");
-        if (!ib) { miss = prefix + ".in_layers." + std::to_string(l) + ".bias"; return -1; }
+        const HostTensor* ib = rd.get(prefix + ".in_layers." + std::to_string(l) + ".bias", {});
+        if (!ib) return;
         for (int p = 0; p < 2 * H; ++p) {
           const int o = tc_order ? paired_row32(p, H) : paired_row(p, H);
           wrow.push_back(first_row + l * 2 * H + o);
@@ -614,33 +629,28 @@ static int finalize(ovc_ctx* c) {
           cbias.push_back(cb->data[l * 2 * H + o] + ib->data[o]);
         }
       }
-      return 0;
+    };
+    auto flows = [&](int selv, bool add_matrix, bool tc_order) {
+      for (int f = 0; f < 4; ++f)
+        add_wn("flow.flows." + std::to_string(2 * f) + ".enc", 4, 16 * 2 * H + f * 4 * 2 * H, selv, add_matrix, tc_order);
     };
     c->cond_off_enc = 0;
-    if (add_wn("enc_q.enc", 16, 0, hp.zero_g ? 0 : 1, true)) return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
+    add_wn("enc_q.enc", 16, 0, hp.zero_g ? 0 : 1, true, false);
     c->cond_off_fsrc = (int)wrow.size();
-    for (int f = 0; f < 4; ++f)
-      if (add_wn("flow.flows." + std::to_string(2 * f) + ".enc", 4, 16 * 2 * H + f * 4 * 2 * H, 1, true))
-        return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
+    flows(1, true, false);
     c->cond_off_ftgt = (int)wrow.size();
-    for (int f = 0; f < 4; ++f)
-      if (add_wn("flow.flows." + std::to_string(2 * f) + ".enc", 4, 16 * 2 * H + f * 4 * 2 * H, 2, false))
-        return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
+    flows(2, false, false);
     // the same conditioning vectors once more in the tensor-core kernel's column order
     c->cond_off_enc_tc = (int)wrow.size();
-    if (add_wn("enc_q.enc", 16, 0, hp.zero_g ? 0 : 1, false, true)) return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
+    add_wn("enc_q.enc", 16, 0, hp.zero_g ? 0 : 1, false, true);
     c->cond_off_fsrc_tc = (int)wrow.size();
-    for (int f = 0; f < 4; ++f)
-      if (add_wn("flow.flows." + std::to_string(2 * f) + ".enc", 4, 16 * 2 * H + f * 4 * 2 * H, 1, false, true))
-        return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
+    flows(1, false, true);
     c->cond_off_ftgt_tc = (int)wrow.size();
-    for (int f = 0; f < 4; ++f)
-      if (add_wn("flow.flows." + std::to_string(2 * f) + ".enc", 4, 16 * 2 * H + f * 4 * 2 * H, 2, false, true))
-        return fail(OVC_ERR_MISSING, "checkpoint tensor '%s' is missing or mis-shaped", miss.c_str());
+    flows(2, false, true);
     c->cond_off_dec = (int)wrow.size();
-    NEED(dw, "dec.cond.weight");
-    NEED(db, "dec.cond.bias");
-    if (dw->shape[0] != 512 || dw->shape[1] != G) return fail(OVC_ERR_INVALID, "dec.cond.weight has the wrong shape");
+    const HostTensor* dw = rd.get("dec.cond.weight", {512, G, -1});
+    const HostTensor* db = rd.get("dec.cond.bias", {});
+    if (!rd.ok()) return rd.status();
     const int dec_first = (int)(cw.size() / G);
     cw.insert(cw.end(), dw->data.begin(), dw->data.end());
     for (int r = 0; r < 512; ++r) {
@@ -649,55 +659,38 @@ static int finalize(ovc_ctx* c) {
       cbias.push_back(db->data[r] + cpb->data[r]);
     }
     c->cond_rows_out = (int)wrow.size();
-    c->cond_w_off = round_up(c->h_w.size(), 64);
-    c->h_w.resize(c->cond_w_off + cw.size());
-    std::copy(cw.begin(), cw.end(), c->h_w.begin() + c->cond_w_off);
-    c->cond_b_off = round_up(c->h_w.size(), 64);
-    c->h_w.resize(c->cond_b_off + cbias.size());
-    std::copy(cbias.begin(), cbias.end(), c->h_w.begin() + c->cond_b_off);
+    c->cond_w_off = rd.put(cw);
+    c->cond_b_off = rd.put(cbias);
   }
   // ---- ReferenceEncoder (optional: only extract_se needs it; models.py:301-338)
   c->has_refenc = false;
   if (find(c, "ref_enc.proj.weight")) {
-    auto put = [&](const std::vector<float>& v) { size_t o = round_up(c->h_w.size(), 64); c->h_w.resize(o + v.size()); std::copy(v.begin(), v.end(), c->h_w.begin() + o); return o; };
     static const int filt[7] = {1, 32, 32, 64, 64, 128, 128};
     for (int i = 0; i < 6; ++i) {
       const std::string q = "ref_enc.convs." + std::to_string(i);
-      WEFF(cw, q);
-      NEED(cb, q + ".bias");
-      if (cw.shape.size() != 4 || cw.shape[0] != filt[i + 1] || cw.shape[1] != filt[i] || cw.shape[2] != 3 || cw.shape[3] != 3)
-        return fail(OVC_ERR_INVALID, "%s weight has the wrong shape", q.c_str());
-      c->re_conv_w[i] = put(cw.data);
-      c->re_conv_b[i] = put(cb->data);
+      const HostTensor cw = rd.weff(q, {filt[i + 1], filt[i], 3, 3});
+      const HostTensor* cb = rd.get(q + ".bias", {});
+      if (!rd.ok()) return rd.status();
+      c->re_conv_w[i] = rd.put(cw.data);
+      c->re_conv_b[i] = rd.put(cb);
     }
-    NEED(wih, "ref_enc.gru.weight_ih_l0"); NEED(whh, "ref_enc.gru.weight_hh_l0");
-    NEED(bih, "ref_enc.gru.bias_ih_l0"); NEED(bhh, "ref_enc.gru.bias_hh_l0");
-    NEED(rpw, "ref_enc.proj.weight"); NEED(rpb, "ref_enc.proj.bias");
-    NEED(lng, "ref_enc.layernorm.weight"); NEED(lnb, "ref_enc.layernorm.bias");
-    if (wih->shape[0] != 384 || whh->shape[0] != 384 || whh->shape[1] != 128 || rpw->shape[0] != G || rpw->shape[1] != 128 ||
-        lng->shape[0] != S)
-      return fail(OVC_ERR_INVALID, "ref_enc.* tensors have the wrong shape");
-    {
-      int w6 = S;   // width after the six stride-2 convs (models.py:330-337)
-      for (int i = 0; i < 6; ++i) w6 = (w6 - 1) / 2 + 1;
-      if (wih->shape.size() != 2 || wih->shape[1] != 128 * w6 || bih->numel() != 384 || bhh->numel() != 384 ||
-          lnb->numel() != S || rpb->numel() != G)
-        return fail(OVC_ERR_INVALID, "ref_enc.gru / layernorm / proj tensors do not match spec_channels %d (GRU input %d expected)",
-                    S, 128 * w6);
-      c->re_gru_in = 128 * w6;
-    }
-    c->re_wih = put(wih->data); c->re_whh = put(whh->data); c->re_bih = put(bih->data); c->re_bhh = put(bhh->data);
-    c->re_pw = put(rpw->data); c->re_pb = put(rpb->data); c->re_lng = put(lng->data); c->re_lnb = put(lnb->data);
+    int w6 = S;   // width after the six stride-2 convs (models.py:330-337)
+    for (int i = 0; i < 6; ++i) w6 = (w6 - 1) / 2 + 1;
+    c->re_gru_in = 128 * w6;
+    c->re_wih = rd.put(rd.get("ref_enc.gru.weight_ih_l0", {384, 128 * w6}));
+    c->re_whh = rd.put(rd.get("ref_enc.gru.weight_hh_l0", {384, 128}));
+    c->re_bih = rd.put(rd.get("ref_enc.gru.bias_ih_l0", {384}));
+    c->re_bhh = rd.put(rd.get("ref_enc.gru.bias_hh_l0", {384}));
+    c->re_pw = rd.put(rd.get("ref_enc.proj.weight", {G, 128}));
+    c->re_pb = rd.put(rd.get("ref_enc.proj.bias", {G}));
+    c->re_lng = rd.put(rd.get("ref_enc.layernorm.weight", {S}));
+    c->re_lnb = rd.put(rd.get("ref_enc.layernorm.bias", {S}));
+    if (!rd.ok()) return rd.status();
     c->has_refenc = true;
   }
   // ---- V1 TTS front half (optional: base-speaker checkpoints only, models.py:451-465)
   c->tts = TtsLayers();
-  if (find(c, "enc_p.emb.weight")) {
-    const int rc = pack_tts(c);
-    if (rc != OVC_OK) return rc;
-  }
-#undef NEED
-#undef WEFF
+  if (find(c, "enc_p.emb.weight")) TRY(pack_tts(c, rd));
   // ---- upload
   ON_DEVICE(c);
   if (c->d_w) { cudaFree(c->d_w); c->d_w = nullptr; }
@@ -781,95 +774,14 @@ static WsLayout ws_layout(const ovc_ctx* c, int B, int Tmax) {
   return L;
 }
 
-#define TRY(expr)                   \
-  do {                              \
-    int rc_ = (expr);               \
-    if (rc_ != OVC_OK) return rc_;  \
-  } while (0)
-
 struct Run {
   ovc_ctx* c;
   cudaStream_t st;
   int B, Tmax, P;
   const long long* lens;
   const long long* glens;   // generator lengths: lens when ragged, NULL (= Tmax) otherwise
-  double sum_len;           // sum over batch of generator frames (for FLOP/byte accounting): B*Tmax upper bound
 };
 
-static int launch(Run& r, const ConvLayer& L, ConvArgs a, int t_len, bool mrf = false, double flops = 0,
-                  double bytes = 0) {
-  a.w = r.c->d_w + L.w_off;
-  a.n_chunks = L.n_chunks;
-  a.cin = L.cin;
-  a.tmax = r.Tmax;
-  if (a.scale == 0.f) a.scale = 1.f;
-  ovc_ctx* c = r.c;
-  const bool prof = c->prof;
-  if (prof) {
-    if (c->ev_used + 2 > c->ev.size()) {
-      const size_t old = c->ev.size();
-      c->ev.resize(old + 512);
-      for (size_t i = old; i < c->ev.size(); ++i) CK(cudaEventCreate(&c->ev[i]));
-    }
-    CK(cudaEventRecord(c->ev[c->ev_used], r.st));
-  }
-  CK(kLaunch[L.variant](a, t_len, L.row_tiles, r.B, r.st));
-  c->launches++;
-  if (prof) {
-    CK(cudaEventRecord(c->ev[c->ev_used + 1], r.st));
-    c->ev_used += 2;
-    // algorithmic work of this launch over all B * t_len positions (upper bound for ragged batches)
-    const double units = (double)r.B * t_len;
-    c->ev_flops.push_back(2.0 * L.cout * L.cin * L.K * units * L.out_mul);
-    c->ev_bytes.push_back(4.0 * units * ((double)L.cin + (double)L.cout * L.out_mul));
-    c->ev_variant.push_back(L.variant);
-    c->ev_family.push_back(mrf ? 1 : 0);
-    c->ev_tag.push_back(0);
-  }
-  (void)flops; (void)bytes;
-  return OVC_OK;
-}
-
-static int tap(Run& r, const char* name, const float* src, int C, int T, int pitch) {
-  ovc_ctx* c = r.c;
-  if (!c->debug) return OVC_OK;
-  DebugBuf& d = c->taps[name];
-  const size_t n = (size_t)r.B * C * pitch;
-  if (d.floats < n) {
-    if (d.d) cudaFree(d.d);
-    CK(cudaMalloc(&d.d, n * sizeof(float)));
-    d.floats = n;
-  }
-  d.shape[0] = r.B; d.shape[1] = C; d.shape[2] = T; d.shape[3] = pitch;
-  CK(cudaMemcpyAsync(d.d, src, n * sizeof(float), cudaMemcpyDeviceToDevice, r.st));
-  return OVC_OK;
-}
-
-
-// profiling bracket shared by the non-conv1d_f32 launches
-static int prof_begin(Run& r) {
-  ovc_ctx* c = r.c;
-  if (!c->prof) return OVC_OK;
-  if (c->ev_used + 2 > c->ev.size()) {
-    const size_t old = c->ev.size();
-    c->ev.resize(old + 512);
-    for (size_t i = old; i < c->ev.size(); ++i) CK(cudaEventCreate(&c->ev[i]));
-  }
-  CK(cudaEventRecord(c->ev[c->ev_used], r.st));
-  return OVC_OK;
-}
-static int prof_end(Run& r, int variant, int family, double flops, double bytes, int tag = 0) {
-  ovc_ctx* c = r.c;
-  if (!c->prof) return OVC_OK;
-  CK(cudaEventRecord(c->ev[c->ev_used + 1], r.st));
-  c->ev_used += 2;
-  c->ev_flops.push_back(flops);
-  c->ev_bytes.push_back(bytes);
-  c->ev_variant.push_back(variant);
-  c->ev_family.push_back(family);
-  c->ev_tag.push_back(tag);
-  return OVC_OK;
-}
 enum { V_TCPAIR64 = -12, V_TCPAIR32 = -13, V_TC128 = -1, V_TC64 = -2, V_TC32 = -3, V_TRANSPOSE = -4, V_TTS_DENSE = -5, V_TTS_LN = -6, V_TTS_SCORES = -7,
        V_TTS_ATTN = -8, V_TTS_DW = -9, V_TTS_SPLINE = -10, V_TTS_MISC = -11 };
 static const char* variant_name(int v) {
@@ -891,8 +803,78 @@ static const char* variant_name(int v) {
   }
 }
 
-// one conv on the tensor cores (3xFP16 split precision / single-pass fp16), channels-last in/out.  t_len / mul are in INPUT steps.
-struct TcExtra {
+// Every counted kernel launch: `enqueue` puts one kernel on r.st (a <<<>>> launch, or a call that returns its
+// cudaError_t).  With profiling on and a record given, two events bracket the launch and the record is kept.
+template <class F>
+static int launch_kernel(Run& r, const std::optional<ProfRec>& rec, F enqueue) {
+  ovc_ctx* c = r.c;
+  const bool prof = c->prof && rec;
+  const size_t e = 2 * c->prof_log.size();
+  if (prof) {
+    if (e + 2 > c->ev.size()) {
+      const size_t old = c->ev.size();
+      c->ev.resize(old + 512);
+      for (size_t i = old; i < c->ev.size(); ++i) CK(cudaEventCreate(&c->ev[i]));
+    }
+    CK(cudaEventRecord(c->ev[e], r.st));
+  }
+  if constexpr (std::is_void<decltype(enqueue())>::value) enqueue();
+  else CK(enqueue());
+  CK(cudaGetLastError());
+  c->launches++;
+  if (prof) {
+    CK(cudaEventRecord(c->ev[e + 1], r.st));
+    c->prof_log.push_back(*rec);
+  }
+  return OVC_OK;
+}
+
+// ConvArgs of one FFMA conv: x [B][x_C][x_pitch] -> y [B][y_C][y_pitch] over the frame limits `lens` (time axis in
+// units of `mul` samples), leaky-relu `slope` on the input; the layer's own bias unless the caller sets one
+static ConvArgs conv_args(const float* x, int x_C, int x_pitch, float* y, int y_C, int y_pitch, const long long* lens, int mul,
+                          float slope) {
+  ConvArgs a{};
+  a.x = x; a.x_bs = (long long)x_C * x_pitch; a.x_pitch = x_pitch;
+  a.y = y; a.y_bs = (long long)y_C * y_pitch; a.y_pitch = y_pitch;
+  a.lens_in = lens; a.lens_out = lens; a.mul_in = mul; a.mul_out = mul;
+  a.slope = slope; a.scale = 1.f;
+  return a;
+}
+
+static int launch(Run& r, const ConvLayer& L, ConvArgs a, int t_len, bool mrf = false) {
+  a.w = r.c->d_w + L.w_off;
+  if (!a.bias) a.bias = r.c->d_w + L.b_off;
+  a.n_chunks = L.n_chunks;
+  a.cin = L.cin;
+  a.tmax = r.Tmax;
+  // algorithmic work of this launch over all B * t_len positions (upper bound for ragged batches)
+  const double units = (double)r.B * t_len;
+  const ProfRec rec{L.variant, mrf ? 1 : 0, 2.0 * L.cout * L.cin * L.K * units * L.out_mul,
+                    4.0 * units * ((double)L.cin + (double)L.cout * L.out_mul)};
+  return launch_kernel(r, rec, [&] { return kLaunch[L.variant](a, t_len, L.row_tiles, r.B, r.st); });
+}
+
+static int tap(Run& r, const char* name, const float* src, int C, int T, int pitch) {
+  ovc_ctx* c = r.c;
+  if (!c->debug) return OVC_OK;
+  DebugBuf& d = c->taps[name];
+  const size_t n = (size_t)r.B * C * pitch;
+  if (d.floats < n) {
+    if (d.d) cudaFree(d.d);
+    CK(cudaMalloc(&d.d, n * sizeof(float)));
+    d.floats = n;
+  }
+  d.shape[0] = r.B; d.shape[1] = C; d.shape[2] = T; d.shape[3] = pitch;
+  CK(cudaMemcpyAsync(d.d, src, n * sizeof(float), cudaMemcpyDeviceToDevice, r.st));
+  return OVC_OK;
+}
+
+// how one conv runs on the tensor cores; a call sets only what differs from these defaults
+struct TcOpt {
+  float slope = 1.f;              // leaky_relu slope on the input (1 = identity)
+  float scale = 1.f;              // epilogue multiplier (1/3 for the last MRF accumulation)
+  int accumulate = 0;             // y += result
+  int family = 0;                 // profile family: 1 MRF conv, 2 polyphase transposed conv, 0 other
   int epi = 0;                    // 0 linear, 1 WN gate, 2 WN res/skip
   const float* bias = nullptr;    // override (per-utterance conditioning vector), with stride
   long long bias_bs = 0;
@@ -920,26 +902,44 @@ static cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, int block, siz
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
-static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const float* res, int t_len, int mul, float slope,
-                     float scale, int accumulate, int family, const TcExtra& ex = TcExtra()) {
+// activation chunks by tensor-map TMA: the channels-last input as a [B][P * mul][C] fp32 tensor, one box = box_rows x 32
+// channels (128 bytes, 128-byte swizzle); rows outside the tensor are zero-filled by the copy engine
+static CUresult encode_act_map(CUtensorMap* tmap, const Run& r, const float* x, int C, int mul, int box_rows) {
+  memset(tmap, 0, sizeof *tmap);
+  const cuuint64_t gdim[3] = {(cuuint64_t)C, (cuuint64_t)r.P * mul, (cuuint64_t)r.B};
+  const cuuint64_t gstr[2] = {(cuuint64_t)C * 4, (cuuint64_t)((long long)C * r.P * mul) * 4};
+  const cuuint32_t box[3] = {32, (cuuint32_t)box_rows, 1};
+  const cuuint32_t estr[3] = {1, 1, 1};
+  return encode_tiled_fn()(tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(x), gdim, gstr, box, estr,
+                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+}
+
+// one conv on the tensor cores (3xFP16 split precision / single-pass fp16), channels-last in/out.  t_len / mul are in INPUT steps.
+static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const float* res, int t_len, int mul,
+                     const TcOpt& o = TcOpt()) {
   TcConvArgs a{};
-  const int y_ld = ex.y_ld ? ex.y_ld : T.Ntot;
+  const int y_ld = o.y_ld ? o.y_ld : T.Ntot;
   a.x = x; a.x_bs = (long long)T.Cin * r.P * mul;
   a.w = reinterpret_cast<const uint16_t*>(r.c->d_tcw + T.w_off);
-  a.bias = ex.bias ? ex.bias : r.c->d_tcw + T.b_off; a.bias_bs = ex.bias_bs;
+  a.bias = o.bias ? o.bias : r.c->d_tcw + T.b_off; a.bias_bs = o.bias_bs;
   a.y = y; a.y_bs = (long long)y_ld * r.P * mul; a.y_ld = y_ld;
   a.r = res;
-  a.s = ex.s; a.s_bs = a.y_bs;
-  a.epi = ex.epi; a.split = ex.split; a.first = ex.first;
-  a.lens = ex.use_lens_frames ? r.lens : r.glens; a.tmax = r.Tmax; a.mul = mul;
-  a.lens_x = ex.lens_x; a.has_lens_x = ex.has_lens_x ? 1 : 0;
+  a.s = o.s; a.s_bs = a.y_bs;
+  a.epi = o.epi; a.split = o.split; a.first = o.first;
+  a.lens = o.use_lens_frames ? r.lens : r.glens; a.tmax = r.Tmax; a.mul = mul;
+  a.lens_x = o.lens_x; a.has_lens_x = o.has_lens_x ? 1 : 0;
   a.Cin = T.Cin; a.Ntot = T.Ntot; a.K = T.K; a.DIL = T.DIL;
-  a.slope = slope; a.scale = scale; a.accumulate = accumulate;
+  a.slope = o.slope; a.scale = o.scale; a.accumulate = o.accumulate;
   a.passes = r.c->precision == 2 ? 1 : 3;
   a.tune = r.c->tune;
   if (T.TN == 0) return fail(OVC_ERR_INVALID, "conv %d -> %d (k %d, dilation %d) does not fit the tensor-core kernels", T.Cin, T.Ntot, T.K, T.DIL);
-  if (!(slope >= 0.f && slope <= 1.f)) return fail(OVC_ERR_INVALID, "leaky_relu slope %g outside [0, 1]", (double)slope);
-  TRY(prof_begin(r));
+  if (!(o.slope >= 0.f && o.slope <= 1.f)) return fail(OVC_ERR_INVALID, "leaky_relu slope %g outside [0, 1]", (double)o.slope);
+  const double units = (double)r.B * t_len;
+  const int eff_k = o.family == 2 ? 2 : T.K;   // polyphase transposed conv: 2 of the 3 packed taps are non-zero per row
+  const ProfRec rec{T.TN == 128 ? V_TC128 : T.TN == 64 ? V_TC64 : V_TC32, o.family == 1 ? 1 : 0, 2.0 * T.Cin * T.Ntot * eff_k * units,
+                    4.0 * (T.Cin + T.Ntot * (1 + (res ? 1 : 0) + (o.accumulate ? 1 : 0))) * units, (T.Cin << 16) | (T.K << 8) | T.DIL};
+  const bool pdl = r.c->use_pdl == 1 || (r.c->use_pdl == 2 && o.epi != 0);
   // 3 (default): the generator's first stage (k >= 7 at C = 256: few, long tiles) on the two-CTAs-per-SM kernel, whose
   // second CTA fills the tensor pipe while the first waits on a barrier; everything else on the persistent kernel
   int wv = r.c->wide_variant;
@@ -948,49 +948,35 @@ static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const f
     // A/B alternatives of the 128-column layers: 1 = 256-step tiles, one CTA per SM; 2 = 128-step tiles, two CTAs per SM
     const int MT = wv == 1 ? 2 : 1;
     dim3 grid((t_len + MT * 128 - 1) / (MT * 128), T.Ntot / 128, r.B);
-    const bool pdl = r.c->use_pdl == 1 || (r.c->use_pdl == 2 && ex.epi != 0);
-    if (wv == 1) CK(launch_ex(tcconv_wide_kernel<2>, grid, TcwCfg<2>::THREADS, TcwCfg<2>::SMEM_BYTES, r.st, pdl, a));
-    else CK(launch_ex(tcconv_wide_kernel<1>, grid, TcwCfg<1>::THREADS, TcwCfg<1>::SMEM_BYTES, r.st, pdl, a));
-  } else {
-    // persistent: one CTA per SM walks the (utterance, tile) list; column tiles (if any) on grid.y
-    const int MT = T.TN == 128 ? TcnCfg<128>::MT : TcnCfg<64>::MT;
-    const int steps = MT * 128;
-    const int n_tt = (t_len + steps - 1) / steps, total = n_tt * r.B;
-    // activation chunks by tensor-map TMA: the channels-last input as a [B][rows][Cin] fp32 tensor, one box = box_rows x 32
-    // channels (128 bytes, 128-byte swizzle); rows outside the tensor are zero-filled by the copy engine
-    CUtensorMap tmap;
-    memset(&tmap, 0, sizeof tmap);
-    a.act_tma = 0;
-    if (r.c->act_tma && encode_tiled_fn()) {
-      const int rows = tcn_rows(MT, (T.K - 1) / 2 * T.DIL);
-      a.n_box = rows > 256 ? 2 : 1;
-      a.box_rows = rows / a.n_box;
-      const cuuint64_t gdim[3] = {(cuuint64_t)T.Cin, (cuuint64_t)r.P * mul, (cuuint64_t)r.B};
-      const cuuint64_t gstr[2] = {(cuuint64_t)T.Cin * 4, (cuuint64_t)a.x_bs * 4};
-      const cuuint32_t box[3] = {32, (cuuint32_t)a.box_rows, 1};
-      const cuuint32_t estr[3] = {1, 1, 1};
-      const CUresult cr = encode_tiled_fn()(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(x), gdim, gstr, box, estr,
-                                            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                            CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-      if (cr != CUDA_SUCCESS) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a [%d][%d][%d] activation tensor", (int)cr,
-                                          r.B, r.P * mul, T.Cin);
-      a.act_tma = 1;
-    }
-    const int ncol = T.Ntot / T.TN;
-    const int per_col = std::max(1, r.c->sm_count / ncol / std::max(1, ex.grid_div));
-    dim3 pg((unsigned)std::min(total, per_col), ncol, 1);
-    const bool pdl = r.c->use_pdl == 1 || (r.c->use_pdl == 2 && ex.epi != 0);
-    if (T.TN == 128) CK(launch_ex(tcconv_kernel<128>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap));
-    else if (T.TN == 64) CK(launch_ex(tcconv_kernel<64>, pg, TCN_THREADS, TcnCfg<64>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap));
-    else CK(launch_ex(tcconv_kernel<32>, pg, TCN_THREADS, TcnCfg<32>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap));
+    return launch_kernel(r, rec, [&] {
+      return wv == 1 ? launch_ex(tcconv_wide_kernel<2>, grid, TcwCfg<2>::THREADS, TcwCfg<2>::SMEM_BYTES, r.st, pdl, a)
+                     : launch_ex(tcconv_wide_kernel<1>, grid, TcwCfg<1>::THREADS, TcwCfg<1>::SMEM_BYTES, r.st, pdl, a);
+    });
   }
-  CK(cudaGetLastError());
-  r.c->launches++;
-  const double units = (double)r.B * t_len;
-  const int eff_k = family == 2 ? 2 : T.K;   // polyphase transposed conv: 2 of the 3 packed taps are non-zero per row
-  TRY(prof_end(r, T.TN == 128 ? V_TC128 : T.TN == 64 ? V_TC64 : V_TC32, family == 1 ? 1 : 0, 2.0 * T.Cin * T.Ntot * eff_k * units,
-               4.0 * (T.Cin + T.Ntot * (1 + (res ? 1 : 0) + (accumulate ? 1 : 0))) * units, (T.Cin << 16) | (T.K << 8) | T.DIL));
-  return OVC_OK;
+  // persistent: one CTA per SM walks the (utterance, tile) list; column tiles (if any) on grid.y
+  const int MT = T.TN == 128 ? TcnCfg<128>::MT : TcnCfg<64>::MT;
+  const int steps = MT * 128;
+  const int n_tt = (t_len + steps - 1) / steps, total = n_tt * r.B;
+  CUtensorMap tmap;
+  memset(&tmap, 0, sizeof tmap);
+  a.act_tma = 0;
+  if (r.c->act_tma && encode_tiled_fn()) {
+    const int rows = tcn_rows(MT, (T.K - 1) / 2 * T.DIL);
+    a.n_box = rows > 256 ? 2 : 1;
+    a.box_rows = rows / a.n_box;
+    const CUresult cr = encode_act_map(&tmap, r, x, T.Cin, mul, a.box_rows);
+    if (cr != CUDA_SUCCESS) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a [%d][%d][%d] activation tensor", (int)cr,
+                                        r.B, r.P * mul, T.Cin);
+    a.act_tma = 1;
+  }
+  const int ncol = T.Ntot / T.TN;
+  const int per_col = std::max(1, r.c->sm_count / ncol / std::max(1, o.grid_div));
+  dim3 pg((unsigned)std::min(total, per_col), ncol, 1);
+  return launch_kernel(r, rec, [&] {
+    if (T.TN == 128) return launch_ex(tcconv_kernel<128>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
+    if (T.TN == 64) return launch_ex(tcconv_kernel<64>, pg, TCN_THREADS, TcnCfg<64>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
+    return launch_ex(tcconv_kernel<32>, pg, TCN_THREADS, TcnCfg<32>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
+  });
 }
 
 // one ResBlock conv pair (c1 dilated, c2 dilation 1, residual = the pair's input) as ONE kernel: C = 64 / 32 stages
@@ -1003,8 +989,8 @@ static bool pair_fits(const TcLayer& T1, const TcLayer& T2) {
   return T1.Ntot == T1.TN && T1.Cin == T1.TN && T2.Ntot == T1.TN && T2.Cin == T1.TN && T2.TN == T1.TN && T2.K == T1.K &&
          T2.DIL == 1 && (T1.K - 1) / 2 * T1.DIL <= hmax && 2 * (T1.Cin / 16) * T1.K <= ring && T1.K <= 5;
 }
-static int launch_pair(Run& r, const TcLayer& T1, const TcLayer& T2, const float* x, float* y, int t_len, int mul, float slope,
-                       float scale, int accumulate) {
+// slope, scale and accumulate of `o` apply (family: always MRF)
+static int launch_pair(Run& r, const TcLayer& T1, const TcLayer& T2, const float* x, float* y, int t_len, int mul, const TcOpt& o) {
   TcPairArgs a{};
   const int C = T1.TN;
   a.x = x; a.x_bs = (long long)C * r.P * mul;
@@ -1014,64 +1000,53 @@ static int launch_pair(Run& r, const TcLayer& T1, const TcLayer& T2, const float
   a.y = y; a.y_bs = a.x_bs;
   a.lens = r.glens; a.tmax = r.Tmax; a.mul = mul;
   a.C = C; a.K = T1.K; a.DIL1 = T1.DIL;
-  a.slope = slope; a.scale = scale; a.accumulate = accumulate;
+  a.slope = o.slope; a.scale = o.scale; a.accumulate = o.accumulate;
   a.passes = r.c->precision == 2 ? 1 : 3;
   if (!encode_tiled_fn()) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled is not available");
   const int H1 = (T1.K - 1) / 2 * T1.DIL, H2 = (T1.K - 1) / 2;
   const int R = 128 - 2 * H2, rows8 = (128 + 2 * H1 + 7) & ~7;
   const int n_tt = (t_len + R - 1) / R, total = n_tt * r.B;
   CUtensorMap tmap;
-  memset(&tmap, 0, sizeof tmap);
-  const cuuint64_t gdim[3] = {(cuuint64_t)C, (cuuint64_t)r.P * mul, (cuuint64_t)r.B};
-  const cuuint64_t gstr[2] = {(cuuint64_t)C * 4, (cuuint64_t)a.x_bs * 4};
-  const cuuint32_t box[3] = {32, (cuuint32_t)rows8, 1};
-  const cuuint32_t estr[3] = {1, 1, 1};
-  const CUresult cr = encode_tiled_fn()(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(x), gdim, gstr, box, estr,
-                                        CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  const CUresult cr = encode_act_map(&tmap, r, x, C, mul, rows8);
   if (cr != CUDA_SUCCESS) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a conv pair", (int)cr);
-  TRY(prof_begin(r));
-  dim3 pg((unsigned)std::min(total, r.c->sm_count), 1, 1);
-  if (C == 64) CK(launch_ex(tcpair_kernel<64>, pg, TCN_THREADS, TcpCfg<64>::SMEM_BYTES, r.st, false, a, n_tt, total, tmap));
-  else CK(launch_ex(tcpair_kernel<32>, pg, TCN_THREADS, TcpCfg<32>::SMEM_BYTES, r.st, false, a, n_tt, total, tmap));
-  CK(cudaGetLastError());
-  r.c->launches++;
   const double units = (double)r.B * t_len;
-  TRY(prof_end(r, C == 64 ? V_TCPAIR64 : V_TCPAIR32, 1, 2.0 * 2.0 * C * C * T1.K * units, 4.0 * C * (2 + (accumulate ? 1 : 0)) * units,
-               (C << 16) | (T1.K << 8) | T1.DIL));
-  return OVC_OK;
+  const ProfRec rec{C == 64 ? V_TCPAIR64 : V_TCPAIR32, 1, 2.0 * 2.0 * C * C * T1.K * units,
+                    4.0 * C * (2 + (o.accumulate ? 1 : 0)) * units, (C << 16) | (T1.K << 8) | T1.DIL};
+  dim3 pg((unsigned)std::min(total, r.c->sm_count), 1, 1);
+  return launch_kernel(r, rec, [&] {
+    return C == 64 ? launch_ex(tcpair_kernel<64>, pg, TCN_THREADS, TcpCfg<64>::SMEM_BYTES, r.st, false, a, n_tt, total, tmap)
+                   : launch_ex(tcpair_kernel<32>, pg, TCN_THREADS, TcpCfg<32>::SMEM_BYTES, r.st, false, a, n_tt, total, tmap);
+  });
 }
 
 static int launch_transpose(Run& r, const float* src, float* dst, int rows, int cols) {
   dim3 grid((cols + 31) / 32, (rows + 31) / 32, r.B);
-  TRY(prof_begin(r));
-  transpose_kernel<<<grid, 256, 0, r.st>>>(src, dst, rows, cols, (long long)rows * cols);
-  CK(cudaGetLastError());
-  r.c->launches++;
-  TRY(prof_end(r, V_TRANSPOSE, 0, 0.0, 8.0 * rows * cols * r.B));
-  return OVC_OK;
+  return launch_kernel(r, ProfRec{V_TRANSPOSE, 0, 0.0, 8.0 * rows * cols * r.B},
+                       [&] { transpose_kernel<<<grid, 256, 0, r.st>>>(src, dst, rows, cols, (long long)rows * cols); });
+}
+
+// every speaker-conditioning 1x1 conv of a call in one launch (rows of the cond section of the workspace)
+static int launch_cond(Run& r, const float* g_src, const float* g_tgt, float* out) {
+  ovc_ctx* c = r.c;
+  CondArgs a;
+  a.w = c->d_w + c->cond_w_off; a.bias = c->d_w + c->cond_b_off;
+  a.w_row = c->d_cond_wrow; a.sel = c->d_cond_sel;
+  a.g_src = g_src; a.g_tgt = g_tgt; a.out = out;
+  a.rows_out = c->cond_rows_out; a.gin = c->hp.gin_channels;
+  dim3 grid((c->cond_rows_out + 7) / 8, r.B);
+  return launch_kernel(r, std::nullopt, [&] { cond_kernel<<<grid, 256, 0, r.st>>>(a); });
 }
 
 // one WN stack (modules.py:185-210): x <- in place, skip <- output
 static int run_wn(Run& r, const WNLayers& wn, float* x, float* skip, float* acts, const float* cond, int cond_bs) {
   const int P = r.P, T = r.Tmax;
-  const long long bs = 192LL * P;
   const int n = (int)wn.in.size();
   for (int i = 0; i < n; ++i) {
-    ConvArgs a{};
-    a.x = x; a.x_bs = bs; a.x_pitch = P;
+    ConvArgs a = conv_args(x, 192, P, acts, 192, P, r.lens, 1, 1.f);
     a.bias = cond + (size_t)i * 384; a.bias_bs = cond_bs;
-    a.y = acts; a.y_bs = bs; a.y_pitch = P;
-    a.lens_in = r.lens; a.lens_out = r.lens; a.mul_in = 1; a.mul_out = 1;
-    a.slope = 1.f;
     TRY(launch(r, wn.in[i], a, T));
-    ConvArgs b{};
-    b.x = acts; b.x_bs = bs; b.x_pitch = P;
-    b.bias = r.c->d_w + wn.rs[i].b_off; b.bias_bs = 0;
-    b.y = x; b.y_bs = bs; b.y_pitch = P;
-    b.s = skip; b.s_bs = bs; b.s_pitch = P;
-    b.lens_in = r.lens; b.lens_out = r.lens; b.mul_in = 1; b.mul_out = 1;
-    b.slope = 1.f;
+    ConvArgs b = conv_args(acts, 192, P, x, 192, P, r.lens, 1, 1.f);
+    b.s = skip; b.s_bs = 192LL * P; b.s_pitch = P;
     b.split = (i < n - 1) ? 192 : 0;
     b.flags = (i == 0) ? F_FIRST : 0;
     TRY(launch(r, wn.rs[i], b, T));
@@ -1087,12 +1062,12 @@ static int run_wn_tc(Run& r, const WNLayers& wn, float* x, float* skip, float* a
   const int n = (int)wn.tc_in.size();
   TRY(launch_transpose(r, x, x_cl, 192, P));
   for (int i = 0; i < n; ++i) {
-    TcExtra g;
+    TcOpt g;
     g.epi = 1; g.bias = cond_tc + (size_t)i * 384; g.bias_bs = cond_bs; g.y_ld = 192; g.use_lens_frames = true;
-    TRY(launch_tc(r, wn.tc_in[i], x_cl, acts, nullptr, T, 1, 1.f, 1.f, 0, 0, g));
-    TcExtra q;
+    TRY(launch_tc(r, wn.tc_in[i], x_cl, acts, nullptr, T, 1, g));
+    TcOpt q;
     q.epi = 2; q.s = skip_cl; q.split = (i < n - 1) ? 192 : 0; q.first = (i == 0); q.y_ld = 192; q.use_lens_frames = true;
-    TRY(launch_tc(r, wn.tc_rs[i], acts, x_cl, nullptr, T, 1, 1.f, 1.f, 0, 0, q));
+    TRY(launch_tc(r, wn.tc_rs[i], acts, x_cl, nullptr, T, 1, q));
   }
   TRY(launch_transpose(r, skip_cl, skip, P, 192));
   return OVC_OK;
@@ -1101,7 +1076,6 @@ static int run_wn_tc(Run& r, const WNLayers& wn, float* x, float* skip, float* a
 static int run_flow(Run& r, const WsLayout& W, float* ws, bool reverse, const float* cond_all) {
   ovc_ctx* c = r.c;
   const int P = r.P, T = r.Tmax;
-  const long long bs = 192LL * P;
   float* z = ws + W.z;
   float* x = ws + W.x;
   float* skip = ws + W.skip;
@@ -1111,13 +1085,7 @@ static int run_flow(Run& r, const WsLayout& W, float* ws, bool reverse, const fl
     const int f = reverse ? 3 - step : step;
     const bool flipped = f & 1;
     // pre: x0 (physical lower half, or upper half when flipped) -> h     (modules.py:438-439)
-    ConvArgs a{};
-    a.x = z + (flipped ? 96 * (size_t)P : 0); a.x_bs = bs; a.x_pitch = P;
-    a.bias = c->d_w + c->flow_pre[f].b_off; a.bias_bs = 0;
-    a.y = x; a.y_bs = bs; a.y_pitch = P;
-    a.lens_in = r.lens; a.lens_out = r.lens; a.mul_in = 1; a.mul_out = 1;
-    a.slope = 1.f; a.scale = 1.f;
-    TRY(launch(r, c->flow_pre[f], a, T));
+    TRY(launch(r, c->flow_pre[f], conv_args(z + (flipped ? 96 * (size_t)P : 0), 192, P, x, 192, P, r.lens, 1, 1.f), T));
     if (c->precision >= 1) {
       const int sect_tc = reverse ? c->cond_off_ftgt_tc : c->cond_off_fsrc_tc;
       TRY(run_wn_tc(r, c->flow_wn[f], x, skip, acts, ws + W.bufA, ws + W.bufB, cond_all + sect_tc + f * 4 * 384, c->cond_rows_out));
@@ -1125,12 +1093,7 @@ static int run_flow(Run& r, const WsLayout& W, float* ws, bool reverse, const fl
       TRY(run_wn(r, c->flow_wn[f], x, skip, acts, cond_all + sect + f * 4 * 384, c->cond_rows_out));
     }
     // post + coupling update of x1 in place                                (modules.py:441-454)
-    ConvArgs b{};
-    b.x = skip; b.x_bs = bs; b.x_pitch = P;
-    b.bias = c->d_w + c->flow_post[f].b_off; b.bias_bs = 0;
-    b.y = z + (flipped ? 0 : 96 * (size_t)P); b.y_bs = bs; b.y_pitch = P;
-    b.lens_in = r.lens; b.lens_out = r.lens; b.mul_in = 1; b.mul_out = 1;
-    b.slope = 1.f;
+    ConvArgs b = conv_args(skip, 192, P, z + (flipped ? 0 : 96 * (size_t)P), 192, P, r.lens, 1, 1.f);
     b.sign = reverse ? -1.f : 1.f;
     TRY(launch(r, c->flow_post[f], b, T));
   }
@@ -1215,49 +1178,94 @@ static uintptr_t option_bits(const ovc_ctx* c) {
   return (uintptr_t)c->precision | ((uintptr_t)c->wide_variant << 4) | ((uintptr_t)c->act_tma << 8) | ((uintptr_t)c->use_pdl << 15) | ((uintptr_t)c->tune << 10) | ((uintptr_t)c->use_branches << 14) | ((uintptr_t)c->use_pair << 17);
 }
 
-static int ensure_ws(ovc_ctx* c, const WsLayout& W, int B, int Tmax, cudaStream_t st) {
-  if (W.total <= c->ws_floats) return OVC_OK;
+// Grow a device arena to `need` floats.  Work queued on `st` may still use the old one, so the stream drains first.  A
+// failed allocation leaves the arena empty and no CUDA error pending, and returns OVC_ERR_NOMEM.
+static int grow_arena(float*& d, size_t& floats, size_t need, cudaStream_t st, const char* what) {
+  if (need <= floats) return OVC_OK;
   CK(cudaStreamSynchronize(st));
-  drop_graphs(c);               // captured launches point into the old workspace
-  if (c->d_ws) CK(cudaFree(c->d_ws));
-  c->d_ws = nullptr;
-  c->ws_floats = 0;
-  cudaError_t e = cudaMalloc(&c->d_ws, W.total * sizeof(float));
+  if (d) CK(cudaFree(d));
+  d = nullptr;
+  floats = 0;
+  const cudaError_t e = cudaMalloc(&d, need * sizeof(float));
   if (e != cudaSuccess) {
+    d = nullptr;
     cudaGetLastError();
-    return fail(OVC_ERR_NOMEM, "workspace of %.2f GB for B=%d Tmax=%d does not fit: %s", W.total * 4e-9, B, Tmax,
-                cudaGetErrorString(e));
+    return fail(OVC_ERR_NOMEM, "%s of %.2f GB does not fit: %s", what, need * 4e-9, cudaGetErrorString(e));
   }
-  c->ws_floats = W.total;
+  floats = need;
   return OVC_OK;
+}
+
+static int ensure_ws(ovc_ctx* c, const WsLayout& W, cudaStream_t st) {
+  if (W.total > c->ws_floats) drop_graphs(c);   // captured launches point into the old workspace
+  return grow_arena(c->d_ws, c->ws_floats, W.total, st, "workspace");
 }
 
 // z (workspace, [B][192][P]) -> a caller tensor [B][192][Tmax], zero past each length
 static int copy_latent_out(Run& r, const WsLayout& W, float* ws, float* dst) {
   if (!dst) return OVC_OK;
   dim3 grid((r.Tmax + 255) / 256, 192, r.B);
-  copy_latent_kernel<<<grid, 256, 0, r.st>>>(ws + W.z, W.P, dst, r.Tmax, 192, r.lens);
-  CK(cudaGetLastError());
-  r.c->launches++;
+  return launch_kernel(r, std::nullopt, [&] { copy_latent_kernel<<<grid, 256, 0, r.st>>>(ws + W.z, W.P, dst, r.Tmax, 192, r.lens); });
+}
+
+// the MRF of upsampling stage i on the tensor cores (models.py:280-286): xs = sum_j ResBlock1_j(bufA) / 3 -> bufD.
+// `par`: a latency-bound call runs the three ResBlock branches side by side -- branch 0 on the caller's stream, 1 and 2
+// on side streams with their own B / C buffers, every kernel on a third of the SMs.  The MRF sum keeps its order (the
+// last conv of branch j waits for that of branch j - 1), so the result is bit-identical to the sequential schedule.
+static int run_mrf_tc(Run& r, const WsLayout& W, float* ws, int i, int Tlen, int up_out, bool par) {
+  ovc_ctx* c = r.c;
+  float* bufA = ws + W.bufA; float* bufD = ws + W.bufD;
+  if (par) CK(cudaEventRecord(c->br_ev[3], r.st));
+  for (int j = 0; j < 3; ++j) {
+    const TcLayer* c1 = c->tc_c1[i * 3 + j];
+    const TcLayer* c2 = c->tc_c2[i * 3 + j];
+    Run rj = r;
+    float* Bj = ws + W.bufB; float* Cj = ws + W.bufC;
+    TcOpt o;
+    o.slope = 0.1f; o.family = 1;
+    if (par) {
+      o.grid_div = 3;
+      if (j > 0) {
+        rj.st = c->br_stream[j - 1];
+        CK(cudaStreamWaitEvent(rj.st, c->br_ev[3], 0));
+        Bj = ws + W.brB[j - 1]; Cj = ws + W.brC[j - 1];
+      }
+    }
+    bool fused = !par && c->use_pair;
+    for (int d = 0; d < 3; ++d) fused = fused && pair_fits(c1[d], c2[d]);
+    for (int d = 0; d < 3; ++d) {
+      TcOpt o2 = o;
+      o2.scale = (d == 2 && j == 2) ? 1.0f / 3.0f : 1.f;   // xs / num_kernels (models.py:286), as a multiply
+      o2.accumulate = (d == 2 && j > 0) ? 1 : 0;
+      if (fused) {
+        // one kernel per conv pair; a pair never runs in place (its tiles read x with a halo), so the running
+        // activation ping-pongs bufA -> bufB -> bufC -> bufD (bufC is free: the intermediate stays on chip)
+        const float* xs[3] = {bufA, Bj, Cj};
+        float* ys[3] = {Bj, Cj, bufD};
+        TRY(launch_pair(rj, c1[d], c2[d], xs[d], ys[d], Tlen, up_out, o2));
+        continue;
+      }
+      const float* xin = d == 0 ? bufA : Bj;
+      TRY(launch_tc(rj, c1[d], xin, Cj, nullptr, Tlen, up_out, o));
+      if (par && d == 2 && j > 0) CK(cudaStreamWaitEvent(rj.st, c->br_ev[j - 1], 0));   // xs so far is complete
+      TRY(launch_tc(rj, c2[d], Cj, d < 2 ? Bj : bufD, xin, Tlen, up_out, o2));
+    }
+    if (par) CK(cudaEventRecord(c->br_ev[j], rj.st));
+  }
+  if (par) CK(cudaStreamWaitEvent(r.st, c->br_ev[2], 0));   // join (branch 1 is joined through branch 2's wait)
   return OVC_OK;
 }
 
 // HiFi-GAN generator on the latent in ws.z (models.py:272-291): shared by voice_conversion and the TTS decode
 static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, const long long* lens, float* o_hat) {
   ovc_ctx* c = r.c;
-  cudaStream_t st = r.st;
   const int B = r.B, Tmax = r.Tmax, P = W.P;
-  const long long bs192 = 192LL * P;
   // ---- generator (models.py:272-291).  Lengths: frames * cumulative upsampling.
   const bool pre_tc = c->precision >= 1 && c->tc_pre.TN != 0;
   if (!pre_tc) {
-    ConvArgs a{};
-    a.x = ws + W.z; a.x_bs = bs192; a.x_pitch = P;
+    ConvArgs a = conv_args(ws + W.z, 192, P, ws + W.dpre, 512, P, r.glens, 1, 1.f);
     a.bias = cond + c->cond_off_dec; a.bias_bs = c->cond_rows_out;
-    a.y = ws + W.dpre; a.y_bs = 512LL * P; a.y_pitch = P;
     a.lens_in = lens;          // z_hat * y_mask
-    a.lens_out = r.glens; a.mul_in = 1; a.mul_out = 1;
-    a.slope = 1.f; a.scale = 1.f;
     TRY(launch(r, c->dec_pre, a, Tmax));
     TRY(tap(r, "dec.pre", ws + W.dpre, 512, Tmax, P));
   }
@@ -1277,10 +1285,10 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
       // conv_pre (192 -> 512, k 7) + cond(g) on the tensor cores too: z channels-last through bufA, result straight into
       // bufE; the input is cut at the frame lengths (z_hat * y_mask), the output runs over the generator's own limit
       TRY(launch_transpose(r, ws + W.z, bufA, 192, P));
-      TcExtra e;
+      TcOpt e;
       e.bias = cond + c->cond_off_dec; e.bias_bs = c->cond_rows_out;
       e.lens_x = lens; e.has_lens_x = lens != nullptr;
-      TRY(launch_tc(r, c->tc_pre, bufA, bufE, nullptr, Tmax, 1, 1.f, 1.f, 0, 0, e));
+      TRY(launch_tc(r, c->tc_pre, bufA, bufE, nullptr, Tmax, 1, e));
       TRY(tap_cl("dec.pre", bufE, 512, Tmax, P));
     } else {
       TRY(launch_transpose(r, ws + W.dpre, bufE, 512, P));
@@ -1297,59 +1305,12 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
       const int cout = cin / 2, up_out = up * s;
       const int Tlen = Tmax * up_out, pitch_out = P * up_out;
       char nm[32];
-      TRY(launch_tc(r, c->tc_ups[i], stage_in, bufA, nullptr, Tmax * up, up, 0.1f, 1.f, 0, 2));
+      TcOpt u;
+      u.slope = 0.1f; u.family = 2;
+      TRY(launch_tc(r, c->tc_ups[i], stage_in, bufA, nullptr, Tmax * up, up, u));
       snprintf(nm, sizeof nm, "dec.ups%d", i);
       TRY(tap_cl(nm, bufA, cout, Tlen, pitch_out));
-      if (!par) {
-        for (int j = 0; j < 3; ++j) {
-          bool fused = c->use_pair;
-          for (int d = 0; d < 3; ++d) fused = fused && pair_fits(c->tc_c1[i * 3 + j][d], c->tc_c2[i * 3 + j][d]);
-          if (fused) {
-            // one kernel per conv pair; a pair never runs in place (its tiles read x with a halo), so the running
-            // activation ping-pongs bufA -> bufB -> bufC -> bufD (bufC is free: the intermediate stays on chip)
-            const float* xs[3] = {bufA, bufB, bufC};
-            float* ys[3] = {bufB, bufC, bufD};
-            for (int d = 0; d < 3; ++d)
-              TRY(launch_pair(r, c->tc_c1[i * 3 + j][d], c->tc_c2[i * 3 + j][d], xs[d], ys[d], Tlen, up_out, 0.1f,
-                              (d == 2 && j == 2) ? 1.0f / 3.0f : 1.f, (d == 2 && j > 0) ? 1 : 0));
-            continue;
-          }
-          for (int d = 0; d < 3; ++d) {
-            const float* xin = d == 0 ? bufA : bufB;
-            float* yout = d < 2 ? bufB : bufD;
-            TRY(launch_tc(r, c->tc_c1[i * 3 + j][d], xin, bufC, nullptr, Tlen, up_out, 0.1f, 1.f, 0, 1));
-            TRY(launch_tc(r, c->tc_c2[i * 3 + j][d], bufC, yout, xin, Tlen, up_out, 0.1f,
-                          (d == 2 && j == 2) ? 1.0f / 3.0f : 1.f, (d == 2 && j > 0) ? 1 : 0, 1));
-          }
-        }
-      } else {
-        // a latency-bound call: the three ResBlock branches (models.py:280-285) are independent up to their last conv,
-        // so they run side by side -- branch 0 on the caller's stream, 1 and 2 on side streams, every kernel on a third
-        // of the SMs.  The MRF sum keeps its order (the last conv of branch j waits for that of branch j - 1), so the
-        // result is bit-identical to the sequential schedule.
-        CK(cudaEventRecord(c->br_ev[3], r.st));
-        TcExtra third;
-        third.grid_div = 3;
-        for (int j = 0; j < 3; ++j) {
-          Run rj = r;
-          if (j > 0) {
-            rj.st = c->br_stream[j - 1];
-            CK(cudaStreamWaitEvent(rj.st, c->br_ev[3], 0));
-          }
-          float* Bj = j == 0 ? bufB : ws + W.brB[j - 1];
-          float* Cj = j == 0 ? bufC : ws + W.brC[j - 1];
-          for (int d = 0; d < 3; ++d) {
-            const float* xin = d == 0 ? bufA : Bj;
-            TRY(launch_tc(rj, c->tc_c1[i * 3 + j][d], xin, Cj, nullptr, Tlen, up_out, 0.1f, 1.f, 0, 1, third));
-            if (d == 2 && j > 0) CK(cudaStreamWaitEvent(rj.st, c->br_ev[j - 1], 0));   // xs so far is complete
-            float* yout = d < 2 ? Bj : bufD;
-            TRY(launch_tc(rj, c->tc_c2[i * 3 + j][d], Cj, yout, xin, Tlen, up_out, 0.1f,
-                          (d == 2 && j == 2) ? 1.0f / 3.0f : 1.f, (d == 2 && j > 0) ? 1 : 0, 1, third));
-          }
-          CK(cudaEventRecord(c->br_ev[j], rj.st));
-        }
-        CK(cudaStreamWaitEvent(r.st, c->br_ev[2], 0));   // join (branch 1 is joined through branch 2's wait)
-      }
+      TRY(run_mrf_tc(r, W, ws, i, Tlen, up_out, par));
       snprintf(nm, sizeof nm, "dec.stage%d", i);
       TRY(tap_cl(nm, bufD, cout, Tlen, pitch_out));
       stage_in = bufD;   // the next upsampling consumes xs before that stage's MRF rewrites bufD (stream order)
@@ -1357,11 +1318,10 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
     }
     const int y_len = Tmax * up;
     dim3 grid((y_len + 255) / 256, B);
-    conv_post_cl_kernel<32><<<grid, 256, 0, st>>>(stage_in, 32LL * P * up, c->d_w + c->post_w_off, o_hat, (long long)y_len,
-                                                 y_len, r.glens, Tmax, up);
-    CK(cudaGetLastError());
-    c->launches++;
-    return OVC_OK;
+    return launch_kernel(r, std::nullopt, [&] {
+      conv_post_cl_kernel<32><<<grid, 256, 0, r.st>>>(stage_in, 32LL * P * up, c->d_w + c->post_w_off, o_hat, (long long)y_len,
+                                                      y_len, r.glens, Tmax, up);
+    });
   }
   const float* stage_in = ws + W.dpre;
   int cin = 512, up = 1;
@@ -1370,133 +1330,91 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
     const int cout = cin / 2;
     const int up_out = up * s;
     const int pitch_in = P * up, pitch_out = P * up_out;
-    // leaky_relu(0.1) + ConvTranspose1d (models.py:278-279), polyphase
-    {
-      ConvArgs a{};
-      a.x = stage_in; a.x_bs = (long long)cin * pitch_in; a.x_pitch = pitch_in;
-      a.bias = c->d_w + c->dec_ups[i].b_off; a.bias_bs = 0;
-      a.y = bufA; a.y_bs = (long long)cout * pitch_out; a.y_pitch = pitch_out;
-      a.lens_in = r.glens; a.lens_out = r.glens; a.mul_in = up; a.mul_out = up;   // kernel time axis = input samples
-      a.slope = 0.1f;
-      TRY(launch(r, c->dec_ups[i], a, Tmax * up));
-      char nm[32]; snprintf(nm, sizeof nm, "dec.ups%d", i);
-      TRY(tap(r, nm, bufA, cout, Tmax * up_out, pitch_out));
-    }
+    // leaky_relu(0.1) + ConvTranspose1d (models.py:278-279), polyphase; kernel time axis = input samples
+    TRY(launch(r, c->dec_ups[i], conv_args(stage_in, cin, pitch_in, bufA, cout, pitch_out, r.glens, up, 0.1f), Tmax * up));
+    char nm[32]; snprintf(nm, sizeof nm, "dec.ups%d", i);
+    TRY(tap(r, nm, bufA, cout, Tmax * up_out, pitch_out));
     // MRF: xs = sum_j ResBlock1_j(x) / 3 (models.py:280-286; ResBlock1 = modules.py:296-309)
-    const long long bsC = (long long)cout * pitch_out;
     const int Tlen = Tmax * up_out;
     for (int j = 0; j < 3; ++j) {
-      const int K = c->hp.resblock_kernel_sizes[j];
       for (int d = 0; d < 3; ++d) {
-        const double fl = 2.0 * cout * cout * K * r.sum_len * up_out;
-        const double by = 2.0 * cout * r.sum_len * up_out * 4.0;
         const float* xin = d == 0 ? bufA : bufB;
-        ConvArgs a{};
-        a.x = xin; a.x_bs = bsC; a.x_pitch = pitch_out;
-        a.bias = c->d_w + c->rb_c1[i * 3 + j][d].b_off; a.bias_bs = 0;
-        a.y = bufC; a.y_bs = bsC; a.y_pitch = pitch_out;
-        a.lens_in = r.glens; a.lens_out = r.glens; a.mul_in = up_out; a.mul_out = up_out;
-        a.slope = 0.1f; a.scale = 1.f;
-        TRY(launch(r, c->rb_c1[i * 3 + j][d], a, Tlen, true, fl, by));
-        ConvArgs b{};
-        b.x = bufC; b.x_bs = bsC; b.x_pitch = pitch_out;
-        b.bias = c->d_w + c->rb_c2[i * 3 + j][d].b_off; b.bias_bs = 0;
-        b.r = xin; b.r_bs = bsC; b.r_pitch = pitch_out;
-        b.lens_in = r.glens; b.lens_out = r.glens; b.mul_in = up_out; b.mul_out = up_out;
-        b.slope = 0.1f; b.scale = 1.f;
-        if (d < 2) {
-          b.y = bufB; b.y_bs = bsC; b.y_pitch = pitch_out;
-        } else {
-          b.y = bufD; b.y_bs = bsC; b.y_pitch = pitch_out;
-          if (j > 0) b.flags = F_ACCUM;
-          if (j == 2) b.scale = 1.0f / 3.0f;   // xs / num_kernels (models.py:286), as a multiply
-        }
-        TRY(launch(r, c->rb_c2[i * 3 + j][d], b, Tlen, true, fl, by));
+        TRY(launch(r, c->rb_c1[i * 3 + j][d], conv_args(xin, cout, pitch_out, bufC, cout, pitch_out, r.glens, up_out, 0.1f), Tlen, true));
+        ConvArgs b = conv_args(bufC, cout, pitch_out, d < 2 ? bufB : bufD, cout, pitch_out, r.glens, up_out, 0.1f);
+        b.r = xin; b.r_bs = b.x_bs; b.r_pitch = pitch_out;
+        if (d == 2 && j > 0) b.flags = F_ACCUM;
+        if (d == 2 && j == 2) b.scale = 1.0f / 3.0f;   // xs / num_kernels (models.py:286), as a multiply
+        TRY(launch(r, c->rb_c2[i * 3 + j][d], b, Tlen, true));
       }
     }
-    char nm[32]; snprintf(nm, sizeof nm, "dec.stage%d", i);
+    snprintf(nm, sizeof nm, "dec.stage%d", i);
     TRY(tap(r, nm, bufD, cout, Tlen, pitch_out));
     stage_in = bufD;
     cin = cout; up = up_out;
   }
   // leaky_relu(0.01) + conv_post + tanh (models.py:287-289)
-  {
-    const int y_len = Tmax * up;   // 256 * Tmax
-    dim3 grid((y_len / 4 + 255) / 256, B);
-    conv_post_kernel<32><<<grid, 256, 0, st>>>(stage_in, 32LL * P * up, P * up, c->d_w + c->post_w_off, o_hat,
-                                              (long long)y_len, y_len, r.glens, Tmax, up);
-    CK(cudaGetLastError());
-    c->launches++;
-  }
-  return OVC_OK;
+  const int y_len = Tmax * up;   // 256 * Tmax
+  dim3 grid((y_len / 4 + 255) / 256, B);
+  return launch_kernel(r, std::nullopt, [&] {
+    conv_post_kernel<32><<<grid, 256, 0, r.st>>>(stage_in, 32LL * P * up, P * up, c->d_w + c->post_w_off, o_hat,
+                                                 (long long)y_len, y_len, r.glens, Tmax, up);
+  });
 }
 
 static int run_vc(ovc_ctx* c, const float* spec, int spec_pitch, const long long* lens, const float* g_src, const float* g_tgt,
                   const float* noise, uint64_t seed, float tau, int B, int Tmax, int ragged, float* o_hat,
                   float* z_out, float* zp_out, float* zh_out, cudaStream_t st) {
   const WsLayout W = ws_layout(c, B, Tmax);
-  TRY(ensure_ws(c, W, B, Tmax, st));
+  TRY(ensure_ws(c, W, st));
   float* ws = c->d_ws;
-  Run r{c, st, B, Tmax, W.P, lens, ragged ? lens : nullptr, (double)B * Tmax};
+  Run r{c, st, B, Tmax, W.P, lens, ragged ? lens : nullptr};
   c->launches = 0;
   const int P = W.P;
-  const long long bs192 = 192LL * P;
 
-  // ---- every speaker-conditioning 1x1 conv in one launch
-  {
-    CondArgs a;
-    a.w = c->d_w + c->cond_w_off; a.bias = c->d_w + c->cond_b_off;
-    a.w_row = c->d_cond_wrow; a.sel = c->d_cond_sel;
-    a.g_src = g_src; a.g_tgt = g_tgt; a.out = ws + W.cond;
-    a.rows_out = c->cond_rows_out; a.gin = c->hp.gin_channels;
-    dim3 grid((c->cond_rows_out + 7) / 8, B);
-    cond_kernel<<<grid, 256, 0, st>>>(a);
-    CK(cudaGetLastError());
-    c->launches++;
-  }
+  TRY(launch_cond(r, g_src, g_tgt, ws + W.cond));
   const float* cond = ws + W.cond;
   TRY(tap(r, "cond", cond, 1, c->cond_rows_out, c->cond_rows_out));
 
   // ---- posterior encoder (models.py:212-221)
-  {
-    ConvArgs a{};
-    a.x = spec; a.x_bs = (long long)c->hp.spec_channels * spec_pitch; a.x_pitch = spec_pitch;
-    a.bias = c->d_w + c->enc_pre.b_off; a.bias_bs = 0;
-    a.y = ws + W.x; a.y_bs = bs192; a.y_pitch = P;
-    a.lens_in = lens; a.lens_out = lens; a.mul_in = 1; a.mul_out = 1;
-    a.slope = 1.f; a.scale = 1.f;
-    const bool aligned = (spec_pitch % 4 == 0) && ((reinterpret_cast<uintptr_t>(spec) & 15) == 0);
-    TRY(launch(r, aligned ? c->enc_pre16 : c->enc_pre, a, Tmax));
-    TRY(tap(r, "enc.pre", ws + W.x, 192, Tmax, P));
-    if (c->precision >= 1) {
-      TRY(run_wn_tc(r, c->enc_wn, ws + W.x, ws + W.skip, ws + W.acts, ws + W.bufA, ws + W.bufB, cond + c->cond_off_enc_tc,
-                    c->cond_rows_out));
-    } else {
-      TRY(run_wn(r, c->enc_wn, ws + W.x, ws + W.skip, ws + W.acts, cond + c->cond_off_enc, c->cond_rows_out));
-    }
-    TRY(tap(r, "enc.wn", ws + W.skip, 192, Tmax, P));
-    ConvArgs p{};
-    p.x = ws + W.skip; p.x_bs = bs192; p.x_pitch = P;
-    p.bias = c->d_w + c->enc_proj.b_off; p.bias_bs = 0;
-    p.y = ws + W.z; p.y_bs = bs192; p.y_pitch = P;
-    p.r = noise; p.r_bs = 192LL * Tmax; p.r_pitch = Tmax;
-    p.lens_in = lens; p.lens_out = lens; p.mul_in = 1; p.mul_out = 1;
-    p.slope = 1.f; p.tau = tau; p.seed = seed;
-    p.callp = c->d_callp;       // set_call_params_kernel wrote (seed, tau) there earlier on this stream
-    TRY(launch(r, c->enc_proj, p, Tmax));
+  const bool aligned = (spec_pitch % 4 == 0) && ((reinterpret_cast<uintptr_t>(spec) & 15) == 0);
+  TRY(launch(r, aligned ? c->enc_pre16 : c->enc_pre, conv_args(spec, c->hp.spec_channels, spec_pitch, ws + W.x, 192, P, lens, 1, 1.f), Tmax));
+  TRY(tap(r, "enc.pre", ws + W.x, 192, Tmax, P));
+  if (c->precision >= 1) {
+    TRY(run_wn_tc(r, c->enc_wn, ws + W.x, ws + W.skip, ws + W.acts, ws + W.bufA, ws + W.bufB, cond + c->cond_off_enc_tc,
+                  c->cond_rows_out));
+  } else {
+    TRY(run_wn(r, c->enc_wn, ws + W.x, ws + W.skip, ws + W.acts, cond + c->cond_off_enc, c->cond_rows_out));
   }
-  auto copy_latent = [&](float* dst) -> int { return copy_latent_out(r, W, ws, dst); };
-  TRY(copy_latent(z_out));
+  TRY(tap(r, "enc.wn", ws + W.skip, 192, Tmax, P));
+  ConvArgs p = conv_args(ws + W.skip, 192, P, ws + W.z, 192, P, lens, 1, 1.f);
+  p.r = noise; p.r_bs = 192LL * Tmax; p.r_pitch = Tmax;
+  p.tau = tau; p.seed = seed;
+  p.callp = c->d_callp;       // set_call_params_kernel wrote (seed, tau) there earlier on this stream
+  TRY(launch(r, c->enc_proj, p, Tmax));
+  TRY(copy_latent_out(r, W, ws, z_out));
   // ---- flow forward with g_src, reverse with g_tgt (models.py:496-497)
   TRY(run_flow(r, W, ws, false, cond));
-  TRY(copy_latent(zp_out));
+  TRY(copy_latent_out(r, W, ws, zp_out));
   TRY(run_flow(r, W, ws, true, cond));
-  TRY(copy_latent(zh_out));
+  TRY(copy_latent_out(r, W, ws, zh_out));
 
   return run_dec(r, W, ws, cond, lens, o_hat);
 }
 
 #include "ovc_tts_run.inc"    // run_tts_encode() / run_tts_decode(): SynthesizerTrn.infer on the device
+
+// what every call entry point checks first: a context with finalized weights, and its tensor arguments
+static int check_call(const ovc_ctx* c, std::initializer_list<const void*> tensors) {
+  if (!c) return fail(OVC_ERR_INVALID, "null context");
+  if (!c->finalized) return fail(OVC_ERR_STATE, "ovc_finalize_weights has not been called");
+  for (const void* t : tensors)
+    if (!t) return fail(OVC_ERR_INVALID, "null tensor argument");
+  return OVC_OK;
+}
+// the generator's widest layer (64 channels x 256 samples per frame) must stay inside 32-bit indexing
+static bool too_many_frames(long long T) { return T * 256 * 64 > 2000000000LL; }
+
+static void prof_reset(ovc_ctx* c) { c->prof_log.clear(); }
 
 }  // namespace ovc
 
@@ -1586,16 +1504,13 @@ size_t ovc_workspace_floats(const ovc_ctx* c, int B, int Tmax) {
 int ovc_voice_conversion(ovc_ctx* c, const float* spec, const int64_t* lengths, const float* g_src, const float* g_tgt,
                          const float* noise, uint64_t seed, float tau, int B, int Tmax, int ragged, float* o_hat, float* z,
                          float* z_p, float* z_hat, void* stream) {
-  if (!c) return fail(OVC_ERR_INVALID, "null context");
-  if (!c->finalized) return fail(OVC_ERR_STATE, "ovc_finalize_weights has not been called");
-  if (!spec || !lengths || !g_src || !g_tgt || !o_hat) return fail(OVC_ERR_INVALID, "null tensor argument");
+  TRY(check_call(c, {spec, lengths, g_src, g_tgt, o_hat}));
   if (B < 1 || Tmax < 1) return fail(OVC_ERR_INVALID, "B and Tmax must be positive (got %d, %d)", B, Tmax);
-  if ((long long)Tmax * 256 * 64 > 2000000000LL) return fail(OVC_ERR_INVALID, "Tmax %d too large for 32-bit indexing", Tmax);
+  if (too_many_frames(Tmax)) return fail(OVC_ERR_INVALID, "Tmax %d too large for 32-bit indexing", Tmax);
   if (B > 65535) return fail(OVC_ERR_INVALID, "B %d exceeds the grid limit", B);
   ON_DEVICE(c);
-  c->ev_used = c->prof ? c->ev_used : 0;
   cudaStream_t st = (cudaStream_t)stream;
-  TRY(ensure_ws(c, ws_layout(c, B, Tmax), B, Tmax, st));
+  TRY(ensure_ws(c, ws_layout(c, B, Tmax), st));
   TRY(set_call_params(c, seed, tau, st));
   const std::vector<uintptr_t> key = {1, (uintptr_t)spec, (uintptr_t)lengths, (uintptr_t)g_src, (uintptr_t)g_tgt, (uintptr_t)noise,
                                       (uintptr_t)o_hat, (uintptr_t)z, (uintptr_t)z_p, (uintptr_t)z_hat, (uintptr_t)B, (uintptr_t)Tmax,
@@ -1619,9 +1534,7 @@ static int launch_stft(ovc_ctx* c, const float* wav, const int64_t* wav_lengths,
 
 int ovc_spectrogram(ovc_ctx* c, const float* wav, const int64_t* wav_lengths, int B, int Lmax, int Tmax, float* spec,
                     int64_t* frames, void* stream) {
-  if (!c) return fail(OVC_ERR_INVALID, "null context");
-  if (!c->finalized) return fail(OVC_ERR_STATE, "ovc_finalize_weights has not been called");
-  if (!wav || !wav_lengths || !spec) return fail(OVC_ERR_INVALID, "null tensor argument");
+  TRY(check_call(c, {wav, wav_lengths, spec}));
   if (B < 1 || Lmax < 1 || Tmax < 1 || B > 65535) return fail(OVC_ERR_INVALID, "bad sizes B=%d Lmax=%d Tmax=%d", B, Lmax, Tmax);
   ON_DEVICE(c);
   return launch_stft(c, wav, wav_lengths, B, Lmax, Tmax, spec, Tmax, (long long*)frames, (cudaStream_t)stream);
@@ -1630,16 +1543,14 @@ int ovc_spectrogram(ovc_ctx* c, const float* wav, const int64_t* wav_lengths, in
 int ovc_convert_waveform(ovc_ctx* c, const float* wav, const int64_t* wav_lengths, int B, int Lmax, const float* g_src,
                          const float* g_tgt, const float* noise, uint64_t seed, float tau, float* o_hat, int64_t* frames,
                          void* stream) {
-  if (!c) return fail(OVC_ERR_INVALID, "null context");
-  if (!c->finalized) return fail(OVC_ERR_STATE, "ovc_finalize_weights has not been called");
-  if (!wav || !wav_lengths || !g_src || !g_tgt || !o_hat) return fail(OVC_ERR_INVALID, "null tensor argument");
+  TRY(check_call(c, {wav, wav_lengths, g_src, g_tgt, o_hat}));
   const int Tmax = Lmax / c->hp.hop_length;
   if (B < 1 || Tmax < 1 || B > 65535) return fail(OVC_ERR_INVALID, "bad sizes B=%d Lmax=%d", B, Lmax);
-  if ((long long)Tmax * 256 * 64 > 2000000000LL) return fail(OVC_ERR_INVALID, "Lmax %d too large for 32-bit indexing", Lmax);
+  if (too_many_frames(Tmax)) return fail(OVC_ERR_INVALID, "Lmax %d too large for 32-bit indexing", Lmax);
   ON_DEVICE(c);
   cudaStream_t st = (cudaStream_t)stream;
   const WsLayout W = ws_layout(c, B, Tmax);
-  TRY(ensure_ws(c, W, B, Tmax, st));
+  TRY(ensure_ws(c, W, st));
   TRY(set_call_params(c, seed, tau, st));
   const std::vector<uintptr_t> key = {2, (uintptr_t)wav, (uintptr_t)wav_lengths, (uintptr_t)g_src, (uintptr_t)g_tgt, (uintptr_t)noise,
                                       (uintptr_t)o_hat, (uintptr_t)frames, (uintptr_t)B, (uintptr_t)Lmax, option_bits(c)};
@@ -1655,8 +1566,7 @@ int ovc_convert_waveform(ovc_ctx* c, const float* wav, const int64_t* wav_length
 }
 
 int ovc_reference_encoder(ovc_ctx* c, const float* spec, int N, int T, float* out, void* stream) {
-  if (!c) return fail(OVC_ERR_INVALID, "null context");
-  if (!c->finalized) return fail(OVC_ERR_STATE, "ovc_finalize_weights has not been called");
+  TRY(check_call(c, {}));
   if (!c->has_refenc) return fail(OVC_ERR_MISSING, "the checkpoint had no ref_enc.* tensors");
   if (!spec || !out || N < 1 || T < 1) return fail(OVC_ERR_INVALID, "bad argument to ovc_reference_encoder");
   ON_DEVICE(c);
@@ -1674,13 +1584,7 @@ int ovc_reference_encoder(ovc_ctx* c, const float* spec, int N, int T, float* ou
     return fail(OVC_ERR_INVALID, "ref_enc.gru.weight_ih_l0 takes %d inputs but spec_channels %d gives %d", c->re_gru_in, F, 128 * W[6]);
   const size_t gi_floats = (size_t)N * H[6] * 384;
   const size_t need = 2 * round_up(maxact, 64) + round_up(gi_floats, 64);
-  if (need > c->re_floats) {
-    CK(cudaStreamSynchronize(st));
-    if (c->d_re) CK(cudaFree(c->d_re));
-    c->d_re = nullptr; c->re_floats = 0;
-    CK(cudaMalloc(&c->d_re, need * sizeof(float)));
-    c->re_floats = need;
-  }
+  TRY(grow_arena(c->d_re, c->re_floats, need, st, "reference-encoder scratch"));
   float* a0 = c->d_re;
   float* a1 = a0 + round_up(maxact, 64);
   float* gi = a1 + round_up(maxact, 64);
@@ -1720,15 +1624,13 @@ int ovc_tts_info(const ovc_ctx* c, int32_t* out8) {
 int ovc_tts_encode(ovc_ctx* c, const int64_t* tokens, const int64_t* x_lengths, const int64_t* sid, const float* noise_w,
                    uint64_t seed, float noise_scale_w, float length_scale, float sdp_ratio, int B, int T, int64_t* y_lengths,
                    float* w_ceil, float* logw, void* stream) {
-  if (!c) return fail(OVC_ERR_INVALID, "null context");
-  if (!c->finalized) return fail(OVC_ERR_STATE, "ovc_finalize_weights has not been called");
+  TRY(check_call(c, {}));
   if (!c->tts.ready) return fail(OVC_ERR_STATE, "the checkpoint has no TTS members (enc_p / dp / sdp / emb_g): not a V1 base speaker");
   if (!tokens || !x_lengths || !sid || !y_lengths) return fail(OVC_ERR_INVALID, "null tensor argument");
   if (B < 1 || T < 1) return fail(OVC_ERR_INVALID, "B and T must be positive (got %d, %d)", B, T);
   if (B > 65535 || (long long)T * T > 2000000000LL / 256) return fail(OVC_ERR_INVALID, "B %d / T %d exceed the grid limits", B, T);
   if (!(length_scale > 0.f)) return fail(OVC_ERR_INVALID, "length_scale must be positive");
   ON_DEVICE(c);
-  c->ev_used = c->prof ? c->ev_used : 0;
   return run_tts_encode(c, (const long long*)tokens, (const long long*)x_lengths, (const long long*)sid, noise_w, seed,
                         noise_scale_w, length_scale, sdp_ratio, B, T, (long long*)y_lengths, w_ceil, logw, (cudaStream_t)stream);
 }
@@ -1741,9 +1643,8 @@ int ovc_tts_decode(ovc_ctx* c, const float* noise, uint64_t seed, float noise_sc
   if (B != c->tts_B) return fail(OVC_ERR_INVALID, "B = %d but the pending ovc_tts_encode had B = %d", B, c->tts_B);
   if (!o) return fail(OVC_ERR_INVALID, "null tensor argument");
   if (Ymax < 1) return fail(OVC_ERR_INVALID, "Ymax must be positive");
-  if ((long long)Ymax * 256 * 64 > 2000000000LL) return fail(OVC_ERR_INVALID, "Ymax %d too large for 32-bit indexing", Ymax);
+  if (too_many_frames(Ymax)) return fail(OVC_ERR_INVALID, "Ymax %d too large for 32-bit indexing", Ymax);
   ON_DEVICE(c);
-  c->ev_used = c->prof ? c->ev_used : 0;
   if (max_len < 0) return fail(OVC_ERR_INVALID, "max_len must be >= 0 (0 = no limit)");
   return run_tts_decode(c, noise, seed, noise_scale, B, Ymax, max_len, ragged, o, z, z_p, (cudaStream_t)stream);
 }
@@ -1783,12 +1684,7 @@ int ovc_graph_replays(const ovc_ctx* c) { return c ? c->graph_replays : 0; }
 int ovc_profile_enable(ovc_ctx* c, int enable) {
   if (!c) return fail(OVC_ERR_INVALID, "null context");
   c->prof = enable != 0;
-  c->ev_used = 0;
-  c->ev_flops.clear();
-  c->ev_bytes.clear();
-  c->ev_variant.clear();
-  c->ev_family.clear();
-  c->ev_tag.clear();
+  prof_reset(c);
   return OVC_OK;
 }
 
@@ -1796,44 +1692,41 @@ int ovc_profile_read(ovc_ctx* c, double* ms, int64_t* launches, double* flops, d
   if (!c) return fail(OVC_ERR_INVALID, "null context");
   double tms = 0, tf = 0, tb = 0;
   int64_t n = 0;
-  for (size_t i = 0; i + 1 < c->ev_used; i += 2) {
-    if (!c->ev_family[i / 2]) continue;
+  for (size_t k = 0; k < c->prof_log.size(); ++k) {
+    const ProfRec& p = c->prof_log[k];
+    if (!p.family) continue;
     float m = 0;
-    CK(cudaEventElapsedTime(&m, c->ev[i], c->ev[i + 1]));
+    CK(cudaEventElapsedTime(&m, c->ev[2 * k], c->ev[2 * k + 1]));
     tms += m;
-    tf += c->ev_flops[i / 2];
-    tb += c->ev_bytes[i / 2];
+    tf += p.flops;
+    tb += p.bytes;
     ++n;
   }
   if (ms) *ms = tms;
   if (launches) *launches = n;
   if (flops) *flops = tf;
   if (bytes) *bytes = tb;
-  c->ev_used = 0;
-  c->ev_flops.clear();
-  c->ev_bytes.clear();
-  c->ev_variant.clear();
-  c->ev_family.clear();
-  c->ev_tag.clear();
+  prof_reset(c);
   return OVC_OK;
 }
 
 int ovc_profile_detail(ovc_ctx* c, int max, char* names /* max x 16 */, double* ms, double* flops, double* bytes, int* family) {
   if (!c) return fail(OVC_ERR_INVALID, "null context");
   int n = 0;
-  for (size_t i = 0; i + 1 < c->ev_used && n < max; i += 2, ++n) {
+  for (; n < (int)c->prof_log.size() && n < max; ++n) {
+    const ProfRec& p = c->prof_log[n];
     float m = 0;
-    CK(cudaEventElapsedTime(&m, c->ev[i], c->ev[i + 1]));
+    CK(cudaEventElapsedTime(&m, c->ev[2 * n], c->ev[2 * n + 1]));
     if (names) {
-      const int tag = c->ev_tag[i / 2], v = c->ev_variant[i / 2];
+      const int tag = p.tag, v = p.variant;
       if (tag && (v == V_TCPAIR64 || v == V_TCPAIR32)) snprintf(names + 16 * n, 16, "P%dk%dd%d", tag >> 16, (tag >> 8) & 255, tag & 255);
       else if (tag) snprintf(names + 16 * n, 16, "T%dc%dk%dd%d", v == V_TC128 ? 128 : v == V_TC64 ? 64 : 32, tag >> 16, (tag >> 8) & 255, tag & 255);
       else { strncpy(names + 16 * n, variant_name(v), 15); names[16 * n + 15] = 0; }
     }
     if (ms) ms[n] = m;
-    if (flops) flops[n] = c->ev_flops[i / 2];
-    if (bytes) bytes[n] = c->ev_bytes[i / 2];
-    if (family) family[n] = c->ev_family[i / 2];
+    if (flops) flops[n] = p.flops;
+    if (bytes) bytes[n] = p.bytes;
+    if (family) family[n] = p.family;
   }
   return n;
 }
