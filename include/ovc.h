@@ -25,7 +25,8 @@
 extern "C" {
 #endif
 
-#define OVC_ABI_VERSION 2   /* 2: ovc_graph_replays, OVC_OPT_PDL .. OVC_OPT_PAIR */
+#define OVC_ABI_VERSION 3   /* 2: ovc_graph_replays, OVC_OPT_PDL .. OVC_OPT_PAIR; 3: OVC_OPT_ACT_TMA, OVC_OPT_TUNE and
+                             * OVC_OPT_WIDE_VARIANT 1 retired (ovc_set_option refuses them) */
 
 #if defined(__GNUC__)
 #define OVC_API __attribute__((visibility("default")))
@@ -179,24 +180,20 @@ OVC_API int ovc_set_precision(ovc_ctx* ctx, int mode);
 
 /* Tuning / diagnostics switches (never change results beyond fp32 reordering):
  *   OVC_OPT_WIDE_VARIANT  kernel of the 128-column tensor-core layers: 0 the persistent kernel (one CTA per SM,
- *                         TMA-staged activations, overlapped epilogue); 1: one 256-step tile per CTA; 2: one 128-step
- *                         tile per CTA, two CTAs per SM; 3 (default): 2 for k >= 7 at Cin >= 256, else 0
+ *                         TMA-staged activations, overlapped epilogue); 2: one 128-step tile per CTA, two CTAs per SM;
+ *                         3 (default): 2 for k >= 7 at Cin >= 256, else 0.  (1, 256-step tiles, is retired.)
  *   OVC_OPT_TTS_SIMPLE    1: one-thread-per-element text-side kernels (the CPU-checked element functions) instead of
  *                         the warp-cooperative LayerNorm / fused attention
- *   OVC_OPT_ACT_TMA       1 (default): the persistent conv kernel receives its activation tiles by tensor-map TMA;
- *                         0: its converter warps load them from global memory
  *   OVC_OPT_GRAPH         1 (default): replay the launch sequence of a repeated (shape, buffers) call from a CUDA graph
  *   OVC_OPT_PDL           programmatic stream serialization of the tensor-core conv launches (the prologue of kernel n+1 --
  *                         barriers, TMEM, weight TMA -- overlaps the drain of kernel n): 0 off, 1 all of them, 2 (default)
  *                         the WaveNet stacks only.  Measured on a B200: 2 saves 0.5-0.8 % at batch 32 and 2.4 % at batch 1;
- *                         1 costs 3 % at batch 32 */
+ *                         1 costs 3 % at batch 32
+ * Keys 4 (OVC_OPT_ACT_TMA) and 6 (OVC_OPT_TUNE) are retired: ovc_set_option returns OVC_ERR_INVALID for them. */
 #define OVC_OPT_WIDE_VARIANT 1
 #define OVC_OPT_TTS_SIMPLE 2
 #define OVC_OPT_GRAPH 3
-#define OVC_OPT_ACT_TMA 4
 #define OVC_OPT_PDL 5
-#define OVC_OPT_TUNE 6       /* A/B bits of the persistent conv kernel: 1 = L2 prefetch of the residual tile (default off),
-                              * 2 = two items per converter iteration (default on) */
 #define OVC_OPT_BRANCHES 7   /* 1 (default): latency-bound calls (B * Tmax <= 512 frames) run the three ResBlock branches of an
                               * MRF stage concurrently (three streams, a third of the SMs per kernel); results are bit-identical */
 #define OVC_OPT_PAIR 8       /* 1 (default): the HBM-bound ResBlock conv pairs (C <= 64, k = 3) run as ONE kernel each

@@ -13,7 +13,7 @@ from typing import Dict, Iterable, Optional, Tuple
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libovc_b200.so")
 
-ABI_VERSION = 2
+ABI_VERSION = 3
 EXPORTS = (
     "ovc_abi_version", "ovc_last_error", "ovc_create", "ovc_destroy", "ovc_load_tensor",
     "ovc_finalize_weights", "ovc_workspace_floats", "ovc_voice_conversion", "ovc_last_launch_count",
@@ -155,8 +155,6 @@ class NativeConverter:
         self.finalized = False
         if os.environ.get("OVC_WIDE_VARIANT"):      # tuning experiments: kernel of the 128-column tensor-core layers
             self.set_option("wide_variant", int(os.environ["OVC_WIDE_VARIANT"]))
-        if os.environ.get("OVC_ACT_TMA"):
-            self.set_option("act_tma", int(os.environ["OVC_ACT_TMA"]))
 
     def close(self):
         if getattr(self, "handle", None):
@@ -197,8 +195,8 @@ class NativeConverter:
         self.precision = mode
 
     def set_option(self, key: str, value: int):
-        """Tuning switches of include/ovc.h: 'wide_variant' (0..3), 'tts_simple', 'graph', 'act_tma', 'pdl' (0/1/2), 'tune' (bits), 'branches', 'pair' (0/1)."""
-        k = {"wide_variant": 1, "tts_simple": 2, "graph": 3, "act_tma": 4, "pdl": 5, "tune": 6, "branches": 7, "pair": 8}[key]
+        """Tuning switches of include/ovc.h: 'wide_variant' (0/2/3), 'tts_simple', 'graph', 'pdl' (0/1/2), 'branches', 'pair' (0/1)."""
+        k = {"wide_variant": 1, "tts_simple": 2, "graph": 3, "pdl": 5, "branches": 7, "pair": 8}[key]
         _check(self.lib, self.lib.ovc_set_option(self.handle, k, int(value)), "ovc_set_option")
 
     # ---- hot path --------------------------------------------------------------------------

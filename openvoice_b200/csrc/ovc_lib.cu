@@ -205,13 +205,11 @@ struct ovc_ctx {
   std::vector<float> h_tcw;
   int precision = 0;           // 0: fp32 FFMA everywhere; 1: 3xFP16 split-precision tcgen05 convs; 2: single-pass fp16
   int wide_variant = 3;        // kernel of the 128-column tensor-core layers (see launch_tc); 3 = chosen per layer
-  bool act_tma = true;         // OVC_OPT_ACT_TMA
   bool tts_simple = false;     // OVC_OPT_TTS_SIMPLE
   bool use_graph = true;       // OVC_OPT_GRAPH
   int use_pdl = 2;             // OVC_OPT_PDL: 0 off, 1 every tensor-core conv, 2 (default) the WaveNet stacks only -- short kernels
                                // whose fill / drain dominates (measured: 2 gives -0.5 .. -0.8 % at batch 32 and -2.4 % at
                                // batch 1; 1 gives +3 % at batch 32)
-  int tune = 2;                // OVC_OPT_TUNE (TcConvArgs.tune)
   // small calls: the three ResBlock branches of an MRF stage run concurrently on three streams, each kernel on a third
   // of the SMs (OVC_OPT_BRANCHES; taken when B * Tmax <= par_frames = 512 frames: measured -8 % at 258 frames, +2 % at 861)
   bool use_branches = true;
@@ -702,8 +700,7 @@ static int finalize(ovc_ctx* c) {
   CK(cudaMemcpy(c->d_tcw, c->h_tcw.data(), c->h_tcw.size() * sizeof(float), cudaMemcpyHostToDevice));
   c->h_tcw.clear();
   c->h_tcw.shrink_to_fit();
-  CK(cudaFuncSetAttribute(tcconv_wide_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcwCfg<1>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_wide_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcwCfg<2>::SMEM_BYTES));
+  CK(cudaFuncSetAttribute(tcconv_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcwCfg::SMEM_BYTES));
   CK(cudaFuncSetAttribute(tcconv_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<128>::SMEM_BYTES));
   CK(cudaFuncSetAttribute(tcconv_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<64>::SMEM_BYTES));
   CK(cudaFuncSetAttribute(tcconv_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<32>::SMEM_BYTES));
@@ -932,7 +929,6 @@ static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const f
   a.Cin = T.Cin; a.Ntot = T.Ntot; a.K = T.K; a.DIL = T.DIL;
   a.slope = o.slope; a.scale = o.scale; a.accumulate = o.accumulate;
   a.passes = r.c->precision == 2 ? 1 : 3;
-  a.tune = r.c->tune;
   if (T.TN == 0) return fail(OVC_ERR_INVALID, "conv %d -> %d (k %d, dilation %d) does not fit the tensor-core kernels", T.Cin, T.Ntot, T.K, T.DIL);
   if (!(o.slope >= 0.f && o.slope <= 1.f)) return fail(OVC_ERR_INVALID, "leaky_relu slope %g outside [0, 1]", (double)o.slope);
   const double units = (double)r.B * t_len;
@@ -944,31 +940,23 @@ static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const f
   // second CTA fills the tensor pipe while the first waits on a barrier; everything else on the persistent kernel
   int wv = r.c->wide_variant;
   if (wv == 3) wv = (T.K >= 7 && T.Cin >= 256) ? 2 : 0;
-  if (T.TN == 128 && wv != 0) {
-    // A/B alternatives of the 128-column layers: 1 = 256-step tiles, one CTA per SM; 2 = 128-step tiles, two CTAs per SM
-    const int MT = wv == 1 ? 2 : 1;
-    dim3 grid((t_len + MT * 128 - 1) / (MT * 128), T.Ntot / 128, r.B);
-    return launch_kernel(r, rec, [&] {
-      return wv == 1 ? launch_ex(tcconv_wide_kernel<2>, grid, TcwCfg<2>::THREADS, TcwCfg<2>::SMEM_BYTES, r.st, pdl, a)
-                     : launch_ex(tcconv_wide_kernel<1>, grid, TcwCfg<1>::THREADS, TcwCfg<1>::SMEM_BYTES, r.st, pdl, a);
-    });
+  if (T.TN == 128 && wv == 2) {
+    // 128-step tiles, two CTAs per SM
+    dim3 grid((t_len + 127) / 128, T.Ntot / 128, r.B);
+    return launch_kernel(r, rec, [&] { return launch_ex(tcconv_wide_kernel, grid, TcwCfg::THREADS, TcwCfg::SMEM_BYTES, r.st, pdl, a); });
   }
   // persistent: one CTA per SM walks the (utterance, tile) list; column tiles (if any) on grid.y
   const int MT = T.TN == 128 ? TcnCfg<128>::MT : TcnCfg<64>::MT;
   const int steps = MT * 128;
   const int n_tt = (t_len + steps - 1) / steps, total = n_tt * r.B;
+  if (!encode_tiled_fn()) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled is not available");
+  const int rows = tcn_rows(MT, (T.K - 1) / 2 * T.DIL);
+  a.n_box = rows > 256 ? 2 : 1;
+  a.box_rows = rows / a.n_box;
   CUtensorMap tmap;
-  memset(&tmap, 0, sizeof tmap);
-  a.act_tma = 0;
-  if (r.c->act_tma && encode_tiled_fn()) {
-    const int rows = tcn_rows(MT, (T.K - 1) / 2 * T.DIL);
-    a.n_box = rows > 256 ? 2 : 1;
-    a.box_rows = rows / a.n_box;
-    const CUresult cr = encode_act_map(&tmap, r, x, T.Cin, mul, a.box_rows);
-    if (cr != CUDA_SUCCESS) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a [%d][%d][%d] activation tensor", (int)cr,
-                                        r.B, r.P * mul, T.Cin);
-    a.act_tma = 1;
-  }
+  const CUresult cr = encode_act_map(&tmap, r, x, T.Cin, mul, a.box_rows);
+  if (cr != CUDA_SUCCESS) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a [%d][%d][%d] activation tensor", (int)cr,
+                                      r.B, r.P * mul, T.Cin);
   const int ncol = T.Ntot / T.TN;
   const int per_col = std::max(1, r.c->sm_count / ncol / std::max(1, o.grid_div));
   dim3 pg((unsigned)std::min(total, per_col), ncol, 1);
@@ -1175,7 +1163,8 @@ static int set_call_params(ovc_ctx* c, uint64_t seed, float tau, cudaStream_t st
   return OVC_OK;
 }
 static uintptr_t option_bits(const ovc_ctx* c) {
-  return (uintptr_t)c->precision | ((uintptr_t)c->wide_variant << 4) | ((uintptr_t)c->act_tma << 8) | ((uintptr_t)c->use_pdl << 15) | ((uintptr_t)c->tune << 10) | ((uintptr_t)c->use_branches << 14) | ((uintptr_t)c->use_pair << 17);
+  return (uintptr_t)c->precision | ((uintptr_t)c->wide_variant << 4) | ((uintptr_t)c->use_branches << 14) | ((uintptr_t)c->use_pdl << 15) |
+         ((uintptr_t)c->use_pair << 17);
 }
 
 // Grow a device arena to `need` floats.  Work queued on `st` may still use the old one, so the stream drains first.  A
@@ -1660,17 +1649,18 @@ int ovc_set_option(ovc_ctx* c, int key, int value) {
   if (!c) return fail(OVC_ERR_INVALID, "null context");
   switch (key) {
     case OVC_OPT_WIDE_VARIANT:
-      if (value < 0 || value > 3) return fail(OVC_ERR_INVALID, "wide variant must be 0, 1, 2 or 3");
+      if (value != 0 && value != 2 && value != 3) return fail(OVC_ERR_INVALID, "wide variant must be 0, 2 or 3 (1 is retired)");
       c->wide_variant = value;
       return OVC_OK;
     case OVC_OPT_TTS_SIMPLE: c->tts_simple = value != 0; return OVC_OK;
     case OVC_OPT_GRAPH: c->use_graph = value != 0; return OVC_OK;
-    case OVC_OPT_ACT_TMA: c->act_tma = value != 0; return OVC_OK;
     case OVC_OPT_PDL:
       if (value < 0 || value > 2) return fail(OVC_ERR_INVALID, "pdl must be 0, 1 or 2");
       c->use_pdl = value;
       return OVC_OK;
-    case OVC_OPT_TUNE: c->tune = value; return OVC_OK;
+    case 4:   // activation loads by the converter warps (OVC_OPT_ACT_TMA = 0): retired
+    case 6:   // A/B switches of the persistent conv kernel (OVC_OPT_TUNE): retired
+      return fail(OVC_ERR_INVALID, "option %d is retired", key);
     case OVC_OPT_BRANCHES: c->use_branches = value != 0; return OVC_OK;
     case OVC_OPT_PAIR: c->use_pair = value != 0; return OVC_OK;
     default: return fail(OVC_ERR_INVALID, "unknown option %d", key);

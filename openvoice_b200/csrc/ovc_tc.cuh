@@ -171,6 +171,13 @@ __device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
 // at twice the TF32 rate and move half the operand bytes, at the same 11-bit-per-part precision as 3xTF32.
 constexpr float kLoScale = 2048.f, kLoInv = 1.f / 2048.f;
 
+// two values -> their hi parts and their lo parts
+__device__ __forceinline__ void split_f16x2(float x0, float x1, __half2& hi, __half2& lo) {
+  hi = __floats2half2_rn(x0, x1);
+  const float2 hf = __half22float2(hi);
+  lo = __floats2half2_rn((x0 - hf.x) * kLoScale, (x1 - hf.y) * kLoScale);
+}
+
 // 8 consecutive channels of one row (after the input leaky-relu) -> 16 bytes of hi parts + 16 bytes of lo parts
 __device__ __forceinline__ void split_f16x8(float4 a, float4 b, float slope, uint4& hi, uint4& lo) {
   float x[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
@@ -180,9 +187,8 @@ __device__ __forceinline__ void split_f16x8(float4 a, float4 b, float slope, uin
     float x0 = x[2 * i], x1 = x[2 * i + 1];
     x0 = fmaxf(x0, x0 * slope);   // leaky_relu for 0 <= slope <= 1 (launch_tc checks), bit-identical to the select
     x1 = fmaxf(x1, x1 * slope);
-    const __half2 hh = __floats2half2_rn(x0, x1);
-    const float2 hf = __half22float2(hh);
-    const __half2 ll = __floats2half2_rn((x0 - hf.x) * kLoScale, (x1 - hf.y) * kLoScale);
+    __half2 hh, ll;
+    split_f16x2(x0, x1, hh, ll);
     h[i] = *reinterpret_cast<const uint32_t*>(&hh);
     l[i] = *reinterpret_cast<const uint32_t*>(&ll);
   }

@@ -17,7 +17,7 @@
 // descriptor's start address, so all taps (any dilation) read ONE staged halo tile.  Two kernels:
 //   tcconv_kernel<TN>        TN = 128 / 64 / 32 output columns, persistent: one CTA per SM walks the (utterance, tile)
 //                            list, activations staged by TMA, epilogue of tile i under the MMAs of tile i+1
-//   tcconv_wide_kernel<MT>   TN = 128, one tile set (MT x 128 steps) per CTA (kept as the A/B alternative)
+//   tcconv_wide_kernel       TN = 128, one 128-step tile per CTA, two CTAs per SM (the generator's first stage at k >= 7)
 #pragma once
 #include <cuda.h>   // CUtensorMap (the driver entry point that encodes it is resolved at run time, ovc_lib.cu)
 
@@ -41,10 +41,7 @@ struct TcConvArgs {
   int Cin; int Ntot; int K; int DIL;   // Ntot = output row width (C for a ResBlock conv, stride*Cout for a polyphase transposed conv)
   float slope; float scale; int accumulate;
   int passes;   // 3: split precision (a_hi*b_hi + a_lo*b_hi + a_hi*b_lo); 1: single-pass fp16 (11-bit operands, like cuDNN's TF32 default)
-  int act_tma;  // persistent kernel: 1 = activation chunks arrive by tensor-map TMA (box_rows x 32 channels, n_box boxes per
-  int box_rows; //                    chunk), 0 = the converter warps load them from global memory themselves
-  int n_box;
-  int tune;     // A/B switches (OVC_OPT_TUNE): bit 0 = L2 prefetch of the residual tile, bit 1 = two items per converter iteration
+  int box_rows; int n_box;   // persistent kernel: an activation chunk arrives by tensor-map TMA as n_box boxes of box_rows x 32 channels
 };
 
 // one box of a [B][rows][Cin] fp32 tensor -> shared memory (128-byte swizzle), completion on an mbarrier
@@ -54,11 +51,6 @@ __device__ __forceinline__ void tma_tensor3d_g2s(void* dst, const CUtensorMap* m
           smem_u32(dst)),
       "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar))
       : "memory");
-}
-
-// ask the L2 for `bytes` (multiple of 16) starting at `p`: no destination, no completion -- the loads that follow hit L2
-__device__ __forceinline__ void l2_prefetch_bulk(const void* p, uint32_t bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
 }
 
 // Programmatic dependent launch (launch_tc sets the stream-serialization attribute): the NEXT kernel's CTAs may start
@@ -90,7 +82,7 @@ __device__ __forceinline__ void tc_item(int i, int& row, int& kc) {
 // sectors (the thread-per-row layout moved 16 bytes per sector and spilled).  Operands with DRAM latency -- the
 // residual of a ResBlock conv, the read-modify-write target of the WaveNet res/skip update -- are fetched one block
 // ahead, and those of the first block BEFORE the wait on the accumulator barrier `bar`: they arrive under the MMAs.
-template <int TN, int MT>
+template <int TN>
 __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, int b, int t0, int n0, int lim, int warp, int lane,
                                             int mt_lo, int mt_hi, int c_lo, int c_hi, uint64_t* bar, uint32_t parity) {
   const int lane_base = (warp & 3) * 32;
@@ -235,51 +227,115 @@ __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, i
   }
 }
 
-// one thread issues the MMAs of MMA tiles [mt_lo, mt_hi) for one (k-step, tap) against weight slot b_slot = [b_hi ; b_lo]
-#define OVC_TC_ISSUE_MMAS(ACC)                                                                       \
-  _Pragma("unroll") for (int mt = mt_lo; mt < mt_hi; ++mt) {                                         \
-    const uint64_t ad_hi = a_cur + mt * 128, ad_lo = ad_hi + A_LO16;                                 \
-    const uint32_t d = (ACC) + 2 * mt * TN;                                                          \
-    if (three) {                                                                                     \
-      tc::mma_f16(d, ad_hi, b_slot, idesc2, !first);      /* [main | low] (+)= a_hi * [b_hi ; b_lo]^T */ \
-      tc::mma_f16(d + TN, ad_lo, b_slot, idesc1, true);   /* low += a_lo * b_hi^T */                 \
-    } else {                                                                                         \
-      tc::mma_f16(d, ad_hi, b_slot, idesc1, !first);                                                 \
-    }                                                                                                \
+// The MMAs of one (k-step, tap) of one 128-row MMA tile against weight slot b = [b_hi ; b_lo] (2 x TN rows), the A
+// tile's lo parts a_lo16 16-byte units after its hi parts.  Three passes: [main | low] (+)= a_hi * [b_hi ; b_lo]^T,
+// low += a_lo * b_hi^T; one pass: main (+)= a_hi * b_hi^T.  For one thread: the issuing warp runs its loop converged
+// and calls this under tc::elect_one() (ovc_tc.cuh: a divergent issuer costs a replay sequence per MMA).
+template <int TN>
+__device__ __forceinline__ void tc_mma_step(uint32_t acc, uint64_t a_hi, uint32_t a_lo16, uint64_t b, bool three, bool accumulate) {
+  constexpr uint32_t idesc1 = tc::make_idesc_f16(128, TN), idesc2 = tc::make_idesc_f16(128, 2 * TN);
+  if (three) {
+    tc::mma_f16(acc, a_hi, b, idesc2, accumulate);
+    tc::mma_f16(acc + TN, a_hi + a_lo16, b, idesc1, true);
+  } else {
+    tc::mma_f16(acc, a_hi, b, idesc1, accumulate);
   }
+}
+
+// A raw fp32 stage of rows x 32 channels (row r = step t_first + r), 128-byte swizzled: 16-byte piece c of row r sits
+// at r * 128 + ((c ^ (r & 7)) << 4) -> leaky-relu -> hi/lo operand tile of row pitch ROWS (column block kc of row r at
+// (kc * ROWS + r) * 16, the lo parts after the 4 hi column blocks).  Rows outside [0, lim) become zeros: zero padding,
+// x_mask and the ragged batch in one rule.  Item i = (row i / 4, column block i % 4), NT threads, thread pt.  Two items
+// per iteration: both pairs of shared-memory loads are in flight before the first conversion (one item at a time left
+// the LDS latency exposed: a single warp per scheduler runs this role).
+template <int ROWS, int NT>
+__device__ __forceinline__ void tc_convert_raw(const unsigned char* raw, unsigned char* ah, int pt, int items, int t_first, int lim,
+                                               float slope) {
+  unsigned char* al = ah + 4 * ROWS * 16;
+  auto fetch = [&](int i, float4& v0, float4& v1) {
+    const int row = i >> 2, kc = i & 3;
+    const int t = t_first + row;
+    v0 = make_float4(0.f, 0.f, 0.f, 0.f);
+    v1 = v0;
+    if (i < items && t >= 0 && t < lim) {
+      const unsigned char* rr = raw + row * 128;
+      v0 = *reinterpret_cast<const float4*>(rr + (((2 * kc) ^ (row & 7)) << 4));
+      v1 = *reinterpret_cast<const float4*>(rr + (((2 * kc + 1) ^ (row & 7)) << 4));
+    }
+  };
+  auto emit = [&](int i, const float4& v0, const float4& v1) {
+    if (i >= items) return;
+    const int row = i >> 2, kc = i & 3;
+    uint4 hi, lo;
+    tc::split_f16x8(v0, v1, slope, hi, lo);
+    *reinterpret_cast<uint4*>(ah + (kc * ROWS + row) * 16) = hi;
+    *reinterpret_cast<uint4*>(al + (kc * ROWS + row) * 16) = lo;
+  };
+  for (int i = pt; i < items; i += 2 * NT) {
+    float4 a0, a1, b0, b1;
+    fetch(i, a0, a1);
+    fetch(i + NT, b0, b1);
+    emit(i, a0, a1);
+    emit(i + NT, b0, b1);
+  }
+}
+
+// Tile `tile` of a persistent kernel's (utterance, tile) list, `steps` output steps per tile: utterance b, first step t0,
+// valid steps lim = min(tmax, lens[b]) * mul (lens NULL: tmax * mul) and the input's own limit lim_x (the same from
+// lens_x; lens_x NULL: lim).  A tile with t0 >= lim lies past its utterance's end: every role skips it.
+struct TcTile {
+  int b, t0, lim, lim_x;
+};
+__device__ __forceinline__ TcTile tc_tile(int tile, int n_tt, int steps, const long long* lens, const long long* lens_x, int tmax,
+                                          int mul) {
+  TcTile t;
+  t.b = tile / n_tt;
+  t.t0 = (tile % n_tt) * steps;
+  t.lim = (lens ? (int)min((long long)tmax, lens[t.b]) : tmax) * mul;
+  t.lim_x = lens_x ? (int)min((long long)tmax, lens_x[t.b]) * mul : t.lim;
+  return t;
+}
+
+// n weight slots of SLOT bytes, resident for the whole launch: one thread copies them from `src` into slots [0, n) of
+// `ring` (completion on bars[0, n)) and waits for them.  A CTA whose tiles all lie past their utterances never waits on
+// these copies otherwise, and they must have landed before it exits (its shared memory may go to the next kernel's CTA).
+template <int SLOT>
+__device__ __forceinline__ void tc_load_resident(unsigned char* ring, uint64_t* bars, const void* src, int n) {
+  const unsigned char* s = reinterpret_cast<const unsigned char*>(src);
+  for (int it = 0; it < n; ++it) {
+    mbar_expect_tx(&bars[it], SLOT);
+    tma_bulk_g2s(ring + it * SLOT, s + (size_t)it * SLOT, SLOT, &bars[it]);
+  }
+  for (int it = 0; it < n; ++it) mbar_wait(&bars[it], 0u);
+}
 
 // ---------------------------------------------------------------------------------------------------------
-// tcconv_wide_kernel: TN = 128 output columns, one tile set (MT x 128 steps) per CTA.
-//   MT = 1: 256 TMEM columns and ~109 KB of shared memory per CTA -> TWO CTAs per SM, so one CTA's prologue /
-//           epilogue overlaps the other's MMAs (the layer's weights are re-streamed per 128 steps).
-//   MT = 2: all 512 TMEM columns, one CTA per SM, weights streamed once per 256 steps, serial epilogue.
+// tcconv_wide_kernel: TN = 128 output columns, one 128-step tile per CTA: 256 TMEM columns and ~109 KB of shared
+// memory per CTA -> TWO CTAs per SM, so one CTA's prologue / epilogue overlaps the other's MMAs (the layer's weights
+// are re-streamed per 128 steps).
 // (A 2-CTA-cluster variant that multicast the weight stream was measured in round 2: no faster, and wrong results
 // whenever both CTAs of a cluster were active -- removed.)
-// Warp roles: warp 0 TMA weight producer; warp 1 (and 6 when MT >= 2) one MMA-issuing thread each; warps 2..5
-// A producers (cp.async raw rows RAWD chunks ahead -> lrelu -> hi/lo fp16 split -> operand layout), then epilogue.
+// Warp roles: warp 0 TMA weight producer; warp 1 one MMA-issuing thread; warps 2..5 A producers (cp.async raw rows
+// RAWD chunks ahead -> lrelu -> hi/lo fp16 split -> operand layout), then epilogue.
 // ---------------------------------------------------------------------------------------------------------
-template <int MT_>
 struct TcwCfg {
-  static constexpr int TN = 128, MT = MT_;
+  static constexpr int TN = 128;
   static constexpr int KCH = 16, NKC = KCH / 8, KS = KCH / 16;    // channels per A stage
-  static constexpr int NISS = MT >= 2 ? 2 : 1;                    // MMA-issuing threads
-  static constexpr int THREADS = NISS == 2 ? 224 : 192;
-  static constexpr int ROWS = MT * 128 + 64;                      // staged rows per A buffer (tile + 2*25 halo, padded)
+  static constexpr int THREADS = 192;
+  static constexpr int ROWS = 128 + 64;                           // staged rows per A buffer (tile + 2*25 halo, padded)
   static constexpr int NABUF = 2;                                 // converted A stages
   static constexpr int RAWD = 2, NST = RAWD + 1;                  // raw fp32 landing stages in flight ahead
-  static constexpr int SLOTS = MT == 1 ? 6 : 14;                  // weight ring depth
+  static constexpr int SLOTS = 6;                                 // weight ring depth
   static constexpr int A_BUF_BYTES = 2 * NKC * ROWS * 16;         // [hi|lo][column block][row][8 halfs]
   static constexpr int SLOT_BYTES = 2 * 2 * TN * 16;              // [column block][hi|lo][n][8 halfs]
   static constexpr int RAW_BYTES = ROWS * KCH * 4;
   static constexpr size_t SMEM_BYTES = 512 + NABUF * A_BUF_BYTES + SLOTS * SLOT_BYTES + NST * RAW_BYTES;
-  static constexpr uint32_t TMEM_COLS = 2 * MT * TN;              // main + low-order accumulators
-  static constexpr int MINB = MT == 1 ? 2 : 1;
+  static constexpr uint32_t TMEM_COLS = 2 * TN;                   // main + low-order accumulators
 };
 
-template <int MT>
-__global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_wide_kernel(const TcConvArgs a) {
-  using Cfg = TcwCfg<MT>;
-  constexpr int TN = Cfg::TN, NABUF = Cfg::NABUF, SLOTS = Cfg::SLOTS, ROWS = Cfg::ROWS, NKC = Cfg::NKC, NISS = Cfg::NISS;
+__global__ void __launch_bounds__(TcwCfg::THREADS, 2) tcconv_wide_kernel(const TcConvArgs a) {
+  using Cfg = TcwCfg;
+  constexpr int TN = Cfg::TN, NABUF = Cfg::NABUF, SLOTS = Cfg::SLOTS, ROWS = Cfg::ROWS, NKC = Cfg::NKC;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw);
   uint64_t* a_full = bars, *a_empty = bars + NABUF, *b_full = bars + 2 * NABUF, *b_empty = b_full + SLOTS,
@@ -291,7 +347,7 @@ __global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_
   unsigned char* raw = bring + SLOTS * Cfg::SLOT_BYTES;
 
   const int b = blockIdx.z;
-  const int t0 = blockIdx.x * (MT * 128);
+  const int t0 = blockIdx.x * 128;
   const int n0 = blockIdx.y * TN;
   const int lim = (a.lens ? (int)min((long long)a.tmax, a.lens[b]) : a.tmax) * a.mul;
   const int lim_x = a.has_lens_x ? (int)min((long long)a.tmax, a.lens_x[b]) * a.mul : lim;
@@ -304,9 +360,9 @@ __global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_
   const int n_slots = (a.Cin / 16) * a.K;
 
   if (tid == 0) {
-    for (int i = 0; i < NABUF; ++i) { mbar_init(&a_full[i], 128); mbar_init(&a_empty[i], NISS); }
-    for (int i = 0; i < SLOTS; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], NISS); }
-    mbar_init(acc_full, NISS);
+    for (int i = 0; i < NABUF; ++i) { mbar_init(&a_full[i], 128); mbar_init(&a_empty[i], 1); }
+    for (int i = 0; i < SLOTS; ++i) { mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1); }
+    mbar_init(acc_full, 1);
     fence_mbar_init();
   }
   if (warp == 1) tc::tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
@@ -332,15 +388,13 @@ __global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_
         if (++slot == SLOTS) { slot = 0; phase ^= 1; }
       }
     }
-  } else if (warp == 1 || (NISS == 2 && warp == 6)) {
-    // ------------------------------------------------------------ MMA issuers (one elected thread per warp)
+  } else if (warp == 1) {
+    // ------------------------------------------------------------ MMA issuer (one elected thread)
     // The whole warp runs the loop converged and only the tcgen05 instructions are predicated on elect.sync: the
     // descriptors then live in uniform registers and advance by plain adds (they differ only in their 14-bit
     // start-address field).  [A divergent `if (lane == 0)` around the loop made ptxas wrap every MMA in an
     // ELECT / R2UR / BRA.U.ANY replay sequence: ~60 dependent instructions per MMA pair, 35 % tensor-pipe activity.]
     {
-      const int mt_lo = (warp == 1 ? 0 : MT / NISS), mt_hi = mt_lo + MT / NISS;
-      const uint32_t idesc1 = tc::make_idesc_f16(128, TN), idesc2 = tc::make_idesc_f16(128, 2 * TN);
       constexpr uint32_t LBO_A = ROWS * 16, LBO_B = 2 * TN * 16, SBO = 128;
       constexpr uint32_t A_LO16 = (NKC * ROWS * 16) >> 4;        // hi -> lo inside an A buffer, in 16-byte units
       constexpr uint32_t SLOT16 = Cfg::SLOT_BYTES >> 4;
@@ -361,9 +415,9 @@ __global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_
             mbar_wait(&b_full[slot], bphase);
             tc::fence_after();
             const uint64_t b_slot = b_ring + (uint32_t)slot * SLOT16;
-            // output step (t0 + mt*128 + i) reads staged row (mt*128 + i + tap*DIL): the halo tile starts at t0 - H
+            // output step (t0 + i) reads staged row (i + tap*DIL): the halo tile starts at t0 - H
             if (tc::elect_one()) {
-              OVC_TC_ISSUE_MMAS(tmem_d)
+              tc_mma_step<TN>(tmem_d, a_cur, A_LO16, b_slot, three, !first);
               tc::mma_commit(&b_empty[slot]);       // slot reusable once these MMAs have read it
             }
             __syncwarp();
@@ -382,7 +436,7 @@ __global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_
     // ------------------------------------------------------------ A producers, then epilogue
     const int pt = tid - 64;                                   // 0..127
     const float* xb = a.x + (size_t)b * a.x_bs;
-    const int rows8 = (MT * 128 + 2 * H + 7) & ~7;
+    const int rows8 = (128 + 2 * H + 7) & ~7;
     constexpr int NP = Cfg::KCH / 4;                           // 16-byte pieces per raw row
     const int pieces = rows8 * NP, items = rows8 * NKC;
     // raw fp32 rows land by cp.async (zero-filled outside [0, lim)), fully coalesced, RAWD chunks ahead; piece p of
@@ -427,7 +481,7 @@ __global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_
       mbar_arrive(&a_full[buf]);
     }
     // epilogue: warp w may read TMEM lanes [32*(w%4), +32)
-    tc_epilogue<TN, MT>(a, tmem_d, b, t0, n0, lim, warp, lane, 0, MT, 0, TN, acc_full, 0);
+    tc_epilogue<TN>(a, tmem_d, b, t0, n0, lim, warp, lane, 0, 1, 0, TN, acc_full, 0);
   }
   tc::fence_before();
   __syncthreads();
@@ -439,16 +493,14 @@ __global__ void __launch_bounds__(TcwCfg<MT>::THREADS, TcwCfg<MT>::MINB) tcconv_
 // One CTA per SM loops over tiles (TN = 128: 128 steps, else 256): barriers / TMEM live for the whole launch, the
 // layer's weights stay resident in shared memory when they fit (C = 32: <= 44 KB; C = 64, k = 3: 48 KB; otherwise a
 // ring streams them per tile), and every stage runs ahead across tile boundaries:
-//   warp 15     activation TMA (act_tma): a chunk of a halo tile = rows x 32 channels of the channels-last tensor is
+//   warp 15     activation TMA: a chunk of a halo tile = rows x 32 channels of the channels-last tensor is
 //               ONE tensor-map box (two when it has more than 256 rows): cp.async.bulk.tensor lands it in a raw fp32
 //               stage, 128-byte swizzled, NRAW chunks ahead, rows before the tensor's start zero-filled by the copy
 //               engine -- the copy engine, not registers, holds the bytes in flight (the narrow layers are HBM-bound:
 //               a whole tile must be in flight per SM to cover the latency).  [Measured: one 128-byte bulk copy per
 //               row instead costs ~55 cycles of TMA issue each and caps the kernel at 1.1 TB/s.]
-//   warps 3-6   (2-6 when TN = 128: its second MMA-issuer warp is free) converters: raw stage (or, act_tma = 0, global
-//               memory) -> lrelu -> fp16 hi/lo split -> operand
-//               layout; rows outside the utterance become zeros here (zero padding, x_mask and the ragged batch in
-//               one rule)
+//   warps 3-6   (2-6 when TN = 128: its second MMA-issuer warp is free) converters: raw stage -> lrelu -> fp16 hi/lo
+//               split -> operand layout (tc_convert_raw)
 //   warp 0      weight TMA; warps 1-2 one MMA-issuing thread each (TN = 128: one)
 //   warps 7-14  epilogue of tile i (second TMEM accumulator set) while the MMAs of tile i+1 run
 // The raw stage's 128-byte swizzle and the operand tiles' ROWS = 2 (mod 8) column-block pitch make both sides of
@@ -510,7 +562,7 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
   const int nq = a.Cin / Cfg::KCH;
   const int n_slots = (a.Cin / 16) * a.K;
   const bool resident = n_slots <= RING;
-  const bool act_tma = a.act_tma != 0;
+  const long long* lens_x = a.has_lens_x ? a.lens_x : nullptr;
   constexpr uint32_t BYTES = Cfg::SLOT_BYTES;
 
   if (tid == 0) {
@@ -529,31 +581,18 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
   if (warp != 0) pdl_wait();   // warp 0 only streams the (constant) weights: it may run ahead of the previous kernel's end
 
   // every role walks the same tile sequence
-#define TCN_FOR_TILES                                                                                   \
-  for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {                                        \
-    const int b = tile / n_tt, t0 = (tile % n_tt) * (MT * 128);                                         \
-    const int lim = (a.lens ? (int)min((long long)a.tmax, a.lens[b]) : a.tmax) * a.mul;                 \
-    const int lim_x = a.has_lens_x ? (int)min((long long)a.tmax, a.lens_x[b]) * a.mul : lim;            \
-    (void)lim_x;                                                                                        \
-    if (t0 >= lim) continue;
-
   if (warp == 0) {
     // ------------------------------------------------------------ weights
     if (lane == 0) {
       const unsigned char* wt = reinterpret_cast<const unsigned char*>(a.w) + (size_t)blockIdx.y * n_slots * Cfg::SLOT_BYTES;
       if (resident) {
-        for (int it = 0; it < n_slots; ++it) {
-          mbar_expect_tx(&b_full[it], BYTES);
-          tma_bulk_g2s(bring + it * Cfg::SLOT_BYTES, wt + (size_t)it * Cfg::SLOT_BYTES, BYTES, &b_full[it]);
-        }
-        // a CTA whose tiles all lie past their utterances never waits on these copies: they must have landed before the
-        // CTA can exit (its shared memory may be handed to the next kernel's CTA)
-        for (int it = 0; it < n_slots; ++it) mbar_wait(&b_full[it], 0u);
+        tc_load_resident<Cfg::SLOT_BYTES>(bring, b_full, wt, n_slots);
       } else {
         int slot = 0;
         uint32_t phase = 1;
-        TCN_FOR_TILES
-          (void)b; (void)lim;
+        for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+          const TcTile tl = tc_tile(tile, n_tt, MT * 128, a.lens, lens_x, a.tmax, a.mul);
+          if (tl.t0 >= tl.lim) continue;
           for (int it = 0; it < n_slots; ++it) {
             mbar_wait(&b_empty[slot], phase);
             mbar_expect_tx(&b_full[slot], BYTES);
@@ -565,31 +604,19 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
     }
   } else if (warp == 15) {
     // ------------------------------------------------------------ activation chunks by tensor-map TMA
-    if (lane == 0 && act_tma) {
+    if (lane == 0) {
       int st = 0;
       uint32_t phase = 1;   // the first pass finds every raw stage free
       const uint32_t box_bytes = (uint32_t)a.box_rows * 128u;
-      // the epilogue reads the residual (and the previous output when accumulating) of this tile long after its
-      // activations were requested: when the tile is contiguous in memory (one column tile: Ntot == TN == y_ld), pull it
-      // into L2 now, so that those loads -- few bytes in flight per warp -- pay L2 latency, not DRAM latency
-      const bool pf = (a.tune & 1) && a.epi == 0 && a.Ntot == TN && a.y_ld == TN && (a.r != nullptr || a.accumulate);
-      TCN_FOR_TILES
-        if (pf) {
-          const int rows = min(MT * 128, lim - t0);
-          const size_t off = ((size_t)b * a.y_bs + (size_t)t0 * TN) * sizeof(float);
-          const uint32_t bytes = (uint32_t)rows * TN * 4u;
-          for (uint32_t o = 0; o < bytes; o += 16384u) {
-            const uint32_t n = min(16384u, bytes - o);
-            if (a.r) l2_prefetch_bulk(reinterpret_cast<const char*>(a.r) + off + o, n);
-            if (a.accumulate) l2_prefetch_bulk(reinterpret_cast<const char*>(a.y) + off + o, n);
-          }
-        }
+      for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+        const TcTile tl = tc_tile(tile, n_tt, MT * 128, a.lens, lens_x, a.tmax, a.mul);
+        if (tl.t0 >= tl.lim) continue;
         for (int q = 0; q < nq; ++q) {
           mbar_wait(&raw_empty[st], phase);
           mbar_expect_tx(&raw_full[st], box_bytes * (uint32_t)a.n_box);
           unsigned char* dst = raw + st * Cfg::RAW_STAGE_BYTES;
           for (int i = 0; i < a.n_box; ++i)   // coordinates: channel, row (may be negative: zero-filled), utterance
-            tma_tensor3d_g2s(dst + i * box_bytes, &tmap, q * Cfg::KCH, t0 - H + i * a.box_rows, b, &raw_full[st]);
+            tma_tensor3d_g2s(dst + i * box_bytes, &tmap, q * Cfg::KCH, tl.t0 - H + i * a.box_rows, tl.b, &raw_full[st]);
           if (++st == NRAW) { st = 0; phase ^= 1; }
         }
       }
@@ -597,22 +624,23 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
   } else if (warp == 1 || (NISS == 2 && warp == 2)) {
     // ------------------------------------------------------------ MMA issuers (one elected thread per warp, converged loop)
     {
-      const int mt_lo = (warp - 1) * (MT / NISS), mt_hi = mt_lo + MT / NISS;
-      const uint32_t idesc1 = tc::make_idesc_f16(128, TN), idesc2 = tc::make_idesc_f16(128, 2 * TN);
+      static_assert(MT == NISS, "one MMA tile per issuer");
+      const int mt = warp - 1;
       constexpr uint32_t LBO_A = ROWS * 16, LBO_B = 2 * TN * 16, SBO = 128;
       constexpr uint32_t A_LO16 = (NKC * ROWS * 16) >> 4, SLOT16 = Cfg::SLOT_BYTES >> 4;
-      const uint64_t a_proto = tc::make_desc(0, LBO_A, SBO), b_proto = tc::make_desc(0, LBO_B, SBO);
+      const uint64_t a_proto = tc::make_desc(0, LBO_A, SBO) + mt * 128, b_proto = tc::make_desc(0, LBO_B, SBO);
       const uint64_t b_ring = b_proto + (tc::smem_addr(bring) >> 4);
       const uint32_t dil = (uint32_t)a.DIL;
       const bool three = a.passes == 3;
       int slot = 0, buf = 0, n = 0;
       uint32_t bphase = 0, aphase = 0;
-      TCN_FOR_TILES
-        (void)b; (void)lim;
+      for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+        const TcTile tl = tc_tile(tile, n_tt, MT * 128, a.lens, lens_x, a.tmax, a.mul);
+        if (tl.t0 >= tl.lim) continue;
         const int set = n & 1;
         mbar_wait(&acc_empty[set], ((n >> 1) & 1) ^ 1);   // the epilogue has drained this accumulator set
         tc::fence_after();
-        const uint32_t acc = tmem_d + set * SET_COLS;
+        const uint32_t acc = tmem_d + set * SET_COLS + 2 * mt * TN;
         bool first = true;
         if (resident) slot = 0;
         for (int q = 0; q < nq; ++q) {
@@ -627,7 +655,7 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
               }
               const uint64_t b_slot = b_ring + (uint32_t)slot * SLOT16;
               if (tc::elect_one()) {
-                OVC_TC_ISSUE_MMAS(acc)
+                tc_mma_step<TN>(acc, a_cur, A_LO16, b_slot, three, !first);
                 if (!resident) tc::mma_commit(&b_empty[slot]);
               }
               __syncwarp();
@@ -651,88 +679,19 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
     const int items = rows8 * NKC;            // item i = (row i / 4, column block i % 4): 32 bytes of one row
     int buf = 0, st = 0;
     uint32_t ephase = 1, rphase = 0;
-    TCN_FOR_TILES
-      const float* xb = a.x + (size_t)b * a.x_bs;
+    for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+      const TcTile tl = tc_tile(tile, n_tt, MT * 128, a.lens, lens_x, a.tmax, a.mul);
+      if (tl.t0 >= tl.lim) continue;
       for (int q = 0; q < nq; ++q) {
-        if (act_tma) mbar_wait(&raw_full[st], rphase);
+        mbar_wait(&raw_full[st], rphase);
         mbar_wait(&a_empty[buf], ephase);
-        unsigned char* ah = abuf + buf * Cfg::A_BUF_BYTES;
-        unsigned char* al = ah + NKC * ROWS * 16;
-        if (act_tma) {
-          // raw stage, 128-byte swizzle: 16-byte chunk c of row r sits at r * 128 + ((c ^ (r & 7)) << 4).
-          // Two items per iteration: both pairs of shared-memory loads are in flight before the first conversion
-          // (one item at a time left the LDS latency exposed: a single warp per scheduler runs this role).
-          const unsigned char* rsrc = raw + st * Cfg::RAW_STAGE_BYTES;
-          auto fetch = [&](int i, float4& v0, float4& v1) {
-            const int row = i >> 2, kc = i & 3;
-            const int t = t0 - H + row;
-            v0 = make_float4(0.f, 0.f, 0.f, 0.f);
-            v1 = v0;
-            if (i < items && t >= 0 && t < lim_x) {
-              const unsigned char* rr = rsrc + row * 128;
-              v0 = *reinterpret_cast<const float4*>(rr + (((2 * kc) ^ (row & 7)) << 4));
-              v1 = *reinterpret_cast<const float4*>(rr + (((2 * kc + 1) ^ (row & 7)) << 4));
-            }
-          };
-          auto emit = [&](int i, const float4& v0, const float4& v1) {
-            if (i >= items) return;
-            const int row = i >> 2, kc = i & 3;
-            uint4 hi, lo;
-            tc::split_f16x8(v0, v1, a.slope, hi, lo);
-            *reinterpret_cast<uint4*>(ah + (kc * ROWS + row) * 16) = hi;
-            *reinterpret_cast<uint4*>(al + (kc * ROWS + row) * 16) = lo;
-          };
-          if (a.tune & 2) {
-            for (int i = pt; i < items; i += 2 * NCT) {
-              float4 a0, a1, b0, b1;
-              fetch(i, a0, a1);
-              fetch(i + NCT, b0, b1);
-              emit(i, a0, a1);
-              emit(i + NCT, b0, b1);
-            }
-          } else {
-            for (int i = pt; i < items; i += NCT) {
-              float4 a0, a1;
-              fetch(i, a0, a1);
-              emit(i, a0, a1);
-            }
-          }
-        } else {
-          constexpr int PB = 5;   // items (32 bytes each) in flight per thread
-          for (int i0 = pt; i0 < items; i0 += NCT * PB) {
-            float4 v0[PB], v1[PB];
-#pragma unroll
-            for (int u = 0; u < PB; ++u) {
-              const int i = i0 + NCT * u;
-              const int row = i >> 2, kc = i & 3;
-              const int t = t0 - H + row;
-              v0[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-              v1[u] = v0[u];
-              if (i < items && t >= 0 && t < lim_x) {
-                const float4* src = reinterpret_cast<const float4*>(xb + (size_t)t * a.Cin + q * Cfg::KCH + kc * 8);
-                v0[u] = src[0];
-                v1[u] = src[1];
-              }
-            }
-#pragma unroll
-            for (int u = 0; u < PB; ++u) {
-              const int i = i0 + NCT * u;
-              if (i >= items) break;
-              const int row = i >> 2, kc = i & 3;
-              uint4 hi, lo;
-              tc::split_f16x8(v0[u], v1[u], a.slope, hi, lo);
-              *reinterpret_cast<uint4*>(ah + (kc * ROWS + row) * 16) = hi;
-              *reinterpret_cast<uint4*>(al + (kc * ROWS + row) * 16) = lo;
-            }
-          }
-        }
+        tc_convert_raw<ROWS, NCT>(raw + st * Cfg::RAW_STAGE_BYTES, abuf + buf * Cfg::A_BUF_BYTES, pt, items, tl.t0 - H, tl.lim_x,
+                                  a.slope);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         mbar_arrive(&a_full[buf]);
         if (++buf == NABUF) { buf = 0; ephase ^= 1; }
-        if (act_tma) {
-          mbar_arrive(&raw_empty[st]);          // this thread has read everything it needs from the raw stage
-          if (++st == NRAW) { st = 0; rphase ^= 1; }
-        }
+        mbar_arrive(&raw_empty[st]);          // this thread has read everything it needs from the raw stage
+        if (++st == NRAW) { st = 0; rphase ^= 1; }
       }
     }
   } else if (warp >= 7 && warp <= 14) {
@@ -743,22 +702,22 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
     const int mt_lo = MT == 2 ? half : 0, mt_hi = MT == 2 ? half + 1 : 1;
     const int c_lo = MT == 2 ? 0 : half * (TN / 2), c_hi = MT == 2 ? TN : c_lo + TN / 2;
     int n = 0;
-    TCN_FOR_TILES
+    for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+      const TcTile tl = tc_tile(tile, n_tt, MT * 128, a.lens, lens_x, a.tmax, a.mul);
+      if (tl.t0 >= tl.lim) continue;
       const int set = n & 1;
-      tc_epilogue<TN, MT>(a, tmem_d + set * SET_COLS, b, t0, n0, lim, warp, lane, mt_lo, mt_hi, c_lo, c_hi, &acc_full[set],
-                          (n >> 1) & 1);
+      tc_epilogue<TN>(a, tmem_d + set * SET_COLS, tl.b, tl.t0, n0, tl.lim, warp, lane, mt_lo, mt_hi, c_lo, c_hi, &acc_full[set],
+                      (n >> 1) & 1);
       tc::fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&acc_empty[set]);
       ++n;
     }
   }
-#undef TCN_FOR_TILES
   tc::fence_before();
   __syncthreads();
   if (warp == 1) tc::tmem_dealloc(tmem_d, Cfg::TMEM_COLS);
 }
-#undef OVC_TC_ISSUE_MMAS
 
 // conv_post on channels-last input: y[b, t] = tanh(sum_{k<7, ci<C} w[ci, k] * lrelu_0.01(x[b, t+k-3, ci]))
 // (models.py:287-289).  HBM-bound (132 B per sample): a CTA stages 256+6 rows with coalesced 16-byte loads into a

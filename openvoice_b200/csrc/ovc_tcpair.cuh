@@ -11,9 +11,10 @@
 //
 // Measured on a B200 (32 x 10 s, C = 32 stage, per pair): k = 3 0.84 ms fused vs 0.53 + 0.59 ms as two launches; k = 7
 // 1.24 vs 1.27; k = 11 1.74 vs 1.64 -- the k >= 7 layers are bound by shared-memory operand reads, not by HBM, and pay
-// for the 118 / 128 tile efficiency.  The host therefore fuses the k <= 5 pairs only (launch_pair / pair_fits).  The
-// C = 64 pairs do not fit: their weights (2 x 48 KB at k = 3) cannot stay resident next to the operand tiles, and with
-// streamed weights a 118-step tile re-streams twice the weight bytes per step (measured 2x slower).
+// for the 118 / 128 tile efficiency.  The host therefore fuses the k <= 5 pairs only (launch_pair / pair_fits): at C = 32,
+// and at C = 64 for k = 3, whose weights (2 x 48 KB) stay resident next to the operand tiles with a halo of at most 8
+// steps and ONE A2 buffer (TcpCfg<64>).  Larger C = 64 pairs do not fit, and with streamed weights a 118-step tile
+// re-streams twice the weight bytes per step (measured 2x slower).
 //
 // Tile = 128 conv-1 steps; conv 2 needs H2 = (k-1)/2 steps of t on either side, so a tile yields R = 128 - 2*H2 output
 // steps (k = 11: 118, 8 % of the MMA rows recomputed by the neighbours) and conv 1 reads 128 + 2*H1 steps of x.
@@ -93,7 +94,6 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
   const int rows8 = (128 + 2 * H1 + 7) & ~7;        // staged rows of x per chunk
   const int nq = a.C / Cfg::KCH;
   const int n_slots = (a.C / 16) * a.K;             // weight slots per conv
-  constexpr uint32_t BYTES = Cfg::SLOT_BYTES;
   if (2 * n_slots > RING || H1 > Cfg::HMAX) __trap();   // weights resident, halo inside the staged rows (host: pair_fits)
   const bool three = a.passes == 3;
 
@@ -119,32 +119,12 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
   const uint32_t tmem_d = *tmem_slot;
   const uint32_t acc1_base = tmem_d, acc2_base = tmem_d + 4 * TN;
 
-  // tile -> (utterance, first output step, valid steps); a tile past its utterance's end is skipped by every role
-  auto tile_info = [&](int tile, int& b, int& t0, int& lim) -> bool {
-    b = tile / n_tt;
-    t0 = (tile % n_tt) * R;
-    lim = (a.lens ? (int)min((long long)a.tmax, a.lens[b]) : a.tmax) * a.mul;
-    return t0 < lim;
-  };
-#define TCP_FOR_TILES                                                       \
-  for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {            \
-    int b, t0, lim;                                                         \
-    if (!tile_info(tile, b, t0, lim)) continue;
-
+  // every role walks the same tile sequence: tiles of R output steps (tc_tile)
   if (warp == 0) {
     // ------------------------------------------------------------ weights of both convs
     if (lane == 0) {
-      const unsigned char* w1 = reinterpret_cast<const unsigned char*>(a.w1);
-      const unsigned char* w2 = reinterpret_cast<const unsigned char*>(a.w2);
-      for (int it = 0; it < n_slots; ++it) {
-        mbar_expect_tx(&b_full[it], BYTES);
-        tma_bulk_g2s(bring + it * Cfg::SLOT_BYTES, w1 + (size_t)it * Cfg::SLOT_BYTES, BYTES, &b_full[it]);
-      }
-      for (int it = 0; it < n_slots; ++it) {
-        mbar_expect_tx(&b_full[n_slots + it], BYTES);
-        tma_bulk_g2s(bring + (n_slots + it) * Cfg::SLOT_BYTES, w2 + (size_t)it * Cfg::SLOT_BYTES, BYTES, &b_full[n_slots + it]);
-      }
-      for (int it = 0; it < 2 * n_slots; ++it) mbar_wait(&b_full[it], 0u);   // landed before this CTA may exit
+      tc_load_resident<Cfg::SLOT_BYTES>(bring, b_full, a.w1, n_slots);
+      tc_load_resident<Cfg::SLOT_BYTES>(bring + n_slots * Cfg::SLOT_BYTES, b_full + n_slots, a.w2, n_slots);
     }
   } else if (warp == 15) {
     // ------------------------------------------------------------ x chunks by tensor-map TMA
@@ -152,12 +132,13 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
       int st = 0;
       uint32_t phase = 1;
       const uint32_t box_bytes = (uint32_t)rows8 * 128u;
-      TCP_FOR_TILES
-        (void)lim;
+      for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+        const TcTile tl = tc_tile(tile, n_tt, R, a.lens, nullptr, a.tmax, a.mul);
+        if (tl.t0 >= tl.lim) continue;
         for (int q = 0; q < nq; ++q) {
           mbar_wait(&raw_empty[st], phase);
           mbar_expect_tx(&raw_full[st], box_bytes);
-          tma_tensor3d_g2s(raw + st * Cfg::RAW_STAGE_BYTES, &tmap, q * Cfg::KCH, t0 - H2 - H1, b, &raw_full[st]);
+          tma_tensor3d_g2s(raw + st * Cfg::RAW_STAGE_BYTES, &tmap, q * Cfg::KCH, tl.t0 - H2 - H1, tl.b, &raw_full[st]);
           if (++st == NRAW) { st = 0; phase ^= 1; }
         }
       }
@@ -166,19 +147,20 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
     // ------------------------------------------------------------ MMA issuers (converged warps, elected lane issues):
     // warp 1 issues conv 1, warp 2 conv 2 -- one thread cannot feed the tensor pipe at N <= 64 (an MMA pair lasts 88
     // cycles).  Conv 1 of tile i+1 runs on the tensor pipe while E1 builds the A2 operand of tile i.
-    const uint32_t idesc1 = tc::make_idesc_f16(128, TN), idesc2 = tc::make_idesc_f16(128, 2 * TN);
     constexpr uint32_t LBO1 = ROWS1 * 16, LBO2 = ROWS2 * 16, LBO_B = 2 * TN * 16, SBO = 128;
     constexpr uint32_t A1_LO16 = (4 * ROWS1 * 16) >> 4, A2_LO16 = (NKC2 * ROWS2 * 16) >> 4, SLOT16 = Cfg::SLOT_BYTES >> 4;
     const uint64_t a1_proto = tc::make_desc(0, LBO1, SBO), a2_proto = tc::make_desc(0, LBO2, SBO), b_proto = tc::make_desc(0, LBO_B, SBO);
     const uint64_t b_ring = b_proto + (tc::smem_addr(bring) >> 4);
     const uint32_t dil = (uint32_t)a.DIL1;
-    for (int it = 0; it < 2 * n_slots; ++it) mbar_wait(&b_full[it], 0u);   // resident weights: waited on once
+    const int conv = warp - 1;
+    for (int it = 0; it < n_slots; ++it) mbar_wait(&b_full[conv * n_slots + it], 0u);   // resident weights: waited on once
     tc::fence_after();
     if (warp == 1) {
       int buf1 = 0, n1 = 0;
       uint32_t a1phase = 0;
-      TCP_FOR_TILES
-        (void)b; (void)t0; (void)lim;
+      for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+        const TcTile tl = tc_tile(tile, n_tt, R, a.lens, nullptr, a.tmax, a.mul);
+        if (tl.t0 >= tl.lim) continue;
         const int set = n1 & 1;
         mbar_wait(&acc1_empty[set], ((n1 >> 1) & 1) ^ 1);
         tc::fence_after();
@@ -191,14 +173,7 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
             uint64_t a_cur = a1_proto + ((tc::smem_addr(a1buf + buf1 * Cfg::A1_BYTES) + 2 * j * LBO1) >> 4);
             uint64_t b_slot = b_ring + (uint32_t)((q * 2 + j) * a.K) * SLOT16;
             for (int tap = 0; tap < a.K; ++tap) {
-              if (tc::elect_one()) {
-                if (three) {
-                  tc::mma_f16(acc, a_cur, b_slot, idesc2, !first);
-                  tc::mma_f16(acc + TN, a_cur + A1_LO16, b_slot, idesc1, true);
-                } else {
-                  tc::mma_f16(acc, a_cur, b_slot, idesc1, !first);
-                }
-              }
+              if (tc::elect_one()) tc_mma_step<TN>(acc, a_cur, A1_LO16, b_slot, three, !first);
               __syncwarp();
               first = false;
               a_cur += dil;
@@ -215,8 +190,9 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
       }
     } else {
       int n2 = 0;
-      TCP_FOR_TILES
-        (void)b; (void)t0; (void)lim;
+      for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+        const TcTile tl = tc_tile(tile, n_tt, R, a.lens, nullptr, a.tmax, a.mul);
+        if (tl.t0 >= tl.lim) continue;
         const int set = n2 & 1, buf2 = n2 % NA2;
         mbar_wait(&acc2_empty[set], ((n2 >> 1) & 1) ^ 1);
         mbar_wait(&a2_full[buf2], (n2 / NA2) & 1);
@@ -227,14 +203,7 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
         for (int kk = 0; kk < a.C / 16; ++kk) {
           uint64_t a_cur = a2_proto + ((tc::smem_addr(a2buf + buf2 * Cfg::A2_BYTES) + 2 * kk * LBO2) >> 4);
           for (int tap = 0; tap < a.K; ++tap) {
-            if (tc::elect_one()) {
-              if (three) {
-                tc::mma_f16(acc, a_cur, b_slot, idesc2, !first);
-                tc::mma_f16(acc + TN, a_cur + A2_LO16, b_slot, idesc1, true);
-              } else {
-                tc::mma_f16(acc, a_cur, b_slot, idesc1, !first);
-              }
-            }
+            if (tc::elect_one()) tc_mma_step<TN>(acc, a_cur, A2_LO16, b_slot, three, !first);
             __syncwarp();
             first = false;
             a_cur += 1;             // conv 2 has dilation 1
@@ -255,40 +224,14 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
     const int items = rows8 * 4;
     int buf = 0, st = 0;
     uint32_t ephase = 1, rphase = 0;
-    TCP_FOR_TILES
-      (void)b;
+    for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+      const TcTile tl = tc_tile(tile, n_tt, R, a.lens, nullptr, a.tmax, a.mul);
+      if (tl.t0 >= tl.lim) continue;
       for (int q = 0; q < nq; ++q) {
         mbar_wait(&raw_full[st], rphase);
         mbar_wait(&a1_empty[buf], ephase);
-        unsigned char* ah = a1buf + buf * Cfg::A1_BYTES;
-        unsigned char* al = ah + 4 * ROWS1 * 16;
-        const unsigned char* rsrc = raw + st * Cfg::RAW_STAGE_BYTES;
-        auto fetch = [&](int i, float4& v0, float4& v1) {
-          const int row = i >> 2, kc = i & 3;
-          const int t = t0 - H2 - H1 + row;
-          v0 = make_float4(0.f, 0.f, 0.f, 0.f);
-          v1 = v0;
-          if (i < items && t >= 0 && t < lim) {
-            const unsigned char* rr = rsrc + row * 128;
-            v0 = *reinterpret_cast<const float4*>(rr + (((2 * kc) ^ (row & 7)) << 4));
-            v1 = *reinterpret_cast<const float4*>(rr + (((2 * kc + 1) ^ (row & 7)) << 4));
-          }
-        };
-        auto emit = [&](int i, const float4& v0, const float4& v1) {
-          if (i >= items) return;
-          const int row = i >> 2, kc = i & 3;
-          uint4 hi, lo;
-          tc::split_f16x8(v0, v1, a.slope, hi, lo);
-          *reinterpret_cast<uint4*>(ah + (kc * ROWS1 + row) * 16) = hi;
-          *reinterpret_cast<uint4*>(al + (kc * ROWS1 + row) * 16) = lo;
-        };
-        for (int i = pt; i < items; i += 256) {
-          float4 p0, p1, q0, q1;
-          fetch(i, p0, p1);
-          fetch(i + 128, q0, q1);
-          emit(i, p0, p1);
-          emit(i + 128, q0, q1);
-        }
+        tc_convert_raw<ROWS1, 128>(raw + st * Cfg::RAW_STAGE_BYTES, a1buf + buf * Cfg::A1_BYTES, pt, items, tl.t0 - H2 - H1, tl.lim,
+                                   a.slope);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         mbar_arrive(&a1_full[buf]);
         if (++buf == NA1) { buf = 0; ephase ^= 1; }
@@ -301,8 +244,9 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
     const int lane_base = (warp & 3) * 32;
     const int rsub = lane >> 2, csub = (lane & 3) * 2;
     int n = 0;
-    TCP_FOR_TILES
-      (void)b;
+    for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+      const TcTile tl = tc_tile(tile, n_tt, R, a.lens, nullptr, a.tmax, a.mul);
+      if (tl.t0 >= tl.lim) continue;
       const int set = n & 1, buf2 = n % NA2;
       mbar_wait(&a2_empty[buf2], ((n / NA2) & 1) ^ 1);     // conv 2 of the tile that used this A2 buffer has read it
       mbar_wait(&acc1_full[set], (n >> 1) & 1);
@@ -333,8 +277,8 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
             for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(rm[i]);
           }
           // t lives on steps [0, lim): outside them conv 2 sees zero padding, not conv 1 evaluated on padding
-          const int ta = t0 - H2 + row_a, tb = ta + 8;
-          const bool oka = ta >= 0 && ta < lim, okb = tb >= 0 && tb < lim;
+          const int ta = tl.t0 - H2 + row_a, tb = ta + 8;
+          const bool oka = ta >= 0 && ta < tl.lim, okb = tb >= 0 && tb < tl.lim;
 #pragma unroll
           for (int g = 0; g < 4; ++g) {
             float x0 = v[4 * g] + bq[g].x, x1 = v[4 * g + 1] + bq[g].y, x2 = v[4 * g + 2] + bq[g].x, x3 = v[4 * g + 3] + bq[g].y;
@@ -342,10 +286,9 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
             x1 = oka ? fmaxf(x1, x1 * a.slope) : 0.f;
             x2 = okb ? fmaxf(x2, x2 * a.slope) : 0.f;
             x3 = okb ? fmaxf(x3, x3 * a.slope) : 0.f;
-            const __half2 ha = __floats2half2_rn(x0, x1), hb = __floats2half2_rn(x2, x3);
-            const float2 fa = __half22float2(ha), fb = __half22float2(hb);
-            const __half2 la = __floats2half2_rn((x0 - fa.x) * tc::kLoScale, (x1 - fa.y) * tc::kLoScale);
-            const __half2 lb = __floats2half2_rn((x2 - fb.x) * tc::kLoScale, (x3 - fb.y) * tc::kLoScale);
+            __half2 ha, la, hb, lb;
+            tc::split_f16x2(x0, x1, ha, la);
+            tc::split_f16x2(x2, x3, hb, lb);
             const int kc = (c0 >> 3) + g;
             const int oa = (kc * ROWS2 + row_a) * 16 + (lane & 3) * 4, ob = (kc * ROWS2 + row_b) * 16 + (lane & 3) * 4;
             *reinterpret_cast<__half2*>(a2h + oa) = ha;
@@ -370,17 +313,18 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcpair_kernel(const TcPairArgs
     e.bias = a.bias2; e.bias_bs = 0;
     e.epi = 0; e.accumulate = a.accumulate; e.scale = a.scale; e.passes = a.passes;
     int n = 0;
-    TCP_FOR_TILES
+    for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
+      const TcTile tl = tc_tile(tile, n_tt, R, a.lens, nullptr, a.tmax, a.mul);
+      if (tl.t0 >= tl.lim) continue;
       const int set = n & 1;
-      tc_epilogue<TN, 1>(e, acc2_base + set * 2 * TN, b, t0, 0, min(lim, t0 + R), warp, lane, 0, 1, 0, TN, &acc2_full[set],
-                         (n >> 1) & 1);
+      tc_epilogue<TN>(e, acc2_base + set * 2 * TN, tl.b, tl.t0, 0, min(tl.lim, tl.t0 + R), warp, lane, 0, 1, 0, TN, &acc2_full[set],
+                      (n >> 1) & 1);
       tc::fence_before();
       __syncwarp();
       if (lane == 0) mbar_arrive(&acc2_empty[set]);
       ++n;
     }
   }
-#undef TCP_FOR_TILES
   tc::fence_before();
   __syncthreads();
   if (warp == 1) tc::tmem_dealloc(tmem_d, Cfg::TMEM_COLS);

@@ -155,18 +155,35 @@ def test_graph_replay_is_bit_identical(native):
 def test_fused_conv_pair_equals_two_launches(native):
     """OVC_OPT_PAIR: the fused ResBlock conv-pair kernel of the C = 32 stage (intermediate activation kept in shared memory)
     performs the same arithmetic in the same order as two conv launches: bit-identical audio on a ragged batch whose
-    lengths put tile boundaries, utterance ends and the 118 / 126-step tiling in different places; both tensor-core modes."""
+    lengths put tile boundaries, utterance ends and the 118 / 126-step tiling in different places; both tensor-core modes.
+    The batch is small enough for the concurrent-branch schedule, which never fuses: the sequential one is forced."""
+    import re
+    nat = native.native
     spec, lengths, gs, gt, noise = O.synthetic_inputs(3, 131, 17, lengths=[131, 64, 7])
     outs = {}
-    for mode in ("f16x3", "f16"):
-        native.native.set_precision(mode)
-        for pair in (0, 1):
-            native.native.set_option("pair", pair)
-            o, _, _ = run_native(native, spec, lengths, gs, gt, noise, 0.3, ragged=True)
-            outs[(mode, pair)] = o
-        assert torch.equal(outs[(mode, 0)], outs[(mode, 1)]), mode
-    native.native.set_precision("f16x3")
-    native.native.set_option("pair", 1)
+    nat.set_option("branches", 0)
+    try:
+        for mode in ("f16x3", "f16"):
+            nat.set_precision(mode)
+            for pair in (0, 1):
+                nat.set_option("pair", pair)
+                o, _, _ = run_native(native, spec, lengths, gs, gt, noise, 0.3, ragged=True)
+                outs[(mode, pair)] = o
+            assert torch.equal(outs[(mode, 0)], outs[(mode, 1)]), mode
+        pairs = {}
+        for pair in (0, 1):                       # what ran: the profile names of the pair kernel, P<C>k<k>d<d>
+            nat.set_option("pair", pair)
+            nat.profile_enable(True)
+            try:
+                run_native(native, spec, lengths, gs, gt, noise, 0.3, ragged=True)
+                pairs[pair] = {int(m[1]) for m in (re.fullmatch(r"P(\d+)k\d+d\d+", r[0]) for r in nat.profile_detail()) if m}
+            finally:
+                nat.profile_enable(False)
+        assert 32 in pairs[1] and not pairs[0], pairs
+    finally:
+        nat.set_option("branches", 1)
+        nat.set_precision("f16x3")
+        nat.set_option("pair", 1)
 
 
 def test_flow_roundtrip_property_full_size(native):

@@ -2,7 +2,7 @@
 """Same-box A/B of the tuning switches (ovc_set_option): whole-call device time of convert_waveform, CUDA events,
 settings interleaved round-robin so that clock / thermal drift hits all of them alike.
 
-  python tools/ab_bench.py --batch 32 --secs 10 --rounds 4 --settings "tune=0,pdl=0;tune=1,pdl=0;tune=2,pdl=0;tune=3,pdl=0;tune=3,pdl=1"
+  python tools/ab_bench.py --batch 32 --secs 10 --rounds 4 --settings "pdl=0;pdl=1;pdl=2"
 """
 import argparse
 import json
@@ -21,7 +21,7 @@ def main():
     ap.add_argument("--rounds", type=int, default=4)
     ap.add_argument("--calls", type=int, default=3, help="timed calls per setting per round")
     ap.add_argument("--precision", default="f16x3")
-    ap.add_argument("--settings", default="tune=0,pdl=0;tune=1,pdl=0;tune=2,pdl=0;tune=3,pdl=0;tune=3,pdl=1")
+    ap.add_argument("--settings", default="pdl=0;pdl=1;pdl=2")
     ap.add_argument("--json", default=None)
     args = ap.parse_args()
     import numpy as np
@@ -45,7 +45,7 @@ def main():
     times = [[] for _ in settings]
 
     def apply(st):
-        for k in ("graph", "pdl", "tune", "wide_variant", "act_tma", "branches", "pair"):
+        for k in ("graph", "pdl", "wide_variant", "branches", "pair"):
             if k in st:
                 nat.set_option(k, st[k])
         if "graph" not in st:

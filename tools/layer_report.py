@@ -22,10 +22,8 @@ def main():
     ap.add_argument("--json", default=None)
     ap.add_argument("--precision", default="fp32", choices=["fp32", "f16x3", "f16"])
     ap.add_argument("--wide-variant", type=int, default=None)
-    ap.add_argument("--act-tma", type=int, default=None)
     ap.add_argument("--pdl", type=int, default=None)
     ap.add_argument("--pair", type=int, default=None)
-    ap.add_argument("--tune", type=int, default=None)
     ap.add_argument("--reps", type=int, default=1, help="profiled calls (per-variant times are averaged)")
     args = ap.parse_args()
     import numpy as np
@@ -46,14 +44,10 @@ def main():
     nat.set_precision(args.precision)
     if args.wide_variant is not None:
         nat.set_option("wide_variant", args.wide_variant)
-    if args.act_tma is not None:
-        nat.set_option("act_tma", args.act_tma)
     if args.pdl is not None:
         nat.set_option("pdl", args.pdl)
     if args.pair is not None:
         nat.set_option("pair", args.pair)
-    if args.tune is not None:
-        nat.set_option("tune", args.tune)
     nat.set_option("graph", 0)
     for _ in range(2):
         nat.convert_waveform(wav, wlen, g, g, tau=0.3, seed=1)

@@ -46,16 +46,14 @@ with torch.no_grad():
     ro, _, (rz, rzp, rzh) = O.voice_conversion(sd, spec, lengths, gs, gt, noise, 0.3, taps=taps)
 summary = {}
 names = ["enc.wn", "dec.pre", "dec.ups0", "dec.stage0", "dec.ups1", "dec.stage1", "dec.ups2", "dec.stage2", "dec.ups3", "dec.stage3"]
-for mode, wv, tma, pair in (("fp32", 0, 1, 0), ("f16x3", 3, 1, 0), ("f16x3", 3, 1, 1), ("f16x3", 0, 0, 0), ("f16x3", 2, 1, 0), ("f16x3", 1, 1, 0),
-                            ("f16", 3, 1, 0), ("f16", 3, 1, 1)):
+for mode, wv, pair in (("fp32", 0, 0), ("f16x3", 3, 0), ("f16x3", 3, 1), ("f16x3", 0, 0), ("f16x3", 2, 0), ("f16", 3, 0), ("f16", 3, 1)):
     m.native.set_precision(mode)
     m.native.set_option("wide_variant", wv)
-    m.native.set_option("act_tma", tma)
     m.native.set_option("pair", pair)
     m.native.debug_enable(True)
     o, _, lat = m.voice_conversion(spec.cuda(), lengths.cuda(), gs.cuda(), gt.cuda(), tau=0.3, noise=noise.cuda(), ragged=False)
     torch.cuda.synchronize()
-    print(mode, "wide_variant", wv, "act_tma", tma, "pair", pair, "o_hat", f"{rel(o.cpu().numpy(), ro.numpy()):.3e}", "z", f"{rel(lat[0].cpu().numpy(), rz.numpy()):.3e}",
+    print(mode, "wide_variant", wv, "pair", pair, "o_hat", f"{rel(o.cpu().numpy(), ro.numpy()):.3e}", "z", f"{rel(lat[0].cpu().numpy(), rz.numpy()):.3e}",
           "z_hat", f"{rel(lat[2].cpu().numpy(), rzh.numpy()):.3e}")
     for name in names:
         if name not in taps:
@@ -70,7 +68,7 @@ for mode, wv, tma, pair in (("fp32", 0, 1, 0), ("f16x3", 3, 1, 0), ("f16x3", 3, 
         qo, _, _ = O.voice_conversion_ragged(sd, spec, lengths, gs, gt, noise, 0.3)
     e2 = rel(o2.cpu().numpy(), qo.numpy())
     print("    ragged o_hat", f"{e2:.3e}")
-    summary[f"{mode}:{wv}:{tma}:{pair}"] = max(rel(o.cpu().numpy(), ro.numpy()), e2)
+    summary[f"{mode}:{wv}:{pair}"] = max(rel(o.cpu().numpy(), ro.numpy()), e2)
 import json
 for k in summary:
     if not np.isfinite(summary[k]):
