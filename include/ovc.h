@@ -25,8 +25,8 @@
 extern "C" {
 #endif
 
-#define OVC_ABI_VERSION 3   /* 2: ovc_graph_replays, OVC_OPT_PDL .. OVC_OPT_PAIR; 3: OVC_OPT_ACT_TMA, OVC_OPT_TUNE and
-                             * OVC_OPT_WIDE_VARIANT 1 retired (ovc_set_option refuses them) */
+#define OVC_ABI_VERSION 4   /* 2: ovc_graph_replays, OVC_OPT_PDL .. OVC_OPT_PAIR; 3: OVC_OPT_ACT_TMA, OVC_OPT_TUNE and
+                             * OVC_OPT_WIDE_VARIANT 1 retired (ovc_set_option refuses them); 4: precision mode 3 */
 
 #if defined(__GNUC__)
 #define OVC_API __attribute__((visibility("default")))
@@ -175,7 +175,14 @@ OVC_API int ovc_tts_decode(ovc_ctx* ctx, const float* noise, uint64_t seed, floa
  *                a_hi*b_hi + (a_lo*b_hi + a_hi*b_lo) / 2^11, fp32 accumulation, cross terms in their own
  *                accumulator -- fp32-grade error, same parity gate as mode 0.  Operands must be < 65504 in magnitude.
  *   2            single-pass fp16 on the tensor cores (11-bit operands): the precision class the REFERENCE itself
- *                gets on a GPU by default (cuDNN TF32, torch.backends.cudnn.allow_tf32 = True); own looser gate */
+ *                gets on a GPU by default (cuDNN TF32, torch.backends.cudnn.allow_tf32 = True); own looser gate
+ *   3            fp16 storage in the generator ("f16s"): everything before the generator runs as in mode 1, so z, z_p and
+ *                z_hat are bit-identical to mode 1.  From conv_pre's output to conv_post's input every activation is
+ *                fp16 in memory (channels-last) and every conv is one fp16 pass with fp32 accumulation; bias, residual,
+ *                MRF sum and the 1/3 are fp32 math, each store rounds to fp16.  conv_post reads fp16 and writes fp32.
+ *                Half the generator's HBM traffic and workspace; o_hat SNR >= 50 dB against fp32.  Activations must
+ *                stay below 65504 in magnitude (no saturation).  OVC_OPT_PAIR and OVC_OPT_WIDE_VARIANT have no effect
+ *                on the generator in this mode. */
 OVC_API int ovc_set_precision(ovc_ctx* ctx, int mode);
 
 /* Tuning / diagnostics switches (never change results beyond fp32 reordering):

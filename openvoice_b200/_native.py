@@ -13,7 +13,7 @@ from typing import Dict, Iterable, Optional, Tuple
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libovc_b200.so")
 
-ABI_VERSION = 3
+ABI_VERSION = 4
 EXPORTS = (
     "ovc_abi_version", "ovc_last_error", "ovc_create", "ovc_destroy", "ovc_load_tensor",
     "ovc_finalize_weights", "ovc_workspace_floats", "ovc_voice_conversion", "ovc_last_launch_count",
@@ -35,7 +35,7 @@ class OvcHParams(C.Structure):
     ]
 
 
-PRECISIONS = {"fp32": 0, "f16x3": 1, "f16": 2}
+PRECISIONS = {"fp32": 0, "f16x3": 1, "f16": 2, "f16s": 3}
 
 
 class OvcError(RuntimeError):
@@ -189,7 +189,8 @@ class NativeConverter:
         self.finalized = True
 
     def set_precision(self, mode: str):
-        """'fp32' (CUDA-core FFMA2), 'f16x3' (split-precision fp16 tensor-core convs, fp32-grade) or 'f16' (single pass)."""
+        """'fp32' (CUDA-core FFMA2), 'f16x3' (split-precision fp16 tensor-core convs, fp32-grade), 'f16' (single pass)
+        or 'f16s' (as 'f16x3' up to z_hat, then an fp16-storage generator: fp16 activations, one fp16 pass per conv)."""
         m = PRECISIONS[mode]
         _check(self.lib, self.lib.ovc_set_precision(self.handle, m), "ovc_set_precision")
         self.precision = mode

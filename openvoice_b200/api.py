@@ -121,8 +121,10 @@ class NativeSynthesizer:
     def __init__(self, hps, device: str, precision: Optional[str] = None):
         """``precision``: arithmetic of the generator's ResBlock / upsampling convolutions --
         ``"f16x3"`` (default; split-precision fp16 on the tcgen05 tensor cores, fp32-grade),
-        ``"fp32"`` (CUDA-core FFMA2 everywhere) or ``"f16"`` (single-pass fp16: the 11-bit operand precision the
-        reference itself gets on a GPU through cuDNN's allow_tf32 default; ~1e-2).  Env override: OVC_PRECISION."""
+        ``"fp32"`` (CUDA-core FFMA2 everywhere), ``"f16"`` (single-pass fp16: the 11-bit operand precision the
+        reference itself gets on a GPU through cuDNN's allow_tf32 default; ~1e-2) or ``"f16s"`` (fp16 storage:
+        z / z_p / z_hat exactly as ``"f16x3"``, then a generator with fp16 activations in memory and one fp16 pass
+        per conv -- half its memory traffic and workspace, o_hat SNR >= 50 dB).  Env override: OVC_PRECISION."""
         dev = torch.device(device)
         if dev.type != "cuda":
             raise RuntimeError("openvoice_b200 runs on CUDA (sm_100a) only; there is no CPU path")
@@ -340,7 +342,10 @@ class BaseSpeakerTTS(OpenVoiceBaseClass):
 
 
 class ToneColorConverter(OpenVoiceBaseClass):
-    """openvoice/api.py:101-201."""
+    """openvoice/api.py:101-201.
+
+    ``precision=`` ("f16x3" default, "fp32", "f16" or "f16s") is passed to :class:`NativeSynthesizer`;
+    "f16s" is the fp16 configuration: fp16 generator activations, half the generator's memory, o_hat SNR >= 50 dB."""
 
     def __init__(self, *args, **kwargs):
         enable_watermark = kwargs.pop("enable_watermark", True)

@@ -203,7 +203,8 @@ struct ovc_ctx {
   TcLayer tc_c1[12][3], tc_c2[12][3], tc_ups[4], tc_pre;
   float* d_tcw = nullptr;      // tensor-core weight arena (hi/lo split)
   std::vector<float> h_tcw;
-  int precision = 0;           // 0: fp32 FFMA everywhere; 1: 3xFP16 split-precision tcgen05 convs; 2: single-pass fp16
+  int precision = 0;           // 0: fp32 FFMA everywhere; 1: 3xFP16 split-precision tcgen05 convs; 2: single-pass fp16;
+                               // 3: as 1, but the generator stores fp16 activations and runs one fp16 pass per conv
   int wide_variant = 3;        // kernel of the 128-column tensor-core layers (see launch_tc); 3 = chosen per layer
   bool tts_simple = false;     // OVC_OPT_TTS_SIMPLE
   bool use_graph = true;       // OVC_OPT_GRAPH
@@ -704,6 +705,10 @@ static int finalize(ovc_ctx* c) {
   CK(cudaFuncSetAttribute(tcconv_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<128>::SMEM_BYTES));
   CK(cudaFuncSetAttribute(tcconv_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<64>::SMEM_BYTES));
   CK(cudaFuncSetAttribute(tcconv_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<32>::SMEM_BYTES));
+  CK(cudaFuncSetAttribute(tcconv_kernel<128, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<128>::SMEM_BYTES));
+  CK(cudaFuncSetAttribute(tcconv_kernel<128, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<128>::SMEM_BYTES));
+  CK(cudaFuncSetAttribute(tcconv_kernel<64, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<64>::SMEM_BYTES));
+  CK(cudaFuncSetAttribute(tcconv_kernel<32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<32>::SMEM_BYTES));
   CK(cudaFuncSetAttribute(tcpair_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcpCfg<32>::SMEM_BYTES));
   CK(cudaFuncSetAttribute(tcpair_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcpCfg<64>::SMEM_BYTES));
   if (c->d_cond_wrow) cudaFree(c->d_cond_wrow);
@@ -754,16 +759,20 @@ static WsLayout ws_layout(const ovc_ctx* c, int B, int Tmax) {
   L.z = take((size_t)B * 192 * L.P);
   L.dpre = take((size_t)B * 512 * L.P);
   const size_t big = (size_t)B * 8192 * L.P;
-  L.bufA = take(big);
-  L.bufB = take(big);
-  L.bufC = take(big);
-  L.bufD = take(big);
-  L.bufE = c->precision ? take((size_t)B * 512 * L.P) : 0;     // conv_pre output, channels-last
-  L.bufF = (c->precision && c->debug) ? take(big) : 0;        // [C][T] scratch of the debug taps only
+  // precision 3: the generator's activations are fp16, two per float of these buffers.  bufA still holds the fp32
+  // channels-last z_hat of conv_pre (192 * P floats per utterance) and, earlier in the call, the WN stacks' fp32
+  // scratch; both fit in half.
+  const size_t gen = c->precision == 3 ? big / 2 : big;
+  L.bufA = take(gen);
+  L.bufB = take(gen);
+  L.bufC = take(gen);
+  L.bufD = take(gen);
+  L.bufE = c->precision ? take((size_t)B * (c->precision == 3 ? 256 : 512) * L.P) : 0;   // conv_pre output, channels-last
+  L.bufF = (c->precision && c->debug) ? take(big) : 0;        // fp32 [C][T] scratch of the debug taps only
   L.branches = c->precision && c->use_branches && (long long)B * Tmax <= c->par_frames;
   for (int j = 0; j < 2; ++j) {
-    L.brB[j] = L.branches ? take(big) : 0;
-    L.brC[j] = L.branches ? take(big) : 0;
+    L.brB[j] = L.branches ? take(gen) : 0;
+    L.brC[j] = L.branches ? take(gen) : 0;
   }
   L.spec = take((size_t)B * c->hp.spec_channels * L.P);
   L.frames = take((size_t)2 * B + 4);   // B int64
@@ -779,7 +788,7 @@ struct Run {
   const long long* glens;   // generator lengths: lens when ragged, NULL (= Tmax) otherwise
 };
 
-enum { V_TCPAIR64 = -12, V_TCPAIR32 = -13, V_TC128 = -1, V_TC64 = -2, V_TC32 = -3, V_TRANSPOSE = -4, V_TTS_DENSE = -5, V_TTS_LN = -6, V_TTS_SCORES = -7,
+enum { V_TCH128 = -14, V_TCH64 = -15, V_TCH32 = -16, V_TCPAIR64 = -12, V_TCPAIR32 = -13, V_TC128 = -1, V_TC64 = -2, V_TC32 = -3, V_TRANSPOSE = -4, V_TTS_DENSE = -5, V_TTS_LN = -6, V_TTS_SCORES = -7,
        V_TTS_ATTN = -8, V_TTS_DW = -9, V_TTS_SPLINE = -10, V_TTS_MISC = -11 };
 static const char* variant_name(int v) {
   if (v >= 0) return kInfo[v].name;
@@ -789,6 +798,9 @@ static const char* variant_name(int v) {
     case V_TC128: return "TC3_N128";
     case V_TC64: return "TC3_N64";
     case V_TC32: return "TC3_N32";
+    case V_TCH128: return "TC1H_N128";
+    case V_TCH64: return "TC1H_N64";
+    case V_TCH32: return "TC1H_N32";
     case V_TTS_DENSE: return "TTS_DENSE32";
     case V_TTS_LN: return "TTS_LAYERNORM";
     case V_TTS_SCORES: return "TTS_SCORES";
@@ -881,6 +893,7 @@ struct TcOpt {
   bool use_lens_frames = false;   // limits are the frame lengths (enc/flow) instead of the generator lengths
   const long long* lens_x = nullptr; bool has_lens_x = false;   // the input's own limit (TcConvArgs.lens_x)
   int grid_div = 1;               // persistent kernel: use 1 / grid_div of the SMs (concurrent ResBlock branches)
+  bool in16 = false, out16 = false;   // fp16 input / output activations (precision 3, generator only): one fp16 pass
 };
 // kernel launch with (optionally) the programmatic-stream-serialization attribute: the kernel may begin while its
 // predecessor in the stream drains; it calls griddepcontrol.wait before it touches dependent data (ovc_tcconv.cuh)
@@ -899,17 +912,20 @@ static cudaError_t launch_ex(void (*kernel)(KArgs...), dim3 grid, int block, siz
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
-// activation chunks by tensor-map TMA: the channels-last input as a [B][P * mul][C] fp32 tensor, one box = box_rows x 32
-// channels (128 bytes, 128-byte swizzle); rows outside the tensor are zero-filled by the copy engine
-static CUresult encode_act_map(CUtensorMap* tmap, const Run& r, const float* x, int C, int mul, int box_rows) {
+// activation chunks by tensor-map TMA: the channels-last input as a [B][P * mul][C] tensor, one box = box_rows x 32
+// channels; rows outside the tensor are zero-filled by the copy engine.  fp32: 128-byte rows, 128-byte swizzle (the
+// converter reads them row-strided).  fp16 (f16 = true): 64-byte rows, no swizzle (the converter reads them whole,
+// tc_convert_raw16).
+static CUresult encode_act_map(CUtensorMap* tmap, const Run& r, const float* x, int C, int mul, int box_rows, bool f16 = false) {
   memset(tmap, 0, sizeof *tmap);
+  const cuuint64_t es = f16 ? 2 : 4;
   const cuuint64_t gdim[3] = {(cuuint64_t)C, (cuuint64_t)r.P * mul, (cuuint64_t)r.B};
-  const cuuint64_t gstr[2] = {(cuuint64_t)C * 4, (cuuint64_t)((long long)C * r.P * mul) * 4};
+  const cuuint64_t gstr[2] = {(cuuint64_t)C * es, (cuuint64_t)((long long)C * r.P * mul) * es};
   const cuuint32_t box[3] = {32, (cuuint32_t)box_rows, 1};
   const cuuint32_t estr[3] = {1, 1, 1};
-  return encode_tiled_fn()(tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(x), gdim, gstr, box, estr,
-                           CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                           CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return encode_tiled_fn()(tmap, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(x), gdim,
+                           gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, f16 ? CU_TENSOR_MAP_SWIZZLE_NONE : CU_TENSOR_MAP_SWIZZLE_128B,
+                           CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
 
 // one conv on the tensor cores (3xFP16 split precision / single-pass fp16), channels-last in/out.  t_len / mul are in INPUT steps.
@@ -928,19 +944,26 @@ static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const f
   a.lens_x = o.lens_x; a.has_lens_x = o.has_lens_x ? 1 : 0;
   a.Cin = T.Cin; a.Ntot = T.Ntot; a.K = T.K; a.DIL = T.DIL;
   a.slope = o.slope; a.scale = o.scale; a.accumulate = o.accumulate;
-  a.passes = r.c->precision == 2 ? 1 : 3;
+  const bool f16s = o.in16 || o.out16;   // fp16 storage: one pass, the persistent kernel, the linear epilogue
+  a.passes = (r.c->precision == 2 || f16s) ? 1 : 3;
   if (T.TN == 0) return fail(OVC_ERR_INVALID, "conv %d -> %d (k %d, dilation %d) does not fit the tensor-core kernels", T.Cin, T.Ntot, T.K, T.DIL);
   if (!(o.slope >= 0.f && o.slope <= 1.f)) return fail(OVC_ERR_INVALID, "leaky_relu slope %g outside [0, 1]", (double)o.slope);
+  // the instantiations that exist: <TN, true, true> and <128, false, true> (conv_pre), linear epilogue only
+  if (f16s && (!o.out16 || o.epi != 0 || (!o.in16 && T.TN != 128)))
+    return fail(OVC_ERR_INVALID, "no fp16-storage tensor-core kernel for conv %d -> %d (fp16 in %d, epilogue %d)", T.Cin, T.Ntot, (int)o.in16, o.epi);
   const double units = (double)r.B * t_len;
   const int eff_k = o.family == 2 ? 2 : T.K;   // polyphase transposed conv: 2 of the 3 packed taps are non-zero per row
-  const ProfRec rec{T.TN == 128 ? V_TC128 : T.TN == 64 ? V_TC64 : V_TC32, o.family == 1 ? 1 : 0, 2.0 * T.Cin * T.Ntot * eff_k * units,
-                    4.0 * (T.Cin + T.Ntot * (1 + (res ? 1 : 0) + (o.accumulate ? 1 : 0))) * units, (T.Cin << 16) | (T.K << 8) | T.DIL};
+  const double in_b = o.in16 ? 2.0 : 4.0, out_b = o.out16 ? 2.0 : 4.0;   // bytes per element
+  const int var = f16s ? (T.TN == 128 ? V_TCH128 : T.TN == 64 ? V_TCH64 : V_TCH32) : (T.TN == 128 ? V_TC128 : T.TN == 64 ? V_TC64 : V_TC32);
+  const ProfRec rec{var, o.family == 1 ? 1 : 0, 2.0 * T.Cin * T.Ntot * eff_k * units,
+                    (in_b * T.Cin + out_b * T.Ntot * (1 + (res ? 1 : 0) + (o.accumulate ? 1 : 0))) * units, (T.Cin << 16) | (T.K << 8) | T.DIL};
   const bool pdl = r.c->use_pdl == 1 || (r.c->use_pdl == 2 && o.epi != 0);
   // 3 (default): the generator's first stage (k >= 7 at C = 256: few, long tiles) on the two-CTAs-per-SM kernel, whose
-  // second CTA fills the tensor pipe while the first waits on a barrier; everything else on the persistent kernel
+  // second CTA fills the tensor pipe while the first waits on a barrier; everything else on the persistent kernel.
+  // fp16 storage always runs on the persistent kernel (the wide kernel is fp32-only).
   int wv = r.c->wide_variant;
   if (wv == 3) wv = (T.K >= 7 && T.Cin >= 256) ? 2 : 0;
-  if (T.TN == 128 && wv == 2) {
+  if (T.TN == 128 && wv == 2 && !f16s) {
     // 128-step tiles, two CTAs per SM
     dim3 grid((t_len + 127) / 128, T.Ntot / 128, r.B);
     return launch_kernel(r, rec, [&] { return launch_ex(tcconv_wide_kernel, grid, TcwCfg::THREADS, TcwCfg::SMEM_BYTES, r.st, pdl, a); });
@@ -954,13 +977,20 @@ static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const f
   a.n_box = rows > 256 ? 2 : 1;
   a.box_rows = rows / a.n_box;
   CUtensorMap tmap;
-  const CUresult cr = encode_act_map(&tmap, r, x, T.Cin, mul, a.box_rows);
+  const CUresult cr = encode_act_map(&tmap, r, x, T.Cin, mul, a.box_rows, o.in16);
   if (cr != CUDA_SUCCESS) return fail(OVC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d) for a [%d][%d][%d] activation tensor", (int)cr,
                                       r.B, r.P * mul, T.Cin);
   const int ncol = T.Ntot / T.TN;
   const int per_col = std::max(1, r.c->sm_count / ncol / std::max(1, o.grid_div));
   dim3 pg((unsigned)std::min(total, per_col), ncol, 1);
   return launch_kernel(r, rec, [&] {
+    if (o.in16) {
+      if (T.TN == 128) return launch_ex(tcconv_kernel<128, true, true>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
+      if (T.TN == 64) return launch_ex(tcconv_kernel<64, true, true>, pg, TCN_THREADS, TcnCfg<64>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
+      return launch_ex(tcconv_kernel<32, true, true>, pg, TCN_THREADS, TcnCfg<32>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
+    }
+    if (o.out16)   // conv_pre: fp32 z_hat in, fp16 out
+      return launch_ex(tcconv_kernel<128, false, true>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
     if (T.TN == 128) return launch_ex(tcconv_kernel<128>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
     if (T.TN == 64) return launch_ex(tcconv_kernel<64>, pg, TCN_THREADS, TcnCfg<64>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
     return launch_ex(tcconv_kernel<32>, pg, TCN_THREADS, TcnCfg<32>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
@@ -1007,10 +1037,15 @@ static int launch_pair(Run& r, const TcLayer& T1, const TcLayer& T2, const float
   });
 }
 
-static int launch_transpose(Run& r, const float* src, float* dst, int rows, int cols) {
+// src16: the source is fp16 (read through the same pointer type as the fp32 workspace buffers), dst is always fp32
+static int launch_transpose(Run& r, const float* src, float* dst, int rows, int cols, bool src16 = false) {
   dim3 grid((cols + 31) / 32, (rows + 31) / 32, r.B);
-  return launch_kernel(r, ProfRec{V_TRANSPOSE, 0, 0.0, 8.0 * rows * cols * r.B},
-                       [&] { transpose_kernel<<<grid, 256, 0, r.st>>>(src, dst, rows, cols, (long long)rows * cols); });
+  return launch_kernel(r, ProfRec{V_TRANSPOSE, 0, 0.0, (src16 ? 6.0 : 8.0) * rows * cols * r.B}, [&] {
+    if (src16)
+      transpose_kernel<<<grid, 256, 0, r.st>>>(reinterpret_cast<const __half*>(src), dst, rows, cols, (long long)rows * cols);
+    else
+      transpose_kernel<<<grid, 256, 0, r.st>>>(src, dst, rows, cols, (long long)rows * cols);
+  });
 }
 
 // every speaker-conditioning 1x1 conv of a call in one launch (rows of the cond section of the workspace)
@@ -1212,6 +1247,7 @@ static int run_mrf_tc(Run& r, const WsLayout& W, float* ws, int i, int Tlen, int
     float* Bj = ws + W.bufB; float* Cj = ws + W.bufC;
     TcOpt o;
     o.slope = 0.1f; o.family = 1;
+    o.in16 = o.out16 = c->precision == 3;
     if (par) {
       o.grid_div = 3;
       if (j > 0) {
@@ -1220,7 +1256,7 @@ static int run_mrf_tc(Run& r, const WsLayout& W, float* ws, int i, int Tlen, int
         Bj = ws + W.brB[j - 1]; Cj = ws + W.brC[j - 1];
       }
     }
-    bool fused = !par && c->use_pair;
+    bool fused = !par && c->use_pair && c->precision != 3;   // the pair kernel is fp32-only
     for (int d = 0; d < 3; ++d) fused = fused && pair_fits(c1[d], c2[d]);
     for (int d = 0; d < 3; ++d) {
       TcOpt o2 = o;
@@ -1251,6 +1287,8 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
   const int B = r.B, Tmax = r.Tmax, P = W.P;
   // ---- generator (models.py:272-291).  Lengths: frames * cumulative upsampling.
   const bool pre_tc = c->precision >= 1 && c->tc_pre.TN != 0;
+  const bool f16s = c->precision == 3;   // fp16 activations from conv_pre's output to conv_post's input
+  if (f16s && !pre_tc) return fail(OVC_ERR_INVALID, "precision 3 needs conv_pre on the tensor cores (inter_channels %% 32 == 0)");
   if (!pre_tc) {
     ConvArgs a = conv_args(ws + W.z, 192, P, ws + W.dpre, 512, P, r.glens, 1, 1.f);
     a.bias = cond + c->cond_off_dec; a.bias_bs = c->cond_rows_out;
@@ -1264,10 +1302,10 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
     // ConvTranspose1d = polyphase conv Cin -> s*Cout whose row n IS output rows s*n .. s*n+s-1 of the
     // channels-last result; ResBlock convs = tcconv with fused lrelu / bias / residual / MRF average.
     float* bufE = ws + W.bufE;
-    float* bufF = ws + W.bufF;   // [C][T] scratch for debug taps
+    float* bufF = ws + W.bufF;   // fp32 [C][T] scratch for debug taps
     auto tap_cl = [&](const char* nm, const float* cl, int C, int T_, int pitch) -> int {
       if (!c->debug) return OVC_OK;
-      TRY(launch_transpose(r, cl, bufF, pitch, C));
+      TRY(launch_transpose(r, cl, bufF, pitch, C, f16s));
       return tap(r, nm, bufF, C, T_, pitch);
     };
     if (pre_tc) {
@@ -1277,6 +1315,7 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
       TcOpt e;
       e.bias = cond + c->cond_off_dec; e.bias_bs = c->cond_rows_out;
       e.lens_x = lens; e.has_lens_x = lens != nullptr;
+      e.out16 = f16s;
       TRY(launch_tc(r, c->tc_pre, bufA, bufE, nullptr, Tmax, 1, e));
       TRY(tap_cl("dec.pre", bufE, 512, Tmax, P));
     } else {
@@ -1296,6 +1335,7 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
       char nm[32];
       TcOpt u;
       u.slope = 0.1f; u.family = 2;
+      u.in16 = u.out16 = f16s;
       TRY(launch_tc(r, c->tc_ups[i], stage_in, bufA, nullptr, Tmax * up, up, u));
       snprintf(nm, sizeof nm, "dec.ups%d", i);
       TRY(tap_cl(nm, bufA, cout, Tlen, pitch_out));
@@ -1308,8 +1348,12 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
     const int y_len = Tmax * up;
     dim3 grid((y_len + 255) / 256, B);
     return launch_kernel(r, std::nullopt, [&] {
-      conv_post_cl_kernel<32><<<grid, 256, 0, r.st>>>(stage_in, 32LL * P * up, c->d_w + c->post_w_off, o_hat, (long long)y_len,
-                                                      y_len, r.glens, Tmax, up);
+      if (f16s)
+        conv_post_cl_kernel<32, __half><<<grid, 256, 0, r.st>>>(reinterpret_cast<const __half*>(stage_in), 32LL * P * up, c->d_w + c->post_w_off,
+                                                        o_hat, (long long)y_len, y_len, r.glens, Tmax, up);
+      else
+        conv_post_cl_kernel<32><<<grid, 256, 0, r.st>>>(stage_in, 32LL * P * up, c->d_w + c->post_w_off, o_hat, (long long)y_len,
+                                                        y_len, r.glens, Tmax, up);
     });
   }
   const float* stage_in = ws + W.dpre;
@@ -1640,7 +1684,9 @@ int ovc_tts_decode(ovc_ctx* c, const float* noise, uint64_t seed, float noise_sc
 
 int ovc_set_precision(ovc_ctx* c, int mode) {
   if (!c) return fail(OVC_ERR_INVALID, "null context");
-  if (mode < 0 || mode > 2) return fail(OVC_ERR_INVALID, "precision mode must be 0 (fp32 FFMA2), 1 (3xTF32 tensor cores) or 2 (single-pass TF32)");
+  if (mode < 0 || mode > 3)
+    return fail(OVC_ERR_INVALID, "precision mode must be 0 (fp32 FFMA2), 1 (3xFP16 tensor cores), 2 (single-pass fp16) or 3 (fp16 generator "
+                                 "storage)");
   c->precision = mode;
   return OVC_OK;
 }
@@ -1710,7 +1756,11 @@ int ovc_profile_detail(ovc_ctx* c, int max, char* names /* max x 16 */, double* 
     if (names) {
       const int tag = p.tag, v = p.variant;
       if (tag && (v == V_TCPAIR64 || v == V_TCPAIR32)) snprintf(names + 16 * n, 16, "P%dk%dd%d", tag >> 16, (tag >> 8) & 255, tag & 255);
-      else if (tag) snprintf(names + 16 * n, 16, "T%dc%dk%dd%d", v == V_TC128 ? 128 : v == V_TC64 ? 64 : 32, tag >> 16, (tag >> 8) & 255, tag & 255);
+      else if (tag) {
+        const bool h = v == V_TCH128 || v == V_TCH64 || v == V_TCH32;   // fp16-storage launch: "H..." instead of "T..."
+        snprintf(names + 16 * n, 16, "%c%dc%dk%dd%d", h ? 'H' : 'T', v == V_TC128 || v == V_TCH128 ? 128 : v == V_TC64 || v == V_TCH64 ? 64 : 32,
+                 tag >> 16, (tag >> 8) & 255, tag & 255);
+      }
       else { strncpy(names + 16 * n, variant_name(v), 15); names[16 * n + 15] = 0; }
     }
     if (ms) ms[n] = m;

@@ -2,7 +2,7 @@
 //
 //   Y[t, n] = (bias[n] + sum_{tap, c} W[n, c, tap] * lrelu(X[t + (tap - (K-1)/2) * DIL, c]) [+ R[t, n]] [+ Y_old[t, n]]) * scale
 //
-// Channels-last fp32 activations X[b][t][C] (time-major rows).  Every operand is split x = hi + lo / 2^11 with
+// Channels-last fp32 activations X[b][t][C] (time-major rows; fp16 in precision mode 3, tcconv_kernel<TN, true, true>).  Every operand is split x = hi + lo / 2^11 with
 // hi = fp16(x), lo = fp16((x - hi) * 2^11) (22 mantissa bits, ovc_tc.cuh) and every product is evaluated as
 // a_hi*b_hi + (a_lo*b_hi + a_hi*b_lo) / 2^11 by tcgen05.mma.kind::f16 with fp32 accumulation in TMEM: the hi*hi
 // products in one accumulator, the two cross terms in a second one ("low-order accumulator"), joined in the
@@ -74,6 +74,22 @@ __device__ __forceinline__ void tc_item(int i, int& row, int& kc) {
   row = (i / (8 * NKC)) * 8 + (i & 7);
 }
 
+// Storage type of the activations a kernel reads or writes: fp32, or fp16 (precision mode 3, the generator only).
+// Two consecutive channels are loaded / stored as one float2 or half2 and the arithmetic is always fp32; an fp16 store
+// rounds to nearest.
+template <bool F16>
+struct TcAct {
+  using T = float;
+};
+template <>
+struct TcAct<true> {
+  using T = __half;
+};
+__device__ __forceinline__ float2 tc_ld2(const float* p) { return *reinterpret_cast<const float2*>(p); }
+__device__ __forceinline__ float2 tc_ld2(const __half* p) { return __half22float2(*reinterpret_cast<const __half2*>(p)); }
+__device__ __forceinline__ void tc_st2(float* p, float2 v) { *reinterpret_cast<float2*>(p) = v; }
+__device__ __forceinline__ void tc_st2(__half* p, float2 v) { *reinterpret_cast<__half2*>(p) = __floats2half2_rn(v.x, v.y); }
+
 // Epilogue of MMA tiles [mt_lo, mt_hi) x columns [c_lo, c_hi) of one CTA tile (MT x 128 steps x TN columns): TMEM ->
 // registers -> fused ops -> global.  Warp w may read TMEM lanes [32*(w%4), +32); tile mt owns columns [2*mt*TN, +TN)
 // (main accumulator) and the next TN (low-order accumulator).
@@ -82,16 +98,19 @@ __device__ __forceinline__ void tc_item(int i, int& row, int& kc) {
 // sectors (the thread-per-row layout moved 16 bytes per sector and spilled).  Operands with DRAM latency -- the
 // residual of a ResBlock conv, the read-modify-write target of the WaveNet res/skip update -- are fetched one block
 // ahead, and those of the first block BEFORE the wait on the accumulator barrier `bar`: they arrive under the MMAs.
-template <int TN>
+// OUT16: y, r and the accumulate target are fp16 (half2 per thread and row, fp32 math, one rounding at the store); a
+// quad then covers 16 bytes of a row per 8-column group, and groups g and g + 1 fill one 32-byte sector.
+template <int TN, bool OUT16 = false>
 __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, int b, int t0, int n0, int lim, int warp, int lane,
                                             int mt_lo, int mt_hi, int c_lo, int c_hi, uint64_t* bar, uint32_t parity) {
+  using T = typename TcAct<OUT16>::T;
   const int lane_base = (warp & 3) * 32;
   const int rsub = lane >> 2, csub = (lane & 3) * 2;
-  float* yb = a.y + (size_t)b * a.y_bs;
-  const float* rb = a.r ? a.r + (size_t)b * a.y_bs : nullptr;
-  float* sb = a.s ? a.s + (size_t)b * a.s_bs : nullptr;
+  T* yb = reinterpret_cast<T*>(a.y) + (size_t)b * a.y_bs;
+  const T* rb = a.r ? reinterpret_cast<const T*>(a.r) + (size_t)b * a.y_bs : nullptr;
+  T* sb = a.s ? reinterpret_cast<T*>(a.s) + (size_t)b * a.s_bs : nullptr;
   const float* bias = a.bias + (size_t)b * a.bias_bs;
-  const bool two = a.passes == 3;
+  const bool two = !OUT16 && a.passes == 3;   // the fp16-storage instantiations run one pass
   const int ncb = (c_hi - c_lo) >> 5;
   const int nblk = (mt_hi - mt_lo) * ncb * 2;
 
@@ -103,9 +122,9 @@ __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, i
     row = lane_base + 16 * h + rsub;
   };
   // where block k's read-modify-write / residual operand lives (nullptr: none)
-  auto operand = [&](int c0, bool& add) -> const float* {
+  auto operand = [&](int c0, bool& add) -> const T* {
     add = true;
-    if (a.epi == 0) return rb ? rb + n0 + c0 + csub : nullptr;
+    if (OUT16 || a.epi == 0) return rb ? rb + n0 + c0 + csub : nullptr;
     if (a.epi == 2) {
       const int col = n0 + c0;
       const bool to_x = col < a.split;          // uniform per 32-column group (split is a multiple of 32)
@@ -118,15 +137,15 @@ __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, i
     int mt, c0, row;
     geom(k, mt, c0, row);
     bool add;
-    const float* src = operand(c0, add);
+    const T* src = operand(c0, add);
     const int ta = t0 + mt * 128 + row, tb = ta + 8;
 #pragma unroll
     for (int g = 0; g < 4; ++g) {
       q[2 * g] = make_float2(0.f, 0.f);
       q[2 * g + 1] = make_float2(0.f, 0.f);
       if (src && add) {
-        if (ta < lim) q[2 * g] = *reinterpret_cast<const float2*>(src + (size_t)ta * a.y_ld + 8 * g);
-        if (tb < lim) q[2 * g + 1] = *reinterpret_cast<const float2*>(src + (size_t)tb * a.y_ld + 8 * g);
+        if (ta < lim) q[2 * g] = tc_ld2(src + (size_t)ta * a.y_ld + 8 * g);
+        if (tb < lim) q[2 * g + 1] = tc_ld2(src + (size_t)tb * a.y_ld + 8 * g);
       }
     }
   };
@@ -156,14 +175,14 @@ __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, i
     float2 bq[4], ya[4], yc[4];
 #pragma unroll
     for (int g = 0; g < 4; ++g) bq[g] = __ldg(reinterpret_cast<const float2*>(bias + n0 + c0 + 8 * g + csub));
-    const bool accum = a.epi == 0 && a.accumulate;
+    const bool accum = (OUT16 || a.epi == 0) && a.accumulate;
     if (accum) {
 #pragma unroll
       for (int g = 0; g < 4; ++g) {
         ya[g] = make_float2(0.f, 0.f);
         yc[g] = make_float2(0.f, 0.f);
-        if (oka) ya[g] = *reinterpret_cast<const float2*>(yb + (size_t)ta * a.y_ld + n0 + c0 + 8 * g + csub);
-        if (okb) yc[g] = *reinterpret_cast<const float2*>(yb + (size_t)tb * a.y_ld + n0 + c0 + 8 * g + csub);
+        if (oka) ya[g] = tc_ld2(yb + (size_t)ta * a.y_ld + n0 + c0 + 8 * g + csub);
+        if (okb) yc[g] = tc_ld2(yb + (size_t)tb * a.y_ld + n0 + c0 + 8 * g + csub);
       }
     }
     float v[16];
@@ -180,10 +199,10 @@ __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, i
     for (int g = 0; g < 4; ++g) {
       v[4 * g] += bq[g].x; v[4 * g + 1] += bq[g].y; v[4 * g + 2] += bq[g].x; v[4 * g + 3] += bq[g].y;
     }
-    if (a.epi == 0) {
-      // ---- linear: bias, residual, MRF accumulate, scale
-      float* ypa = yb + (size_t)ta * a.y_ld + n0 + c0 + csub;
-      float* ypb = yb + (size_t)tb * a.y_ld + n0 + c0 + csub;
+    if (OUT16 || a.epi == 0) {   // an fp16 output has the linear epilogue only (launch_tc refuses the others)
+      // ---- linear: bias, residual, MRF accumulate, scale (fp32 math; an fp16 output rounds once, at the store)
+      T* ypa = yb + (size_t)ta * a.y_ld + n0 + c0 + csub;
+      T* ypb = yb + (size_t)tb * a.y_ld + n0 + c0 + csub;
 #pragma unroll
       for (int g = 0; g < 4; ++g) {
         float2 oa = make_float2(v[4 * g] + rq[2 * g].x, v[4 * g + 1] + rq[2 * g].y);
@@ -193,33 +212,33 @@ __device__ __forceinline__ void tc_epilogue(const TcConvArgs& a, uint32_t acc, i
           ob.x = yc[g].x + ob.x; ob.y = yc[g].y + ob.y;
         }
         if (a.scale != 1.f) { oa.x *= a.scale; oa.y *= a.scale; ob.x *= a.scale; ob.y *= a.scale; }
-        if (oka) *reinterpret_cast<float2*>(ypa + 8 * g) = oa;
-        if (okb) *reinterpret_cast<float2*>(ypb + 8 * g) = ob;
+        if (oka) tc_st2(ypa + 8 * g, oa);
+        if (okb) tc_st2(ypb + 8 * g, ob);
       }
     } else if (a.epi == 1) {
       // ---- WaveNet gate (modules.py:185-210): columns [0,16) of the group are the tanh inputs of 16 channels,
       // [16,32) their sigmoid partners -> 16 output channels at column (n0 + c0) / 2
-      float* ypa = yb + (size_t)ta * a.y_ld + ((n0 + c0) >> 1) + csub;
-      float* ypb = yb + (size_t)tb * a.y_ld + ((n0 + c0) >> 1) + csub;
+      T* ypa = yb + (size_t)ta * a.y_ld + ((n0 + c0) >> 1) + csub;
+      T* ypb = yb + (size_t)tb * a.y_ld + ((n0 + c0) >> 1) + csub;
 #pragma unroll
       for (int g = 0; g < 2; ++g) {
         const float2 oa = make_float2(tanhf(v[4 * g]) * sigmoidf_acc(v[4 * (g + 2)]),
                                       tanhf(v[4 * g + 1]) * sigmoidf_acc(v[4 * (g + 2) + 1]));
         const float2 ob = make_float2(tanhf(v[4 * g + 2]) * sigmoidf_acc(v[4 * (g + 2) + 2]),
                                       tanhf(v[4 * g + 3]) * sigmoidf_acc(v[4 * (g + 2) + 3]));
-        if (oka) *reinterpret_cast<float2*>(ypa + 8 * g) = oa;
-        if (okb) *reinterpret_cast<float2*>(ypb + 8 * g) = ob;
+        if (oka) tc_st2(ypa + 8 * g, oa);
+        if (okb) tc_st2(ypb + 8 * g, ob);
       }
     } else {
       // ---- WaveNet res/skip: columns < split update x in place (x += res), the rest go to the skip sum (= / +=)
       bool add;
-      float* dst = const_cast<float*>(operand(c0, add));
+      T* dst = const_cast<T*>(operand(c0, add));
 #pragma unroll
       for (int g = 0; g < 4; ++g) {
         const float2 oa = make_float2(rq[2 * g].x + v[4 * g], rq[2 * g].y + v[4 * g + 1]);
         const float2 ob = make_float2(rq[2 * g + 1].x + v[4 * g + 2], rq[2 * g + 1].y + v[4 * g + 3]);
-        if (oka) *reinterpret_cast<float2*>(dst + (size_t)ta * a.y_ld + 8 * g) = oa;
-        if (okb) *reinterpret_cast<float2*>(dst + (size_t)tb * a.y_ld + 8 * g) = ob;
+        if (oka) tc_st2(dst + (size_t)ta * a.y_ld + 8 * g, oa);
+        if (okb) tc_st2(dst + (size_t)tb * a.y_ld + 8 * g, ob);
       }
     }
 #pragma unroll
@@ -277,6 +296,42 @@ __device__ __forceinline__ void tc_convert_raw(const unsigned char* raw, unsigne
     fetch(i + NT, b0, b1);
     emit(i, a0, a1);
     emit(i + NT, b0, b1);
+  }
+}
+
+// The fp16 counterpart (precision mode 3): a raw fp16 stage of rows x 32 channels, 64 bytes per row, unswizzled ->
+// leaky-relu in fp32 -> fp16 (round to nearest) -> the hi operand tile only (one pass: there is no lo tile).  Item i =
+// (row i / 4, column block i % 4) is one 16-byte piece, so the 8 lanes of a quarter-warp read two whole rows, 128
+// contiguous bytes: conflict-free without a swizzle.  Rows outside [0, lim) become zeros, as above.
+template <int ROWS, int NT>
+__device__ __forceinline__ void tc_convert_raw16(const unsigned char* raw, unsigned char* ah, int pt, int items, int t_first, int lim,
+                                                 float slope) {
+  auto fetch = [&](int i, uint4& v) {
+    const int row = i >> 2, kc = i & 3;
+    const int t = t_first + row;
+    v = make_uint4(0u, 0u, 0u, 0u);
+    if (i < items && t >= 0 && t < lim) v = *reinterpret_cast<const uint4*>(raw + row * 64 + kc * 16);
+  };
+  auto emit = [&](int i, uint4 v) {
+    if (i >= items) return;
+    const int row = i >> 2, kc = i & 3;
+    uint32_t h[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      float2 f = __half22float2(*reinterpret_cast<const __half2*>(&h[k]));
+      f.x = fmaxf(f.x, f.x * slope);   // leaky_relu, as in tc::split_f16x8
+      f.y = fmaxf(f.y, f.y * slope);
+      const __half2 r = __floats2half2_rn(f.x, f.y);
+      h[k] = *reinterpret_cast<const uint32_t*>(&r);
+    }
+    *reinterpret_cast<uint4*>(ah + (kc * ROWS + row) * 16) = make_uint4(h[0], h[1], h[2], h[3]);
+  };
+  for (int i = pt; i < items; i += 2 * NT) {
+    uint4 a, b;
+    fetch(i, a);
+    fetch(i + NT, b);
+    emit(i, a);
+    emit(i + NT, b);
   }
 }
 
@@ -534,7 +589,9 @@ __host__ __device__ inline int tcn_rows(int mt, int H) {
   return r <= 256 ? (r + 7) & ~7 : (r + 15) & ~15;
 }
 
-template <int TN>
+// IN16 / OUT16: the activations read / written are fp16 (precision mode 3).  An fp16 raw stage holds 64-byte rows in
+// the same stage buffers (half of each is used), and these instantiations run one fp16 pass per conv.
+template <int TN, bool IN16 = false, bool OUT16 = false>
 __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs a, int n_tt, int total,
                                                                 const __grid_constant__ CUtensorMap tmap) {
   using Cfg = TcnCfg<TN>;
@@ -607,7 +664,7 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
     if (lane == 0) {
       int st = 0;
       uint32_t phase = 1;   // the first pass finds every raw stage free
-      const uint32_t box_bytes = (uint32_t)a.box_rows * 128u;
+      const uint32_t box_bytes = (uint32_t)a.box_rows * (IN16 ? 64u : 128u);
       for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
         const TcTile tl = tc_tile(tile, n_tt, MT * 128, a.lens, lens_x, a.tmax, a.mul);
         if (tl.t0 >= tl.lim) continue;
@@ -631,7 +688,7 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
       const uint64_t a_proto = tc::make_desc(0, LBO_A, SBO) + mt * 128, b_proto = tc::make_desc(0, LBO_B, SBO);
       const uint64_t b_ring = b_proto + (tc::smem_addr(bring) >> 4);
       const uint32_t dil = (uint32_t)a.DIL;
-      const bool three = a.passes == 3;
+      const bool three = !(IN16 || OUT16) && a.passes == 3;
       int slot = 0, buf = 0, n = 0;
       uint32_t bphase = 0, aphase = 0;
       for (int tile = blockIdx.x; tile < total; tile += gridDim.x) {
@@ -685,8 +742,12 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
       for (int q = 0; q < nq; ++q) {
         mbar_wait(&raw_full[st], rphase);
         mbar_wait(&a_empty[buf], ephase);
-        tc_convert_raw<ROWS, NCT>(raw + st * Cfg::RAW_STAGE_BYTES, abuf + buf * Cfg::A_BUF_BYTES, pt, items, tl.t0 - H, tl.lim_x,
-                                  a.slope);
+        if constexpr (IN16)
+          tc_convert_raw16<ROWS, NCT>(raw + st * Cfg::RAW_STAGE_BYTES, abuf + buf * Cfg::A_BUF_BYTES, pt, items, tl.t0 - H, tl.lim_x,
+                                      a.slope);
+        else
+          tc_convert_raw<ROWS, NCT>(raw + st * Cfg::RAW_STAGE_BYTES, abuf + buf * Cfg::A_BUF_BYTES, pt, items, tl.t0 - H, tl.lim_x,
+                                    a.slope);
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         mbar_arrive(&a_full[buf]);
         if (++buf == NABUF) { buf = 0; ephase ^= 1; }
@@ -706,7 +767,7 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
       const TcTile tl = tc_tile(tile, n_tt, MT * 128, a.lens, lens_x, a.tmax, a.mul);
       if (tl.t0 >= tl.lim) continue;
       const int set = n & 1;
-      tc_epilogue<TN>(a, tmem_d + set * SET_COLS, tl.b, tl.t0, n0, tl.lim, warp, lane, mt_lo, mt_hi, c_lo, c_hi, &acc_full[set],
+      tc_epilogue<TN, OUT16>(a, tmem_d + set * SET_COLS, tl.b, tl.t0, n0, tl.lim, warp, lane, mt_lo, mt_hi, c_lo, c_hi, &acc_full[set],
                       (n >> 1) & 1);
       tc::fence_before();
       __syncwarp();
@@ -719,11 +780,19 @@ __global__ void __launch_bounds__(TCN_THREADS, 1) tcconv_kernel(const TcConvArgs
   if (warp == 1) tc::tmem_dealloc(tmem_d, Cfg::TMEM_COLS);
 }
 
-// conv_post on channels-last input: y[b, t] = tanh(sum_{k<7, ci<C} w[ci, k] * lrelu_0.01(x[b, t+k-3, ci]))
+// four consecutive channels of an fp32 or fp16 activation row
+__device__ __forceinline__ float4 ld_f4(const float* p) { return *reinterpret_cast<const float4*>(p); }
+__device__ __forceinline__ float4 ld_f4(const __half* p) {
+  const uint2 u = *reinterpret_cast<const uint2*>(p);
+  const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+  return make_float4(a.x, a.y, b.x, b.y);
+}
+
+// conv_post on channels-last input (fp32, or fp16 in precision mode 3): y[b, t] = tanh(sum_{k<7, ci<C} w[ci, k] * lrelu_0.01(x[b, t+k-3, ci]))
 // (models.py:287-289).  HBM-bound (132 B per sample): a CTA stages 256+6 rows with coalesced 16-byte loads into a
 // transposed, conflict-free shared tile (leaky_relu applied once), then one thread per output sample.
-template <int C>
-__global__ void __launch_bounds__(256) conv_post_cl_kernel(const float* __restrict__ x, long long x_bs,
+template <int C, class T = float>
+__global__ void __launch_bounds__(256) conv_post_cl_kernel(const T* __restrict__ x, long long x_bs,
                                                            const float* __restrict__ w, float* __restrict__ y,
                                                            long long y_bs, int y_len, const long long* lens, int tmax,
                                                            int mul) {
@@ -734,12 +803,12 @@ __global__ void __launch_bounds__(256) conv_post_cl_kernel(const float* __restri
   const int b = blockIdx.y;
   const int lim = (lens ? (int)min((long long)tmax, lens[b]) : tmax) * mul;
   const int t0 = blockIdx.x * TB;
-  const float* xb = x + (size_t)b * x_bs;
+  const T* xb = x + (size_t)b * x_bs;
   for (int idx = threadIdx.x; idx < ROWS * (C / 4); idx += blockDim.x) {
     const int row = idx / (C / 4), q = idx % (C / 4);
     const int tt = t0 - 3 + row;
     float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (tt >= 0 && tt < lim) v = *reinterpret_cast<const float4*>(xb + (size_t)tt * C + 4 * q);
+    if (tt >= 0 && tt < lim) v = ld_f4(xb + (size_t)tt * C + 4 * q);
     xs[4 * q + 0][row] = v.x > 0.f ? v.x : 0.01f * v.x;
     xs[4 * q + 1][row] = v.y > 0.f ? v.y : 0.01f * v.y;
     xs[4 * q + 2][row] = v.z > 0.f ? v.z : 0.01f * v.z;
@@ -759,17 +828,19 @@ __global__ void __launch_bounds__(256) conv_post_cl_kernel(const float* __restri
   y[(size_t)b * y_bs + t] = acc;
 }
 
-// [B][C][pitch] <-> [B][pitch][C] tiled transpose (32x32 through shared memory)
-__global__ void __launch_bounds__(256) transpose_kernel(const float* __restrict__ src, float* __restrict__ dst, int rows,
+// [B][C][pitch] <-> [B][pitch][C] tiled transpose (32x32 through shared memory); T = __half reads an fp16 source
+// (the generator's debug taps in precision mode 3) and writes fp32
+template <class T = float>
+__global__ void __launch_bounds__(256) transpose_kernel(const T* __restrict__ src, float* __restrict__ dst, int rows,
                                                         int cols, long long bs) {
   __shared__ float tile[32][33];
-  const float* s = src + (size_t)blockIdx.z * bs;
+  const T* s = src + (size_t)blockIdx.z * bs;
   float* d = dst + (size_t)blockIdx.z * bs;
   const int c0 = blockIdx.x * 32, r0 = blockIdx.y * 32;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
   for (int i = ty; i < 32; i += 8) {
     const int r = r0 + i, c = c0 + tx;
-    tile[i][tx] = (r < rows && c < cols) ? s[(size_t)r * cols + c] : 0.f;
+    tile[i][tx] = (r < rows && c < cols) ? static_cast<float>(s[(size_t)r * cols + c]) : 0.f;
   }
   __syncthreads();
   for (int i = ty; i < 32; i += 8) {

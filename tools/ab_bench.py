@@ -3,6 +3,9 @@
 settings interleaved round-robin so that clock / thermal drift hits all of them alike.
 
   python tools/ab_bench.py --batch 32 --secs 10 --rounds 4 --settings "pdl=0;pdl=1;pdl=2"
+  python tools/ab_bench.py --settings "precision=f16x3;precision=f16;precision=f16s"   (modes alternate in one process)
+
+A setting without precision= runs in --precision.
 """
 import argparse
 import json
@@ -41,10 +44,14 @@ def main():
     g = 0.1 * torch.randn(B, 256, generator=torch.Generator().manual_seed(1)).cuda()
     out = torch.empty(B, (L // 256) * 256, device="cuda")
     fr = torch.empty(B, dtype=torch.int64, device="cuda")
-    settings = [dict((kv.split("=")[0], int(kv.split("=")[1])) for kv in s.split(",")) for s in args.settings.split(";")]
+    def value(k, v):
+        return v if k == "precision" else int(v)
+
+    settings = [dict((kv.split("=")[0], value(*kv.split("="))) for kv in s.split(",")) for s in args.settings.split(";")]
     times = [[] for _ in settings]
 
     def apply(st):
+        nat.set_precision(st.get("precision", args.precision))
         for k in ("graph", "pdl", "wide_variant", "branches", "pair"):
             if k in st:
                 nat.set_option(k, st[k])
@@ -69,8 +76,10 @@ def main():
             times[si].append(e0.elapsed_time(e1) / args.calls)
     res = []
     for st, ts in zip(settings, times):
-        res.append({"setting": st, "ms_median": float(np.median(ts)), "ms_min": float(np.min(ts)), "ms_all": ts})
-        print(f"B={B} x {args.secs:g}s  {st}:  median {np.median(ts):8.3f} ms   min {np.min(ts):8.3f} ms", flush=True)
+        res.append({"setting": st, "ms_median": float(np.median(ts)), "ms_min": float(np.min(ts)), "ms_max": float(np.max(ts)),
+                    "ms_all": ts})
+        print(f"B={B} x {args.secs:g}s  {st}:  median {np.median(ts):8.3f} ms   min {np.min(ts):8.3f} ms   "
+              f"max {np.max(ts):8.3f} ms", flush=True)
     if args.json:
         json.dump({"batch": B, "secs": args.secs, "precision": args.precision, "results": res}, open(args.json, "w"), indent=1)
 

@@ -20,7 +20,7 @@ def main():
     ap.add_argument("--batch", type=int, default=32)
     ap.add_argument("--secs", type=float, default=10.0)
     ap.add_argument("--json", default=None)
-    ap.add_argument("--precision", default="fp32", choices=["fp32", "f16x3", "f16"])
+    ap.add_argument("--precision", default="fp32", choices=["fp32", "f16x3", "f16", "f16s"])
     ap.add_argument("--wide-variant", type=int, default=None)
     ap.add_argument("--pdl", type=int, default=None)
     ap.add_argument("--pair", type=int, default=None)

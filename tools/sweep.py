@@ -53,10 +53,14 @@ def main():
             ts.append(time.perf_counter() - t0)
         assert len(out) == B and np.isfinite(out[-1]).all()
         ms = 1e3 * float(np.median(ts))
+        nat = conv.model.native
+        # device workspace of one chunk of max_batch utterances (T = L // 256 frames), in this precision mode
+        ws_gb = nat.lib.ovc_workspace_floats(nat.handle, min(B, args.max_batch), L // 256) * 4e-9
         rows.append({"batch": B, "secs": secs, "ms": ms, "audio_s_per_s": audio_s / (ms * 1e-3),
-                     "launches_last_chunk": int(conv.model.native.last_launch_count),
-                     "graph_replays": int(conv.model.native.graph_replays)})
-        print(f"B={B:4d} x {secs:5.1f} s: {ms:9.2f} ms  {rows[-1]['audio_s_per_s']:9.1f} audio-s/s", flush=True)
+                     "launches_last_chunk": int(nat.last_launch_count), "graph_replays": int(nat.graph_replays),
+                     "workspace_gb": ws_gb})
+        print(f"B={B:4d} x {secs:5.1f} s: {ms:9.2f} ms  {rows[-1]['audio_s_per_s']:9.1f} audio-s/s  workspace {ws_gb:6.2f} GB",
+              flush=True)
     res = {"what": f"ToneColorConverter.convert_batch, host numpy in / out, max_batch {args.max_batch}, {args.precision}, "
                    "median wall time, one B200", "points": rows}
     if args.json:
