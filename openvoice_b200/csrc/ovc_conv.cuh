@@ -25,10 +25,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
-#ifndef OVC_FFMA2
-#define OVC_FFMA2 1   // 1: packed fma.rn.f32x2 inner loop (Blackwell FFMA2); 0: scalar FFMA
-#endif
-
 namespace ovc {
 
 enum EpiKind : int {
@@ -179,17 +175,6 @@ struct ConvCfg {
   static constexpr int MIN_BLOCKS = (THREADS >= 256) ? 2 : (THREADS >= 128 ? 3 : 4);
 };
 
-// Polyphase structure of the transposed convs (row r of a thread's 8 packed rows):
-//   stride 8: r = phase p; taps used: p<4 -> {x[n-1], x[n]}, p>=4 -> {x[n], x[n+1]}
-//   stride 2: r = 2*i + p; p=0 -> {x[n-1], x[n]}, p=1 -> {x[n], x[n+1]}
-template <int EPI>
-__host__ __device__ constexpr bool tap_is_zero(int k, int r) {
-  if (EPI == EPI_UPS8) return (k == 0 && r >= 4) || (k == 2 && r < 4);
-  if (EPI == EPI_UPS2) return (k == 0 && (r & 1)) || (k == 2 && !(r & 1));
-  return false;
-}
-
-#if OVC_FFMA2
 typedef unsigned long long u64;
 // d.lo += a.lo * x ; d.hi += a.hi * x  -- ptxas folds the {x, x} pack into the FFMA2 scalar-broadcast
 // operand form (SASS: FFMA2 Rd, Ra.F32x2.HI_LO, Rx.F32, Rd.F32x2.HI_LO), so it costs no instruction.
@@ -198,6 +183,11 @@ __device__ __forceinline__ void fma2_bcast(u64& d, const u64 a, const float x) {
   asm("mov.b64 %0, {%1, %1};" : "=l"(xx) : "f"(x));
   asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(d) : "l"(a), "l"(xx));
 }
+
+// Polyphase structure of the transposed convs (row r of a thread's 8 packed rows, pair rp = rows 2rp, 2rp+1):
+//   stride 8: r = phase p; taps used: p<4 -> {x[n-1], x[n]}, p>=4 -> {x[n], x[n+1]}
+//   stride 2: r = 2*i + p; p=0 -> {x[n-1], x[n]}, p=1 -> {x[n], x[n+1]}
+// true where tap k is zero for both rows of pair rp, so the packed FMA can be skipped
 template <int EPI>
 __host__ __device__ constexpr bool pair_is_zero(int k, int rp) {
   if (EPI == EPI_UPS8) return (k == 0 && rp >= 2) || (k == 2 && rp < 2);
@@ -248,52 +238,6 @@ __device__ __forceinline__ void compute_chunk(u64 (&acc)[2][4][4], const float* 
     }
   }
 }
-#else
-// one tap group of one 4-wide time chunk: load the X window, run the taps
-template <class C, int G>
-__device__ __forceinline__ void tap_group(float (&acc)[8][4], const float* __restrict__ xrow,
-                                          const float* __restrict__ wrow) {
-  using TG = typename C::G;
-  constexpr int NV = TG::nvec(G);
-  constexpr int LO = TG::lo(G);
-  float win[4 * NV];
-#pragma unroll
-  for (int i = 0; i < NV; ++i) {
-    const float4 v = *reinterpret_cast<const float4*>(xrow + LO + 4 * i);
-    win[4 * i + 0] = v.x; win[4 * i + 1] = v.y; win[4 * i + 2] = v.z; win[4 * i + 3] = v.w;
-  }
-#pragma unroll
-  for (int k = TG::k_lo(G); k < TG::k_hi(G); ++k) {
-    const float4 wa = *reinterpret_cast<const float4*>(wrow + k * C::CO_T);
-    const float4 wb = *reinterpret_cast<const float4*>(wrow + k * C::CO_T + 4);
-    const float wf[8] = {wa.x, wa.y, wa.z, wa.w, wb.x, wb.y, wb.z, wb.w};
-    const int base = TG::off(k) - LO;
-#pragma unroll
-    for (int r = 0; r < 8; ++r) {
-      if (tap_is_zero<C::EPI>(k, r)) continue;
-#pragma unroll
-      for (int j = 0; j < 4; ++j) acc[r][j] = fmaf(wf[r], win[base + j], acc[r][j]);
-    }
-  }
-}
-
-template <class C>
-__device__ __forceinline__ void compute_chunk(float (&acc)[2][8][4], const float* __restrict__ xs,
-                                              const float* __restrict__ ws, int tb, int cb) {
-#pragma unroll 1
-  for (int ci = 0; ci < C::CI_CH; ++ci) {
-    const float* wrow = ws + ci * (C::K * C::CO_T) + cb;
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      const float* xrow = xs + ci * C::XW + C::HL + tb + 32 * c;
-      tap_group<C, 0>(acc[c], xrow, wrow);
-      if constexpr (C::NG >= 2) tap_group<C, 1>(acc[c], xrow, wrow);
-      if constexpr (C::NG >= 3) tap_group<C, 2>(acc[c], xrow, wrow);
-      if constexpr (C::NG >= 4) tap_group<C, 3>(acc[c], xrow, wrow);
-    }
-  }
-}
-#endif
 
 // stage one ci-chunk of X: rows [ci0, ci0+CI_CH), time [t0-HL, t0+T_T+HR)
 template <class C>
@@ -387,7 +331,6 @@ __global__ void __launch_bounds__(C::THREADS, C::MIN_BLOCKS) conv1d_f32(const Co
   stage_x_activate<C>(xsm, a.slope);
   __syncthreads();
 
-#if OVC_FFMA2
   u64 accw[2][4][4];
 #pragma unroll
   for (int c = 0; c < 2; ++c)
@@ -395,15 +338,6 @@ __global__ void __launch_bounds__(C::THREADS, C::MIN_BLOCKS) conv1d_f32(const Co
     for (int r = 0; r < 4; ++r)
 #pragma unroll
       for (int j = 0; j < 4; ++j) accw[c][r][j] = 0ull;
-#else
-  float accw[2][8][4];
-#pragma unroll
-  for (int c = 0; c < 2; ++c)
-#pragma unroll
-    for (int r = 0; r < 8; ++r)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) accw[c][r][j] = 0.f;
-#endif
 
   const int n_chunks = a.n_chunks;
   for (int ch = 0; ch < n_chunks; ++ch) {
@@ -424,7 +358,6 @@ __global__ void __launch_bounds__(C::THREADS, C::MIN_BLOCKS) conv1d_f32(const Co
     __syncthreads();
   }
 
-#if OVC_FFMA2
   float acc[2][8][4];
 #pragma unroll
   for (int c = 0; c < 2; ++c)
@@ -435,9 +368,6 @@ __global__ void __launch_bounds__(C::THREADS, C::MIN_BLOCKS) conv1d_f32(const Co
         acc[c][2 * rp][j] = __uint_as_float((unsigned)(accw[c][rp][j] & 0xffffffffull));
         acc[c][2 * rp + 1][j] = __uint_as_float((unsigned)(accw[c][rp][j] >> 32));
       }
-#else
-  float (&acc)[2][8][4] = accw;
-#endif
 
   // ------------------------------------------------------------------ epilogue
   const int row0 = blockIdx.y * C::CO_T + cb;   // first packed row of this thread

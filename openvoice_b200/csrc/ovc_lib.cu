@@ -102,6 +102,41 @@ static const PrepareFn kPrepare[V_COUNT] = {
 #undef X
 };
 
+// The tensor-core conv instantiations, each with its dynamic shared memory.  launch_tc and launch_pair take their kernel
+// from these tables and finalize sets every kernel's shared-memory limit from them, so whatever can be launched has its
+// limit set.  A new instantiation is one more entry here.
+struct TcConvKernel {
+  int TN; bool in16, out16;   // output columns per CTA; fp16 input / output activations (precision 3)
+  void (*fn)(TcConvArgs, int, int, CUtensorMap);
+  size_t smem;
+};
+template <int TN, bool IN16 = false, bool OUT16 = false>
+static TcConvKernel tcconv_entry() { return {TN, IN16, OUT16, tcconv_kernel<TN, IN16, OUT16>, TcnCfg<TN>::SMEM_BYTES}; }
+static const TcConvKernel kTcConv[] = {
+    tcconv_entry<128>(), tcconv_entry<64>(), tcconv_entry<32>(),
+    tcconv_entry<128, false, true>(),   // conv_pre of precision 3: fp32 z_hat in, fp16 out
+    tcconv_entry<128, true, true>(), tcconv_entry<64, true, true>(), tcconv_entry<32, true, true>()};
+
+struct TcPairKernel {
+  int TN;   // = the pair's channel count
+  void (*fn)(TcPairArgs, int, int, CUtensorMap);
+  size_t smem;
+};
+template <int TN>
+static TcPairKernel tcpair_entry() { return {TN, tcpair_kernel<TN>, TcpCfg<TN>::SMEM_BYTES}; }
+static const TcPairKernel kTcPair[] = {tcpair_entry<64>(), tcpair_entry<32>()};
+
+static const TcConvKernel* find_tcconv(int TN, bool in16, bool out16) {
+  for (const TcConvKernel& k : kTcConv)
+    if (k.TN == TN && k.in16 == in16 && k.out16 == out16) return &k;
+  return nullptr;
+}
+static const TcPairKernel* find_tcpair(int TN) {
+  for (const TcPairKernel& k : kTcPair)
+    if (k.TN == TN) return &k;
+  return nullptr;
+}
+
 struct HostTensor {
   std::vector<int64_t> shape;
   std::vector<float> data;
@@ -702,15 +737,8 @@ static int finalize(ovc_ctx* c) {
   c->h_tcw.clear();
   c->h_tcw.shrink_to_fit();
   CK(cudaFuncSetAttribute(tcconv_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcwCfg::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_kernel<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<128>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<64>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<32>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_kernel<128, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<128>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_kernel<128, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<128>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_kernel<64, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<64>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcconv_kernel<32, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcnCfg<32>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcpair_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcpCfg<32>::SMEM_BYTES));
-  CK(cudaFuncSetAttribute(tcpair_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)TcpCfg<64>::SMEM_BYTES));
+  for (const TcConvKernel& k : kTcConv) CK(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
+  for (const TcPairKernel& k : kTcPair) CK(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem));
   if (c->d_cond_wrow) cudaFree(c->d_cond_wrow);
   if (c->d_cond_sel) cudaFree(c->d_cond_sel);
   CK(cudaMalloc(&c->d_cond_wrow, wrow.size() * sizeof(int)));
@@ -948,9 +976,11 @@ static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const f
   a.passes = (r.c->precision == 2 || f16s) ? 1 : 3;
   if (T.TN == 0) return fail(OVC_ERR_INVALID, "conv %d -> %d (k %d, dilation %d) does not fit the tensor-core kernels", T.Cin, T.Ntot, T.K, T.DIL);
   if (!(o.slope >= 0.f && o.slope <= 1.f)) return fail(OVC_ERR_INVALID, "leaky_relu slope %g outside [0, 1]", (double)o.slope);
-  // the instantiations that exist: <TN, true, true> and <128, false, true> (conv_pre), linear epilogue only
-  if (f16s && (!o.out16 || o.epi != 0 || (!o.in16 && T.TN != 128)))
-    return fail(OVC_ERR_INVALID, "no fp16-storage tensor-core kernel for conv %d -> %d (fp16 in %d, epilogue %d)", T.Cin, T.Ntot, (int)o.in16, o.epi);
+  // the fp16-storage instantiations have the linear epilogue only
+  const TcConvKernel* kern = find_tcconv(T.TN, o.in16, o.out16);
+  if (!kern || (f16s && o.epi != 0))
+    return fail(OVC_ERR_INVALID, "no tensor-core kernel for conv %d -> %d (fp16 in %d, fp16 out %d, epilogue %d)", T.Cin, T.Ntot,
+                (int)o.in16, (int)o.out16, o.epi);
   const double units = (double)r.B * t_len;
   const int eff_k = o.family == 2 ? 2 : T.K;   // polyphase transposed conv: 2 of the 3 packed taps are non-zero per row
   const double in_b = o.in16 ? 2.0 : 4.0, out_b = o.out16 ? 2.0 : 4.0;   // bytes per element
@@ -983,18 +1013,7 @@ static int launch_tc(Run& r, const TcLayer& T, const float* x, float* y, const f
   const int ncol = T.Ntot / T.TN;
   const int per_col = std::max(1, r.c->sm_count / ncol / std::max(1, o.grid_div));
   dim3 pg((unsigned)std::min(total, per_col), ncol, 1);
-  return launch_kernel(r, rec, [&] {
-    if (o.in16) {
-      if (T.TN == 128) return launch_ex(tcconv_kernel<128, true, true>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
-      if (T.TN == 64) return launch_ex(tcconv_kernel<64, true, true>, pg, TCN_THREADS, TcnCfg<64>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
-      return launch_ex(tcconv_kernel<32, true, true>, pg, TCN_THREADS, TcnCfg<32>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
-    }
-    if (o.out16)   // conv_pre: fp32 z_hat in, fp16 out
-      return launch_ex(tcconv_kernel<128, false, true>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
-    if (T.TN == 128) return launch_ex(tcconv_kernel<128>, pg, TCN_THREADS, TcnCfg<128>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
-    if (T.TN == 64) return launch_ex(tcconv_kernel<64>, pg, TCN_THREADS, TcnCfg<64>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
-    return launch_ex(tcconv_kernel<32>, pg, TCN_THREADS, TcnCfg<32>::SMEM_BYTES, r.st, pdl, a, n_tt, total, tmap);
-  });
+  return launch_kernel(r, rec, [&] { return launch_ex(kern->fn, pg, TCN_THREADS, kern->smem, r.st, pdl, a, n_tt, total, tmap); });
 }
 
 // one ResBlock conv pair (c1 dilated, c2 dilation 1, residual = the pair's input) as ONE kernel: C = 64 / 32 stages
@@ -1011,6 +1030,8 @@ static bool pair_fits(const TcLayer& T1, const TcLayer& T2) {
 static int launch_pair(Run& r, const TcLayer& T1, const TcLayer& T2, const float* x, float* y, int t_len, int mul, const TcOpt& o) {
   TcPairArgs a{};
   const int C = T1.TN;
+  const TcPairKernel* kern = find_tcpair(C);
+  if (!kern) return fail(OVC_ERR_INVALID, "no conv-pair kernel for C = %d", C);
   a.x = x; a.x_bs = (long long)C * r.P * mul;
   a.w1 = reinterpret_cast<const uint16_t*>(r.c->d_tcw + T1.w_off);
   a.w2 = reinterpret_cast<const uint16_t*>(r.c->d_tcw + T2.w_off);
@@ -1031,10 +1052,7 @@ static int launch_pair(Run& r, const TcLayer& T1, const TcLayer& T2, const float
   const ProfRec rec{C == 64 ? V_TCPAIR64 : V_TCPAIR32, 1, 2.0 * 2.0 * C * C * T1.K * units,
                     4.0 * C * (2 + (o.accumulate ? 1 : 0)) * units, (C << 16) | (T1.K << 8) | T1.DIL};
   dim3 pg((unsigned)std::min(total, r.c->sm_count), 1, 1);
-  return launch_kernel(r, rec, [&] {
-    return C == 64 ? launch_ex(tcpair_kernel<64>, pg, TCN_THREADS, TcpCfg<64>::SMEM_BYTES, r.st, false, a, n_tt, total, tmap)
-                   : launch_ex(tcpair_kernel<32>, pg, TCN_THREADS, TcpCfg<32>::SMEM_BYTES, r.st, false, a, n_tt, total, tmap);
-  });
+  return launch_kernel(r, rec, [&] { return launch_ex(kern->fn, pg, TCN_THREADS, kern->smem, r.st, false, a, n_tt, total, tmap); });
 }
 
 // src16: the source is fp16 (read through the same pointer type as the fp32 workspace buffers), dst is always fp32
@@ -1286,21 +1304,12 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
   ovc_ctx* c = r.c;
   const int B = r.B, Tmax = r.Tmax, P = W.P;
   // ---- generator (models.py:272-291).  Lengths: frames * cumulative upsampling.
-  const bool pre_tc = c->precision >= 1 && c->tc_pre.TN != 0;
-  const bool f16s = c->precision == 3;   // fp16 activations from conv_pre's output to conv_post's input
-  if (f16s && !pre_tc) return fail(OVC_ERR_INVALID, "precision 3 needs conv_pre on the tensor cores (inter_channels %% 32 == 0)");
-  if (!pre_tc) {
-    ConvArgs a = conv_args(ws + W.z, 192, P, ws + W.dpre, 512, P, r.glens, 1, 1.f);
-    a.bias = cond + c->cond_off_dec; a.bias_bs = c->cond_rows_out;
-    a.lens_in = lens;          // z_hat * y_mask
-    TRY(launch(r, c->dec_pre, a, Tmax));
-    TRY(tap(r, "dec.pre", ws + W.dpre, 512, Tmax, P));
-  }
   float* bufA = ws + W.bufA; float* bufB = ws + W.bufB; float* bufC = ws + W.bufC; float* bufD = ws + W.bufD;
   if (c->precision >= 1) {
     // ---- tensor-core generator: channels-last [t][C] from conv_pre's output to conv_post's input.
     // ConvTranspose1d = polyphase conv Cin -> s*Cout whose row n IS output rows s*n .. s*n+s-1 of the
     // channels-last result; ResBlock convs = tcconv with fused lrelu / bias / residual / MRF average.
+    const bool f16s = c->precision == 3;   // fp16 activations from conv_pre's output to conv_post's input
     float* bufE = ws + W.bufE;
     float* bufF = ws + W.bufF;   // fp32 [C][T] scratch for debug taps
     auto tap_cl = [&](const char* nm, const float* cl, int C, int T_, int pitch) -> int {
@@ -1308,19 +1317,15 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
       TRY(launch_transpose(r, cl, bufF, pitch, C, f16s));
       return tap(r, nm, bufF, C, T_, pitch);
     };
-    if (pre_tc) {
-      // conv_pre (192 -> 512, k 7) + cond(g) on the tensor cores too: z channels-last through bufA, result straight into
-      // bufE; the input is cut at the frame lengths (z_hat * y_mask), the output runs over the generator's own limit
-      TRY(launch_transpose(r, ws + W.z, bufA, 192, P));
-      TcOpt e;
-      e.bias = cond + c->cond_off_dec; e.bias_bs = c->cond_rows_out;
-      e.lens_x = lens; e.has_lens_x = lens != nullptr;
-      e.out16 = f16s;
-      TRY(launch_tc(r, c->tc_pre, bufA, bufE, nullptr, Tmax, 1, e));
-      TRY(tap_cl("dec.pre", bufE, 512, Tmax, P));
-    } else {
-      TRY(launch_transpose(r, ws + W.dpre, bufE, 512, P));
-    }
+    // conv_pre (192 -> 512, k 7) + cond(g) on the tensor cores too: z channels-last through bufA, result straight into
+    // bufE; the input is cut at the frame lengths (z_hat * y_mask), the output runs over the generator's own limit
+    TRY(launch_transpose(r, ws + W.z, bufA, 192, P));
+    TcOpt e;
+    e.bias = cond + c->cond_off_dec; e.bias_bs = c->cond_rows_out;
+    e.lens_x = lens; e.has_lens_x = lens != nullptr;
+    e.out16 = f16s;
+    TRY(launch_tc(r, c->tc_pre, bufA, bufE, nullptr, Tmax, 1, e));
+    TRY(tap_cl("dec.pre", bufE, 512, Tmax, P));
     const float* stage_in = bufE;
     int cin = 512, up = 1;
     const bool par = W.branches && !c->prof && !c->debug;
@@ -1356,6 +1361,12 @@ static int run_dec(Run& r, const WsLayout& W, float* ws, const float* cond, cons
                                                         y_len, r.glens, Tmax, up);
     });
   }
+  // ---- fp32 generator: [C][T] activations, every conv on the FFMA kernels
+  ConvArgs a = conv_args(ws + W.z, 192, P, ws + W.dpre, 512, P, r.glens, 1, 1.f);
+  a.bias = cond + c->cond_off_dec; a.bias_bs = c->cond_rows_out;
+  a.lens_in = lens;          // z_hat * y_mask
+  TRY(launch(r, c->dec_pre, a, Tmax));
+  TRY(tap(r, "dec.pre", ws + W.dpre, 512, Tmax, P));
   const float* stage_in = ws + W.dpre;
   int cin = 512, up = 1;
   for (int i = 0; i < 4; ++i) {

@@ -20,11 +20,8 @@ __device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo_bytes
   return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16) |
          ((uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32) | (1ull << 46);
 }
-// instruction descriptor (cute::UMMA::InstrDescriptor) for kind::tf32, fp32 accumulate, K-major A and B
-__host__ __device__ constexpr uint32_t make_idesc_tf32(int M, int N) {
-  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-// ... for kind::f16 with fp16 A and B (a_format = b_format = 0), fp32 accumulate (c_format = 1), K-major A and B
+// instruction descriptor (cute::UMMA::InstrDescriptor) for kind::f16 with fp16 A and B (a_format = b_format = 0),
+// fp32 accumulate (c_format = 1), K-major A and B
 __host__ __device__ constexpr uint32_t make_idesc_f16(int M, int N) {
   return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
@@ -40,15 +37,6 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {  
 __device__ __forceinline__ void fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 
-// D[tmem] (+)= A[smem] * B[smem]^T, issued by ONE thread
-__device__ __forceinline__ void mma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, bool accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"((uint32_t)accumulate)
-      : "memory");
-}
 // D[tmem] (+)= A[smem] * B[smem]^T with fp16 operands (K = 16 per instruction), fp32 accumulation
 __device__ __forceinline__ void mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, bool accumulate) {
   asm volatile(
@@ -62,57 +50,6 @@ __device__ __forceinline__ void mma_f16(uint32_t tmem_d, uint64_t adesc, uint64_
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_addr(bar)) : "memory");
 }
-// 32 lanes x 8 consecutive fp32 columns: lane i of the warp reads TMEM lane (base_lane + i)
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-               : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// 32 lanes x 32 consecutive fp32 columns (one full 128-byte output line per thread)
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
-}
-
-// issue-only variant + a wait that carries the registers as in/out operands, so no use can be scheduled above it;
-// lets the epilogue overlap the TMEM read with its global loads
-__device__ __forceinline__ void tmem_ld32_issue(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-      "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-__device__ __forceinline__ void tmem_ld_wait(uint32_t (&r)[32]) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]),
-                 "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]), "+r"(r[16]),
-                 "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]), "+r"(r[24]),
-                 "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31])
-               :
-               : "memory");
-}
-
 // 16 TMEM lanes x 32 consecutive fp32 columns in the mma-accumulator fragment layout (16x256b.x4): thread i of the
 // warp receives, for each 8-column group g = 0..3,
 //   r[4g + 0..1] = lane (i / 4),     columns 8g + 2 (i % 4) + {0, 1}
@@ -156,12 +93,6 @@ __device__ __forceinline__ bool elect_one() {
       "selp.b32 %0, 1, 0, p;\n\t}"
       : "=r"(pred));
   return pred != 0;
-}
-
-// split an fp32 into a tf32-exact high part and the fp32 remainder (3xTF32: a*b ~ ah*bh + al*bh + ah*bl)
-__device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
-  hi = __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
-  lo = x - hi;
 }
 
 // ---- split precision on fp16 operands ("3xFP16"):  x = hi + lo / 2^11 (+ 2^-23 |x|), hi = fp16(x),

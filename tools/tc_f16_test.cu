@@ -16,6 +16,17 @@ using namespace ovc;
 
 constexpr int M = 128, N = 64, K = 64, ROWS_A = 160;
 
+// 32 lanes x 8 consecutive fp32 columns: lane i of the warp reads TMEM lane (base_lane + i)
+__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
+  uint32_t r[8];
+  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+               : "r"(taddr));
+  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+  for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
+
 __global__ void __launch_bounds__(128) gemm_test(const float* A, const float* B, float* D, int shift, int split) {
   extern __shared__ __align__(128) unsigned char smem[];
   unsigned char* a_hi = smem;                                   // [K/8][ROWS_A][8 halfs]
@@ -74,9 +85,9 @@ __global__ void __launch_bounds__(128) gemm_test(const float* A, const float* B,
   tc::fence_after();
   for (int c0 = 0; c0 < N; c0 += 8) {
     float v[8], l[8];
-    tc::tmem_ld8(tmem_d + ((uint32_t)(warp * 32) << 16) + c0, v);
+    tmem_ld8(tmem_d + ((uint32_t)(warp * 32) << 16) + c0, v);
     if (split) {
-      tc::tmem_ld8(tmem_d + ((uint32_t)(warp * 32) << 16) + N + c0, l);
+      tmem_ld8(tmem_d + ((uint32_t)(warp * 32) << 16) + N + c0, l);
       for (int i = 0; i < 8; ++i) v[i] = fmaf(l[i], tc::kLoInv, v[i]);
     }
     for (int i = 0; i < 8; ++i) D[(size_t)tid * N + c0 + i] = v[i];
